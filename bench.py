@@ -26,6 +26,8 @@ scaling is "strong".
              at the same N: ms per frame, efficiency against rank 0 rendering the frame alone, frame check
 `--impl reference` times that CPU implementation alone with the same metric/config.
 `--workload` picks another configuration (c0..c4, chess1080, chess4k); the default is the headline one.
+`--dump-outputs DIR` writes the frame the last timed step rendered as DIR/frame.npy (float32 [H, W, 3], what a caller of
+c2rt_render_device receives); inputs are fixed (scene file, camera, RNG seed), so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -62,6 +64,22 @@ def workload_label(name):
 BAND_ROWS = 8
 RNG_SEED = 0xC2E55
 L2_FLUSH_BYTES = 256 << 20  # > 126 MB L2
+DUMP_BYTES = 64 << 20       # --dump-outputs writes at most this much
+
+
+def dump_frame(out_dir, frame):
+    """--dump-outputs: `frame` ([H, W, 3] float32) as out_dir/frame.npy.  A frame larger than DUMP_BYTES (the 8K workload) keeps
+    every k-th row from row 0, the smallest k that fits, and out_dir/frame_rows.npy lists the rows kept."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    frame = np.ascontiguousarray(frame, dtype=np.float32)
+    H = frame.shape[0]
+    if frame.nbytes > DUMP_BYTES:
+        fit = (DUMP_BYTES - 8 * H - 4096) // frame[0].nbytes   # room for the row list and the two .npy headers
+        rows = np.arange(0, H, -(-H // fit))
+        frame = frame[rows]
+        np.save(os.path.join(out_dir, "frame_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "frame.npy"), frame)
 
 
 def load_calibration():
@@ -261,7 +279,10 @@ def main():
     ap.add_argument("--calibrate", nargs="*", default=None, help="(CPU) recount algorithmic FLOPs/rays of the named workloads")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-scaling-target", action="store_true", help="skip the side measurement of the 8K chessboard scene")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step as DIR/frame.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.calibrate is not None:
@@ -451,6 +472,17 @@ def main():
                 raise SystemExit(f"{self.name}: {n_to} gate / frame-complete wait(s) timed out: the timed frames are not complete frames")
             return float(t[0]) / steps, self.launches
 
+        def frame_host(self):
+            """(rank 0) the frame the last step left in HBM, copied to the host as [H, W, 3] float32."""
+            if self.mode == "p2p":
+                import ctypes as C
+                got = torch.empty((self.H, self.W, 3), dtype=torch.float32, pin_memory=True)
+                api._check(api.lib.c2rt_frame_download(got.data_ptr(), C.c_void_p(self.peer_frame_ptr), self.H * self.W * 12,
+                                                       torch.cuda.current_stream().cuda_stream))
+                torch.cuda.synchronize()
+                return got.numpy()
+            return self.frame.cpu().numpy()
+
         def time_alone(self, steps, warmup=2):
             """(N > 1) rank 0 renders the whole frame alone, the other ranks idle: the T(1) of the efficiency figure, same run."""
             ms = 0.0
@@ -544,6 +576,8 @@ def main():
                           # the timed loops alone are shorter than one nvidia-smi period)
     ms_per_step, n_launches = run.time_steps(args.steps, args.warmup)
     kernel_ms = ms_per_step   # one render kernel per rank and step is the whole step (N > 1: it also carries the band gather)
+    if args.dump_outputs and rank == 0:
+        dump_frame(args.dump_outputs, run.frame_host())
 
     frame_check = run.verify()
     if world > 1:

@@ -508,3 +508,19 @@ def test_bench_parity_check_passes_the_oracle_and_fails_a_wrong_frame(tmp_path):
     assert not rep["pass"] and rep["px_over_1e-3"] == 1 and abs(rep["max_abs"] - 2e-3) < 1e-6
     rep = bench.oracle_parity(path, w, h, {}, lambda y0, y1: bad[y0:y1], rows=16)   # two windows, rows 0-7 and 32-39: the bad pixel is outside
     assert rep["pass"] and rep["n"] == 16 * w
+
+
+def test_bench_dump_frame_keeps_whole_frames_and_samples_rows_of_large_ones(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: a frame within the size limit is written whole; a larger one keeps every k-th row, the rows listed
+    beside it, and the files stay within the limit."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    frame = np.random.default_rng(0).random((100, 2000, 3), dtype=np.float32)   # 2.4 MB
+    bench.dump_frame(str(tmp_path / "small"), frame[:10])
+    assert sorted(os.listdir(tmp_path / "small")) == ["frame.npy"]
+    np.testing.assert_array_equal(np.load(tmp_path / "small" / "frame.npy"), frame[:10])
+    bench.dump_frame(str(tmp_path / "big"), frame)
+    rows = np.load(tmp_path / "big" / "frame_rows.npy")
+    assert rows.dtype == np.float64 and rows[0] == 0 and len(set(np.diff(rows))) == 1
+    np.testing.assert_array_equal(np.load(tmp_path / "big" / "frame.npy"), frame[rows.astype(int)])
+    assert sum(os.path.getsize(p) for p in (tmp_path / "big").iterdir()) <= 1 << 20
