@@ -816,6 +816,10 @@ void fill_params(FrameParams& fp, const c2rt_camera* cam, const c2rt_settings* s
         fp.solo_fast = fp.solo_side != 0 && lens_ok && std::isfinite(dray2) && std::isfinite(mag) && mag < 1e6 && dray2 < 1e12 &&
                        std::fabs(h) > lens_y + 1e-5 && (double)fp.solo_side * (ly - y) > 1e-5 && dmin > 1e-6 &&
                        !set->prepass_only && !(no_fast && no_fast[0] == '1');
+        // d.y = fma(dv.y, sy, fma(du.y, sx, ul_rel.y)) + tap_d.y (render_kernel.cu screen_dir): with du.y = +-0 the inner fma is
+        // the same value for every sx >= 0, so d.y is constant along a row.  Tested on the value the kernel uses, not on the
+        // camera's roll: the corners reach the ABI from any host.
+        fp.solo_rows = fp.solo_fast && fp.du[1] == 0.0;
     }
 }
 

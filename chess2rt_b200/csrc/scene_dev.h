@@ -120,9 +120,11 @@ struct FrameParams {
     // DOF / stereo — off the plane, light on the camera's side, moderate magnitudes: c2rt_api.cu fill_params); the kernels
     // without the sampling loop only run such frames, the sampling kernels branch on it.  Then: side of the plane the camera is
     // on (+1 above, -1 below), the sign bit a ray's d.y must NOT have xor'ed in (0x80000000 above the plane: d.y must be
-    // negative), the camera position's height above the plane (pos.y - y), and 1e-18 max|d|^2 over the frame's camera rays
+    // negative), the camera position's height above the plane (pos.y - y), and 1e-18 max|d|^2 over the frame's camera rays.
+    // solo_rows: a regular frame with du.y == 0 (no camera roll): a camera ray's d.y depends on its row and AA tap only, and
+    // render_solo_kernel takes the plane hit and light height from a per-row table (render_kernel.cu row_tap)
     int solo_fast, solo_side;
-    uint32_t solo_sign, pad_solo;
+    uint32_t solo_sign, solo_rows;
     double solo_h, graze_dy2;
     const int* cancel;                // device flag raised by c2rt_cancel: CTAs that start after it skip their tile (nullptr: off)
     // outputs (rgb == nullptr: only the ARGB plane is wanted)
