@@ -19,9 +19,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SC = os.path.join(ROOT, "scenes")
 
 # (scene, overrides, camera roll and pitch in the file): procedural texture, checker, cubemap environment (misses go through
-# env_lookup), bitmap
+# env_lookup), bitmap, and an untextured Phong lobe of exponent 5000 (the FP64 lobe)
 SCENES = [("lecture4-proc-texture.sdl", {}, 0.0, -30.0), ("lecture4.sdl", {}, 0.0, -30.0),
-          ("../tests/scenes/sky_plane.sdl", {}, 5.0, 8.0), ("zaphod.sdl", {"dof": 0}, 2.3, -41.8)]
+          ("../tests/scenes/sky_plane.sdl", {}, 5.0, 8.0), ("zaphod.sdl", {"dof": 0}, 2.3, -41.8),
+          ("../tests/scenes/phong_sharp.sdl", {}, 0.0, -30.0)]
 SIZES = ((333, 187), (130, 61), (66, 9))
 KX, KY = (0.0, 0.3, 0.6, 0.0, 0.6), (0.0, 0.3, 0.0, 0.6, 0.6)   # AA tap offsets (renderer.d:235-242)
 
