@@ -1,6 +1,6 @@
 // C ABI of libc2rt.so (include/c2rt.h): scene validation + upload (scene class, bounding spheres, node runs), frame
-// launches on 1..8 devices (one helper thread per extra device: DevicePool), band copies to the host frame or P2P band
-// stores into device 0's frame, error reporting.  No CPU fallback anywhere:
+// launches on 1..8 devices (one helper thread per extra device: DevicePool), band copies to the host frame, error
+// reporting.  No CPU fallback anywhere:
 // every rendering entry point fails with C2RT_ERR_CUDA if the CUDA runtime cannot run the kernel.
 #include <cuda_runtime.h>
 
@@ -67,7 +67,6 @@ struct DeviceCtx {
     int dev = -1;
     cudaStream_t stream = nullptr, copy_stream = nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
-    cudaEvent_t chunk_done[8] = {};
     std::vector<cudaEvent_t> band_done;
     uint64_t uploaded_scene = 0;   // id of the scene currently in this device's constant memory
     unsigned long long* d_counters = nullptr;
@@ -79,7 +78,6 @@ struct DeviceCtx {
     float* d_rgb = nullptr;
     uint32_t* d_argb = nullptr;
     size_t rgb_cap = 0, argb_cap = 0;
-    bool peer_to_root = false;     // can store straight into device 0's frame
 };
 
 struct Context {
@@ -116,8 +114,7 @@ public:
         for (auto& t : th_) t.join();
         th_.clear();
     }
-    int size() const { return (int)th_.size(); }
-    // runs fn(w) on every worker w = 0..size()-1; returns immediately, wait() joins the round
+    // runs fn(w) on every worker w = 0..n_workers-1; returns immediately, wait() joins the round
     void run(std::function<void(int)> fn) {
         fn_ = std::move(fn);
         pending_.store((int)th_.size(), std::memory_order_relaxed);
@@ -185,7 +182,6 @@ void destroy_device(DeviceCtx& c) {
     cudaSetDevice(c.dev);
     if (c.stream) cudaStreamDestroy(c.stream);
     if (c.copy_stream) cudaStreamDestroy(c.copy_stream);
-    for (auto& e : c.chunk_done) if (e) cudaEventDestroy(e);
     for (auto& e : c.band_done) cudaEventDestroy(e);
     if (c.e0) cudaEventDestroy(c.e0);
     if (c.e1) cudaEventDestroy(c.e1);
@@ -219,7 +215,6 @@ int init_locked(int n_gpus, const int* ids) {
         CU(cudaSetDevice(dev));
         CU(cudaStreamCreateWithFlags(&c.stream, cudaStreamNonBlocking));
         CU(cudaStreamCreateWithFlags(&c.copy_stream, cudaStreamNonBlocking));
-        for (auto& e : c.chunk_done) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         CU(cudaEventCreate(&c.e0));
         CU(cudaEventCreate(&c.e1));
         CU(cudaMalloc(&c.d_counters, 2 * sizeof(unsigned long long)));
@@ -233,17 +228,6 @@ int init_locked(int n_gpus, const int* ids) {
         CU(cudaMemcpy(c.d_lut, g_ctx.lut, 4097, cudaMemcpyHostToDevice));
         CU(cudaMalloc(&c.d_pixel, pixel_out_size()));
         g_ctx.n = i + 1;
-    }
-    // peers store their bands straight into the root device's frame when P2P is available
-    for (int i = 1; i < n_gpus; i++) {
-        int can = 0;
-        cudaDeviceCanAccessPeer(&can, g_ctx.d[i].dev, g_ctx.d[0].dev);
-        if (can) {
-            cudaSetDevice(g_ctx.d[i].dev);
-            cudaError_t pe = cudaDeviceEnablePeerAccess(g_ctx.d[0].dev, 0);
-            if (pe == cudaSuccess || pe == cudaErrorPeerAccessAlreadyEnabled) g_ctx.d[i].peer_to_root = true;
-            cudaGetLastError();
-        }
     }
     cudaSetDevice(g_ctx.d[0].dev);
     g_ctx.inited = true;
@@ -841,73 +825,82 @@ uint32_t local_tile_rows(uint32_t H, uint32_t rank, uint32_t n, uint32_t band_ro
     return (rows + TILE_H - 1) / TILE_H;
 }
 
-int render_direct_device(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb,
-                         uint32_t* launches_out, float* kernel_ms_out) {
-    const uint32_t W = set->frame_width, H = set->frame_height;
-    const size_t npx = (size_t)W * H;
-    uint32_t launches = 0;
-    {
-        DeviceCtx& c = g_ctx.d[i];
-        CU(cudaSetDevice(c.dev));
-        FrameParams fp;
-        fill_params(fp, cam, set, s, i);
-        fp.rank = (uint32_t)i;
-        fp.n_ranks = (uint32_t)n;
-        fp.tiles_per_band = 1;
-        fp.compact = 1;
-        fp.counters = c.d_counters;
-        fp.lut = c.d_lut;
-        fp.cancel = c.d_cancel;
-        // 2..16 interleaved bands per device (one band per ~256k pixels): each band is one launch + one contiguous
-        // D2H copy, so small frames must not be cut into many bands (every launch / copy costs a few host microseconds)
-        uint32_t per_dev = (uint32_t)std::min<size_t>(16, std::max<size_t>(2, npx / (size_t)n / 262144));
-        uint32_t brows = (H / ((uint32_t)n * per_dev) + TILE_H - 1) / TILE_H * TILE_H;
-        if (brows < TILE_H) brows = TILE_H;
-        fp.tiles_per_band = brows / TILE_H;
-        const uint32_t rows_owned = c2rt_band_rows_owned(H, fp.rank, fp.n_ranks, brows);
-        const size_t need = (size_t)rows_owned * W;
-        if (rgb && c.rgb_cap < need * 3) {
-            cudaFree(c.d_rgb);
-            c.d_rgb = nullptr; c.rgb_cap = 0;
-            CU(cudaMalloc(&c.d_rgb, std::max<size_t>(need, 1) * 3 * sizeof(float)));
-            c.rgb_cap = need * 3;
-        }
-        if (argb && c.argb_cap < need) {
-            cudaFree(c.d_argb);
-            c.d_argb = nullptr; c.argb_cap = 0;
-            CU(cudaMalloc(&c.d_argb, std::max<size_t>(need, 1) * sizeof(uint32_t)));
-            c.argb_cap = need;
-        }
-        fp.rgb = rgb ? c.d_rgb : nullptr;
-        fp.argb = argb ? c.d_argb : nullptr;
-        CU(cudaEventRecord(c.e0, c.stream));
-        uint32_t local_row = 0, b = 0;
-        for (uint32_t y0 = (uint32_t)i * brows; y0 < H; y0 += (uint32_t)n * brows, b++) {
-            const uint32_t rows = std::min<uint32_t>(brows, H - y0);
-            if (b >= c.band_done.size()) {
-                cudaEvent_t e;
-                CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                c.band_done.push_back(e);
-            }
-            fp.tile_row0 = b * fp.tiles_per_band;
-            CU(launch_frame(fp, s->mode, (rows + TILE_H - 1) / TILE_H, c.stream));
-            launches++;
-            CU(cudaEventRecord(c.band_done[b], c.stream));
-            CU(cudaStreamWaitEvent(c.copy_stream, c.band_done[b], 0));
-            if (rgb)
-                CU(cudaMemcpyAsync(rgb + (size_t)y0 * W * 3, c.d_rgb + (size_t)local_row * W * 3, (size_t)rows * W * 3 * sizeof(float),
-                                   cudaMemcpyDeviceToHost, c.copy_stream));
-            if (argb)
-                CU(cudaMemcpyAsync(argb + (size_t)y0 * W, c.d_argb + (size_t)local_row * W, (size_t)rows * W * sizeof(uint32_t),
-                                   cudaMemcpyDeviceToHost, c.copy_stream));
-            local_row += rows;
-        }
-        CU(cudaEventRecord(c.e1, c.stream));
-        CU(cudaStreamSynchronize(c.copy_stream));
-        CU(cudaEventSynchronize(c.e1));
-        CU(cudaEventElapsedTime(kernel_ms_out, c.e0, c.e1));
+// Rows per band of a c2rt_render frame on n devices, a whole number of tiles: device i renders bands i, i + n, i + 2n, ...
+// Each band is one launch and one contiguous D2H copy per output plane, and its copy runs while the next band renders.
+uint32_t frame_band_rows(int n, uint32_t H, uint32_t W) {
+    const uint32_t tile_rows = (H + TILE_H - 1) / TILE_H;
+    if (n == 1) {
+        // up to 4 bands: the D2H copy of a float frame costs more than rendering it, so most of it should overlap
+        const uint32_t bands = tile_rows >= 32 ? 4 : 1;
+        return (tile_rows + bands - 1) / bands * TILE_H;
     }
-    *launches_out = launches;
+    // 2..16 interleaved bands per device (one band per ~256k pixels): small frames must not be cut into many bands
+    // (every launch / copy costs a few host microseconds)
+    const uint32_t per_dev = (uint32_t)std::min<size_t>(16, std::max<size_t>(2, (size_t)W * H / (size_t)n / 262144));
+    return std::max<uint32_t>(TILE_H, (H / ((uint32_t)n * per_dev) + TILE_H - 1) / TILE_H * TILE_H);
+}
+
+// Grows a device buffer to at least `elems` elements; its contents are not kept.
+template <class T>
+int grow_buffer(T*& buf, size_t& cap, size_t elems) {
+    if (cap >= elems) return C2RT_OK;
+    cudaFree(buf);
+    buf = nullptr; cap = 0;
+    CU(cudaMalloc(&buf, std::max<size_t>(elems, 1) * sizeof(T)));
+    cap = elems;
+    return C2RT_OK;
+}
+
+// Device slot i's share of an n-device c2rt_render frame: its bands (frame_band_rows) render into the slot's compact
+// buffer, which holds only its own rows in order (the whole frame when n == 1), and each band is copied to its rows of
+// the caller's host frame on copy_stream once its launch has finished.  Returns when the copies are complete.
+int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb,
+                 uint32_t* launches_out, float* kernel_ms_out) {
+    const uint32_t W = set->frame_width, H = set->frame_height;
+    const uint32_t brows = frame_band_rows(n, H, W);
+    DeviceCtx& c = g_ctx.d[i];
+    CU(cudaSetDevice(c.dev));
+    FrameParams fp;
+    fill_params(fp, cam, set, s, i);
+    fp.rank = (uint32_t)i;
+    fp.n_ranks = (uint32_t)n;
+    fp.tiles_per_band = brows / TILE_H;
+    fp.compact = 1;
+    fp.counters = c.d_counters;
+    fp.lut = c.d_lut;
+    fp.cancel = c.d_cancel;
+    const size_t need = (size_t)c2rt_band_rows_owned(H, fp.rank, fp.n_ranks, brows) * W;
+    int rc = rgb ? grow_buffer(c.d_rgb, c.rgb_cap, need * 3) : C2RT_OK;
+    if (rc == C2RT_OK && argb) rc = grow_buffer(c.d_argb, c.argb_cap, need);
+    if (rc) return rc;
+    fp.rgb = rgb ? c.d_rgb : nullptr;
+    fp.argb = argb ? c.d_argb : nullptr;
+    CU(cudaEventRecord(c.e0, c.stream));
+    uint32_t local_row = 0, b = 0;
+    for (uint32_t y0 = (uint32_t)i * brows; y0 < H; y0 += (uint32_t)n * brows, b++) {
+        const uint32_t rows = std::min<uint32_t>(brows, H - y0);
+        if (b >= c.band_done.size()) {
+            cudaEvent_t e;
+            CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            c.band_done.push_back(e);
+        }
+        fp.tile_row0 = b * fp.tiles_per_band;
+        CU(launch_frame(fp, s->mode, (rows + TILE_H - 1) / TILE_H, c.stream));
+        CU(cudaEventRecord(c.band_done[b], c.stream));
+        CU(cudaStreamWaitEvent(c.copy_stream, c.band_done[b], 0));
+        if (rgb)
+            CU(cudaMemcpyAsync(rgb + (size_t)y0 * W * 3, c.d_rgb + (size_t)local_row * W * 3, (size_t)rows * W * 3 * sizeof(float),
+                               cudaMemcpyDeviceToHost, c.copy_stream));
+        if (argb)
+            CU(cudaMemcpyAsync(argb + (size_t)y0 * W, c.d_argb + (size_t)local_row * W, (size_t)rows * W * sizeof(uint32_t),
+                               cudaMemcpyDeviceToHost, c.copy_stream));
+        local_row += rows;
+    }
+    CU(cudaEventRecord(c.e1, c.stream));
+    CU(cudaStreamSynchronize(c.copy_stream));
+    CU(cudaEventSynchronize(c.e1));
+    CU(cudaEventElapsedTime(kernel_ms_out, c.e0, c.e1));
+    *launches_out = b;   // one launch per band
     return C2RT_OK;
 }
 
@@ -1088,174 +1081,36 @@ int c2rt_render(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set,
     if (rc) return rc;
     if (s->n_dev != g_ctx.n) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
     take_cancel_request();   // a cancel that arrived while no frame was in progress cancels nothing
-    const uint32_t W = set->frame_width, H = set->frame_height;
-    const size_t npx = (size_t)W * H;
     const int n = g_ctx.n;
-    const uint32_t band_rows = TILE_H;
-
-    // root frame
-    DeviceCtx& root = g_ctx.d[0];
-    CU(cudaSetDevice(root.dev));
-    if (rgb && root.rgb_cap < npx * 3) {
-        cudaFree(root.d_rgb);
-        root.d_rgb = nullptr; root.rgb_cap = 0;
-        CU(cudaMalloc(&root.d_rgb, npx * 3 * sizeof(float)));
-        root.rgb_cap = npx * 3;
+    // scene residency first, on this thread: make_resident patches the shared host copy of the scene block per device
+    for (int i = 0; i < n; i++) {
+        if (g_ctx.d[i].uploaded_scene == s->id) continue;
+        CU(cudaSetDevice(g_ctx.d[i].dev));
+        rc = make_resident(s, i, g_ctx.d[i].stream);
+        if (rc) return rc;
     }
-    if (argb && root.argb_cap < npx) {
-        cudaFree(root.d_argb);
-        root.d_argb = nullptr; root.argb_cap = 0;
-        CU(cudaMalloc(&root.d_argb, npx * sizeof(uint32_t)));
-        root.argb_cap = npx;
-    }
+    // Every device renders its bands and copies them to the host frame over its own PCIe link: the host copy of a float
+    // frame is the slow part, so N links beat one.  Worker w of the pool drives device w + 1, this thread drives device 0.
+    int rcs[C2RT_MAX_GPUS] = {};
+    uint32_t ls[C2RT_MAX_GPUS] = {};
+    float kms[C2RT_MAX_GPUS] = {};
+    std::string errs[C2RT_MAX_GPUS];
+    if (n > 1)
+        g_pool.run([&](int w) {
+            rcs[w + 1] = render_bands(w + 1, n, s, cam, set, rgb, argb, &ls[w + 1], &kms[w + 1]);
+            if (rcs[w + 1]) errs[w + 1] = g_err;
+        });
+    rcs[0] = render_bands(0, n, s, cam, set, rgb, argb, &ls[0], &kms[0]);
+    if (rcs[0]) errs[0] = g_err;
+    if (n > 1) g_pool.wait();
     uint32_t launches = 0;
-    bool copied = false;
-    double direct_kernel_ms = 0;
-    if (n == 1) {
-        // One device: launch the frame in up to 4 chunks of tile rows and copy each chunk back on a second
-        // stream while the next one renders (the D2H copy of a float frame costs more than rendering it).
-        DeviceCtx& c = root;
-        rc = make_resident(s, 0, c.stream);
-        if (rc) return rc;
-        FrameParams fp;
-        fill_params(fp, cam, set, s, 0);
-        fp.counters = c.d_counters;
-        fp.lut = c.d_lut;
-        fp.cancel = c.d_cancel;
-        fp.rgb = rgb ? root.d_rgb : nullptr;
-        fp.argb = argb ? root.d_argb : nullptr;
-        const uint32_t tile_rows = (H + TILE_H - 1) / TILE_H;
-        const uint32_t n_chunks = tile_rows >= 32 ? 4 : 1;
-        CU(cudaEventRecord(c.e0, c.stream));
-        for (uint32_t k = 0; k < n_chunks; k++) {
-            const uint32_t t0 = tile_rows * k / n_chunks, t1 = tile_rows * (k + 1) / n_chunks;
-            fp.tile_row0 = t0;
-            CU(launch_frame(fp, s->mode, t1 - t0, c.stream));
-            launches++;
-            CU(cudaEventRecord(c.chunk_done[k], c.stream));
-            CU(cudaStreamWaitEvent(c.copy_stream, c.chunk_done[k], 0));
-            const size_t y0 = (size_t)t0 * TILE_H, y1 = std::min<size_t>((size_t)t1 * TILE_H, H);
-            if (rgb)
-                CU(cudaMemcpyAsync(rgb + y0 * W * 3, root.d_rgb + y0 * W * 3, (y1 - y0) * W * 3 * sizeof(float), cudaMemcpyDeviceToHost,
-                                   c.copy_stream));
-            if (argb)
-                CU(cudaMemcpyAsync(argb + y0 * W, root.d_argb + y0 * W, (y1 - y0) * W * sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                                   c.copy_stream));
-        }
-        CU(cudaEventRecord(c.e1, c.stream));
-        CU(cudaStreamSynchronize(c.copy_stream));
-        copied = true;
+    double kernel_ms = 0;
+    for (int i = 0; i < n; i++) {
+        if (rcs[i]) { g_err = errs[i]; return rcs[i]; }
+        launches += ls[i];
+        if (kms[i] > kernel_ms) kernel_ms = kms[i];
     }
-    // N devices.  Default: every device renders its interleaved bands into a compact buffer and copies them to
-    // the caller's HOST frame over its own PCIe link (chunked, overlapped with rendering) — the host copy of a
-    // float frame is the slow part, so N links beat one.  C2RT_GATHER=root keeps the frame on device 0 instead:
-    // peers store their bands straight into it through peer-mapped pointers (NVLink), device 0 copies it back.
-    const char* gather_env = getenv("C2RT_GATHER");
-    const bool direct = n > 1 && !(gather_env && strcmp(gather_env, "root") == 0);
-    if (direct) {
-        // scene residency first, on this thread: make_resident patches the shared host copy of the scene block per device
-        for (int i = 0; i < n; i++) {
-            if (g_ctx.d[i].uploaded_scene == s->id) continue;
-            CU(cudaSetDevice(g_ctx.d[i].dev));
-            rc = make_resident(s, i, g_ctx.d[i].stream);
-            if (rc) return rc;
-        }
-        // one host thread per device (DevicePool): worker w drives device w + 1, this thread drives device 0
-        int rcs[C2RT_MAX_GPUS] = {};
-        uint32_t ls[C2RT_MAX_GPUS] = {};
-        float kms[C2RT_MAX_GPUS] = {};
-        std::string errs[C2RT_MAX_GPUS];
-        const bool pooled = g_pool.size() == n - 1;
-        if (pooled)
-            g_pool.run([&](int w) {
-                rcs[w + 1] = render_direct_device(w + 1, n, s, cam, set, rgb, argb, &ls[w + 1], &kms[w + 1]);
-                if (rcs[w + 1]) errs[w + 1] = g_err;
-            });
-        else
-            for (int i = 1; i < n; i++) {
-                rcs[i] = render_direct_device(i, n, s, cam, set, rgb, argb, &ls[i], &kms[i]);
-                if (rcs[i]) errs[i] = g_err;
-            }
-        rcs[0] = render_direct_device(0, n, s, cam, set, rgb, argb, &ls[0], &kms[0]);
-        if (rcs[0]) errs[0] = g_err;
-        if (pooled) g_pool.wait();
-        for (int i = 0; i < n; i++) {
-            if (rcs[i]) { g_err = errs[i]; return rcs[i]; }
-            launches += ls[i];
-            if (kms[i] > direct_kernel_ms) direct_kernel_ms = kms[i];
-        }
-        copied = true;
-    }
-    for (int i = 0; i < n && n > 1 && !direct; i++) {
-        DeviceCtx& c = g_ctx.d[i];
-        CU(cudaSetDevice(c.dev));
-        rc = make_resident(s, i, c.stream);
-        if (rc) return rc;
-        FrameParams fp;
-        fill_params(fp, cam, set, s, i);
-        fp.rank = (uint32_t)i;
-        fp.n_ranks = (uint32_t)n;
-        fp.tiles_per_band = band_rows / TILE_H;
-        fp.counters = c.d_counters;
-        fp.lut = c.d_lut;
-        fp.cancel = c.d_cancel;
-        const uint32_t rows_owned = c2rt_band_rows_owned(H, fp.rank, fp.n_ranks, band_rows);
-        if (i == 0 || c.peer_to_root) {
-            // bands land directly in the root frame (peer-mapped stores over NVLink for i > 0)
-            fp.compact = 0;
-            fp.rgb = rgb ? root.d_rgb : nullptr;
-            fp.argb = argb ? root.d_argb : nullptr;
-        } else {
-            fp.compact = 1;
-            size_t need = (size_t)rows_owned * W;
-            if (rgb && c.rgb_cap < need * 3) {
-                cudaFree(c.d_rgb);
-                c.d_rgb = nullptr; c.rgb_cap = 0;
-                CU(cudaMalloc(&c.d_rgb, need * 3 * sizeof(float)));
-                c.rgb_cap = need * 3;
-            }
-            if (argb && c.argb_cap < need) {
-                cudaFree(c.d_argb);
-                c.d_argb = nullptr; c.argb_cap = 0;
-                CU(cudaMalloc(&c.d_argb, need * sizeof(uint32_t)));
-                c.argb_cap = need;
-            }
-            fp.rgb = rgb ? c.d_rgb : nullptr;
-            fp.argb = argb ? c.d_argb : nullptr;
-        }
-        CU(cudaEventRecord(c.e0, c.stream));
-        CU(launch_frame(fp, s->mode, local_tile_rows(H, fp.rank, fp.n_ranks, band_rows), c.stream));
-        CU(cudaEventRecord(c.e1, c.stream));
-        launches++;
-        if (i > 0 && !c.peer_to_root) {
-            // no P2P mapping: copy each band into the root frame
-            uint32_t local = 0;
-            for (uint32_t y0 = fp.rank * band_rows; y0 < H; y0 += n * band_rows, local += band_rows) {
-                uint32_t rows = (H - y0 < band_rows) ? H - y0 : band_rows;
-                if (rgb)
-                    CU(cudaMemcpyPeerAsync(root.d_rgb + (size_t)y0 * W * 3, root.dev, c.d_rgb + (size_t)local * W * 3, c.dev,
-                                           (size_t)rows * W * 3 * sizeof(float), c.stream));
-                if (argb)
-                    CU(cudaMemcpyPeerAsync(root.d_argb + (size_t)y0 * W, root.dev, c.d_argb + (size_t)local * W, c.dev,
-                                           (size_t)rows * W * sizeof(uint32_t), c.stream));
-            }
-        }
-    }
-    double kernel_ms = direct_kernel_ms;
-    for (int i = 0; i < n && !direct; i++) {
-        DeviceCtx& c = g_ctx.d[i];
-        CU(cudaSetDevice(c.dev));
-        CU(cudaStreamSynchronize(c.stream));
-        float ms = 0;
-        CU(cudaEventElapsedTime(&ms, c.e0, c.e1));
-        if (ms > kernel_ms) kernel_ms = ms;
-    }
-    CU(cudaSetDevice(root.dev));
-    if (!copied) {
-        if (rgb) CU(cudaMemcpyAsync(rgb, root.d_rgb, npx * 3 * sizeof(float), cudaMemcpyDeviceToHost, root.stream));
-        if (argb) CU(cudaMemcpyAsync(argb, root.d_argb, npx * sizeof(uint32_t), cudaMemcpyDeviceToHost, root.stream));
-        CU(cudaStreamSynchronize(root.stream));
-    }
+    CU(cudaSetDevice(g_ctx.d[0].dev));
     if (stats) {
         memset(stats, 0, sizeof *stats);
         stats->kernel_ms = kernel_ms;
@@ -1271,7 +1126,7 @@ int c2rt_render(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set,
                 stats->primary_rays += v[0];
                 stats->shadow_rays += v[1];
             }
-            CU(cudaSetDevice(root.dev));
+            CU(cudaSetDevice(g_ctx.d[0].dev));
         }
         stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     }

@@ -208,10 +208,9 @@ typedef struct c2rt_scene c2rt_scene;
 
 /* Library lifetime.  device_ids == NULL -> devices 0..n_gpus-1.  With n_gpus > 1 c2rt_render splits
  * the frame into interleaved row bands; every device copies its bands to the caller's host frame over
- * its own PCIe link (C2RT_GATHER=root: the frame lives on device_ids[0] and the other devices store
- * their bands straight into it through peer-mapped pointers, NVLink P2P).  The library then owns
- * n_gpus - 1 helper threads (one per extra device, idle between frames; joined by c2rt_shutdown or the
- * next c2rt_init).  Calling c2rt_init again re-initialises. */
+ * its own PCIe link.  The library then owns n_gpus - 1 helper threads (one per extra device, idle
+ * between frames; joined by c2rt_shutdown or the next c2rt_init).  Calling c2rt_init again
+ * re-initialises. */
 int c2rt_init(int n_gpus, const int* device_ids);
 void c2rt_shutdown(void);
 int c2rt_abi_version(void);
