@@ -25,23 +25,15 @@
 namespace c2rt {
 cudaError_t upload_scene(const DevScene& s, cudaStream_t st);
 cudaError_t launch_frame(const FrameParams& fp, int mode, uint32_t local_tile_rows, cudaStream_t st);
-cudaError_t launch_pixel(const FrameParams& fp, int mode, int x, int y, void* d_out, cudaStream_t st);
+cudaError_t launch_pixel(const FrameParams& fp, int mode, int x, int y, PixelOut* d_out, cudaStream_t st);
 cudaError_t launch_deinterleave(const void* src, void* dst, uint32_t row_words, uint32_t height, uint32_t n_ranks,
                                 uint32_t band_rows, uint32_t rows_pad, cudaStream_t st);
 cudaError_t launch_fma_peak(bool fp64, int blocks, int threads, int iters, void* d_out, cudaStream_t st);
 cudaError_t launch_gate(void* gate, uint32_t round, uint32_t n_ranks, void* err, cudaStream_t st);
 cudaError_t launch_signal(void* flag, uint32_t frame_no, cudaStream_t st);
-size_t pixel_out_size();
 }  // namespace c2rt
 
 using namespace c2rt;
-
-// must match PixelOut in render_kernel.cu
-struct PixelOutHost {
-    float rgb[3];
-    int node;
-    double dist, p[3], n[3], u, v;
-};
 
 namespace {
 
@@ -70,11 +62,11 @@ struct DeviceCtx {
     std::vector<cudaEvent_t> band_done;
     uint64_t uploaded_scene = 0;   // id of the scene currently in this device's constant memory
     unsigned long long* d_counters = nullptr;
-    uint32_t* d_sync = nullptr;    // [0] CTAs of the current launch that finished (in-kernel completion)
+    uint32_t* d_done_counter = nullptr;   // CTAs of the current launch that finished (in-kernel completion)
     int* d_cancel = nullptr;       // raised by c2rt_cancel, cleared at the start of every c2rt_render
     cudaStream_t cancel_stream = nullptr;
     uint8_t* d_lut = nullptr;
-    void* d_pixel = nullptr;
+    PixelOut* d_pixel = nullptr;
     float* d_rgb = nullptr;
     uint32_t* d_argb = nullptr;
     size_t rgb_cap = 0, argb_cap = 0;
@@ -186,7 +178,7 @@ void destroy_device(DeviceCtx& c) {
     if (c.e0) cudaEventDestroy(c.e0);
     if (c.e1) cudaEventDestroy(c.e1);
     cudaFree(c.d_counters);
-    cudaFree(c.d_sync);
+    cudaFree(c.d_done_counter);
     cudaFree(c.d_cancel);
     if (c.cancel_stream) cudaStreamDestroy(c.cancel_stream);
     cudaFree(c.d_lut);
@@ -219,14 +211,14 @@ int init_locked(int n_gpus, const int* ids) {
         CU(cudaEventCreate(&c.e1));
         CU(cudaMalloc(&c.d_counters, 2 * sizeof(unsigned long long)));
         CU(cudaMemset(c.d_counters, 0, 2 * sizeof(unsigned long long)));
-        CU(cudaMalloc(&c.d_sync, 2 * sizeof(uint32_t)));
-        CU(cudaMemset(c.d_sync, 0, 2 * sizeof(uint32_t)));
+        CU(cudaMalloc(&c.d_done_counter, sizeof(uint32_t)));
+        CU(cudaMemset(c.d_done_counter, 0, sizeof(uint32_t)));
         CU(cudaMalloc(&c.d_cancel, sizeof(int)));
         CU(cudaMemset(c.d_cancel, 0, sizeof(int)));
         CU(cudaStreamCreateWithFlags(&c.cancel_stream, cudaStreamNonBlocking));
         CU(cudaMalloc(&c.d_lut, 4097));
         CU(cudaMemcpy(c.d_lut, g_ctx.lut, 4097, cudaMemcpyHostToDevice));
-        CU(cudaMalloc(&c.d_pixel, pixel_out_size()));
+        CU(cudaMalloc(&c.d_pixel, sizeof(PixelOut)));
         g_ctx.n = i + 1;
     }
     cudaSetDevice(g_ctx.d[0].dev);
@@ -432,13 +424,13 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
             if (l < 0 || r < 0 || l >= (int)i || r >= (int)i)
                 return fail(C2RT_ERR_INVALID_ARG, "geometry %u: CSG children must be earlier geometries (left %d, right %d)", i, l, r);
             g.left = l; g.right = r;
-            const int dl = abs(s->geoms[l].pad), dr = abs(s->geoms[r].pad);
-            g.pad = 1 + (dl > dr ? dl : dr);
-            if (g.pad > 3)
+            const int dl = abs(s->geoms[l].depth), dr = abs(s->geoms[r].depth);
+            g.depth = 1 + (dl > dr ? dl : dr);
+            if (g.depth > 3)
                 return fail(C2RT_ERR_UNSUPPORTED, "geometry %u: CSG nesting deeper than 3 levels is not supported", i);
             // tuning / testing aid: C2RT_CSG_LITERAL=1 routes every CSG through the literal emulation
             const char* lit = getenv("C2RT_CSG_LITERAL");
-            if (lit && lit[0] == '1' && g.pad == 1) g.pad = -1;
+            if (lit && lit[0] == '1' && g.depth == 1) g.depth = -1;
         }
     }
     s->tex_offset.assign(d->n_textures + 6, 0);     // + 6: the environment faces
@@ -587,10 +579,11 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
     }
     s->mode = 0;
     for (uint32_t i = 0; i < d->n_nodes; i++) {
-        if (!(s->nodes[i].flags & NODE_UNBOUNDED)) s->mode |= 1;   // MODE_BOUNDED
-        if (s->nodes[i].kind == KIND_GENERIC) s->mode |= 2;        // MODE_GENERIC
+        if (!(s->nodes[i].flags & NODE_UNBOUNDED)) s->mode |= MODE_BOUNDED;
+        if (s->nodes[i].kind == KIND_GENERIC) s->mode |= MODE_GENERIC;
         const DevGeom& ng = s->geoms[s->nodes[i].geom];
-        if (ng.type >= C2RT_GEOM_CSG_UNION && ng.pad != 1) s->mode |= 4 | 2 | 1;  // MODE_NESTED (implies the generic, bounded kernel)
+        // (MODE_NESTED implies the generic, bounded kernel)
+        if (ng.type >= C2RT_GEOM_CSG_UNION && ng.depth != 1) s->mode |= MODE_NESTED | MODE_GENERIC | MODE_BOUNDED;
     }
     // MODE_SOLO: exactly one node, a world-space plane, and exactly one light.  The node's shader and that shader's
     // texture are swapped into record 0 so the kernel addresses every scene constant statically.
@@ -736,7 +729,6 @@ void fill_params(FrameParams& fp, const c2rt_camera* cam, const c2rt_settings* s
         for (int k = 0; k < 3; k++) fp.tap_d[t][k] = fp.du[k] * (kx[t] * fp.inv_w) + fp.dv[k] * (ky[t] * fp.inv_h);
     fp.focal_plane_dist = cam->focal_plane_dist;
     fp.disc_multiplier = cam->disc_multiplier;
-    fp.disc_multiplier_f = (float)cam->disc_multiplier;
     fp.stereo_sep = cam->stereo_separation;
     fp.seed = set->rng_seed;
     fp.W = set->frame_width;
@@ -744,16 +736,13 @@ void fill_params(FrameParams& fp, const c2rt_camera* cam, const c2rt_settings* s
     fp.aa = set->aa_enabled != 0;
     fp.dof = cam->dof != 0;
     fp.num_samples = cam->num_samples;
-    fp.max_trace_depth = set->max_trace_depth;
     fp.count_rays = set->count_rays != 0;
     // GI frame (renderer.d:289-301,378-463): every path returns exactly black — PointLight.solidAngle is 0 (light.d:72-75) so
     // resultDirect is 0, lights cannot be hit, misses read the black environment — and the pixel is the mean of pathsPerPixel zeros
     fp.gi = set->gi_enabled && !cam->dof;
     fp.gi_fill = set->paths_per_pixel ? 0.f : nanf("");
     fp.prepass_bucket = set->prepass_only ? (set->bucket_size ? set->bucket_size : 48u) : 0u;
-    fp.n_ranks = 1;
-    fp.tiles_per_band = 1;
-    if (s->mode & MODE_SOLO) {   // render_kernel.cu isect_plane_solo
+    if (s->mode & MODE_SOLO) {   // render_kernel.cu solo_plane_test
         const double y = s->nodes[0].wp[0], h = cam->pos[1] - y, ly = s->host.lights[0].pos[1];
         fp.solo_side = h > 0 ? 1 : h < 0 ? -1 : 0;
         fp.solo_sign = fp.solo_side > 0 ? 0x80000000u : 0u;
@@ -805,6 +794,29 @@ void fill_params(FrameParams& fp, const c2rt_camera* cam, const c2rt_settings* s
         // camera's roll: the corners reach the ABI from any host.
         fp.solo_rows = fp.solo_fast && fp.du[1] == 0.0;
     }
+}
+
+// The band layout of a launch (c2rt.h c2rt_band: rows in bands of band_rows, band b on rank b % n_ranks; compact outputs hold
+// only this rank's rows) and the device's ray counters and sRGB table
+void set_bands(FrameParams& fp, const DeviceCtx& c, uint32_t rank, uint32_t n_ranks, uint32_t band_rows, bool compact) {
+    fp.rank = rank;
+    fp.n_ranks = n_ranks;
+    fp.tiles_per_band = band_rows / TILE_H;
+    fp.compact = compact;
+    fp.counters = c.d_counters;
+    fp.lut = c.d_lut;
+}
+
+// Reads a device's ray counters behind the work already on `st` (either output may be null) and zeroes them for the next
+// frame.  The caller has made c.dev the current device.
+int take_ray_counters(const DeviceCtx& c, cudaStream_t st, uint64_t* primary, uint64_t* shadow) {
+    unsigned long long v[2];
+    CU(cudaMemcpyAsync(v, c.d_counters, sizeof v, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemsetAsync(c.d_counters, 0, sizeof v, st));
+    CU(cudaStreamSynchronize(st));
+    if (primary) *primary = v[0];
+    if (shadow) *shadow = v[1];
+    return C2RT_OK;
 }
 
 // c2rt_cancel bookkeeping: true iff a cancel was requested since the last call; the device flags are lowered again
@@ -862,12 +874,7 @@ int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt
     CU(cudaSetDevice(c.dev));
     FrameParams fp;
     fill_params(fp, cam, set, s, i);
-    fp.rank = (uint32_t)i;
-    fp.n_ranks = (uint32_t)n;
-    fp.tiles_per_band = brows / TILE_H;
-    fp.compact = 1;
-    fp.counters = c.d_counters;
-    fp.lut = c.d_lut;
+    set_bands(fp, c, (uint32_t)i, (uint32_t)n, brows, true);
     fp.cancel = c.d_cancel;
     const size_t need = (size_t)c2rt_band_rows_owned(H, fp.rank, fp.n_ranks, brows) * W;
     int rc = rgb ? grow_buffer(c.d_rgb, c.rgb_cap, need * 3) : C2RT_OK;
@@ -942,17 +949,7 @@ uint32_t c2rt_band_rows_owned(uint32_t height, uint32_t rank, uint32_t n_ranks, 
 }
 
 uint32_t c2rt_rng_u31(uint64_t seed, uint32_t px, uint32_t py, uint32_t tap, uint32_t sample, uint32_t draw) {
-    // counter-based: four rounds of the 32-bit "lowbias32" finaliser over (seed, pixel) / (tap, sample) / draw.
-    // The pixel and sample rounds do not depend on `draw`, so a compiler hoists them out of the draw sequence.
-    uint32_t h = (uint32_t)seed ^ ((uint32_t)(seed >> 32) * 0x9E3779B9u) ^ (px * 0x85EBCA6Bu);
-    h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
-    h ^= py * 0xC2B2AE35u;
-    h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
-    h ^= tap * 0x27D4EB2Fu + sample * 0x165667B1u;
-    h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
-    h += draw * 0x9E3779B9u;
-    h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
-    return h >> 1;
+    return rng_u31(seed, px, py, tap, sample, draw);   // the kernel's generator (scene_dev.h)
 }
 
 void c2rt_srgb_table(uint8_t out[4097]) {
@@ -1012,36 +1009,29 @@ int c2rt_render_device(c2rt_scene* s, const c2rt_camera* cam, const c2rt_setting
     cudaStream_t st = (cudaStream_t)stream;
     rc = make_resident(s, di, st);
     if (rc) return rc;
+    const c2rt_band whole = {0, 1, TILE_H, 0, nullptr, 0, 0};   // no band: the whole frame on one rank
+    const c2rt_band& b = band ? *band : whole;
+    if (b.n_ranks == 0 || b.rank >= b.n_ranks || b.band_rows == 0 || b.band_rows % TILE_H != 0)
+        return fail(C2RT_ERR_INVALID_ARG, "bad band (rank %u of %u, band_rows %u; band_rows must be a multiple of %d)", b.rank,
+                    b.n_ranks, b.band_rows, TILE_H);
     FrameParams fp;
     fill_params(fp, cam, set, s, di);
-    uint32_t band_rows = TILE_H;
-    if (band) {
-        if (band->n_ranks == 0 || band->rank >= band->n_ranks || band->band_rows == 0 || band->band_rows % TILE_H != 0)
-            return fail(C2RT_ERR_INVALID_ARG, "bad band (rank %u of %u, band_rows %u; band_rows must be a multiple of %d)", band->rank,
-                        band->n_ranks, band->band_rows, TILE_H);
-        fp.rank = band->rank;
-        fp.n_ranks = band->n_ranks;
-        fp.compact = band->compact != 0;
-        band_rows = band->band_rows;
-        if (band->done_flags) {
-            if (band->n_ranks > 32) return fail(C2RT_ERR_INVALID_ARG, "done_flags: at most 32 ranks");
-            fp.frame_no = band->frame_no;
-            if (band->rank == 0) {   // rank 0 waits inside its kernel; peers signal behind theirs (below)
-                fp.done_flags = (uint32_t*)band->done_flags;
-                fp.done_counter = c->d_sync;
-            }
+    set_bands(fp, *c, b.rank, b.n_ranks, b.band_rows, b.compact != 0);
+    if (b.done_flags) {
+        if (b.n_ranks > 32) return fail(C2RT_ERR_INVALID_ARG, "done_flags: at most 32 ranks");
+        fp.frame_no = b.frame_no;
+        if (b.rank == 0) {   // rank 0 waits inside its kernel; peers signal behind theirs (below)
+            fp.done_flags = (uint32_t*)b.done_flags;
+            fp.done_counter = c->d_done_counter;
         }
     }
     if (((uintptr_t)d_rgb & 15u) && (fp.W & 3u) == 0)
         return fail(C2RT_ERR_INVALID_ARG, "d_rgb must be 16-byte aligned when the frame width is a multiple of 4 (float4 band stores)");
-    fp.tiles_per_band = band_rows / TILE_H;
     fp.rgb = d_rgb;
     fp.argb = d_argb;
-    fp.counters = c->d_counters;
-    fp.lut = c->d_lut;
-    CU(launch_frame(fp, s->mode, local_tile_rows(fp.H, fp.rank, fp.n_ranks, band_rows), st));
-    const bool signals = band && band->done_flags && band->rank != 0;
-    if (signals) CU(launch_signal((uint32_t*)band->done_flags + band->rank, band->frame_no, st));
+    CU(launch_frame(fp, s->mode, local_tile_rows(fp.H, b.rank, b.n_ranks, b.band_rows), st));
+    const bool signals = b.done_flags && b.rank != 0;
+    if (signals) CU(launch_signal((uint32_t*)b.done_flags + b.rank, b.frame_no, st));
     if (stats) {
         memset(stats, 0, sizeof *stats);
         stats->n_gpus = 1;
@@ -1057,14 +1047,7 @@ int c2rt_read_ray_counters(c2rt_scene*, void* stream, uint64_t* primary, uint64_
     CU(cudaGetDevice(&dev));
     DeviceCtx* c = find_device(dev);
     if (!c) return fail(C2RT_ERR_INVALID_ARG, "current device %d is not part of the c2rt context", dev);
-    cudaStream_t st = (cudaStream_t)stream;
-    unsigned long long v[2];
-    CU(cudaMemcpyAsync(v, c->d_counters, sizeof v, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemsetAsync(c->d_counters, 0, sizeof v, st));
-    CU(cudaStreamSynchronize(st));
-    if (primary) *primary = v[0];
-    if (shadow) *shadow = v[1];
-    return C2RT_OK;
+    return take_ray_counters(*c, (cudaStream_t)stream, primary, shadow);
 }
 
 int c2rt_render(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb, c2rt_stats* stats) {
@@ -1120,11 +1103,11 @@ int c2rt_render(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set,
             for (int i = 0; i < n; i++) {
                 DeviceCtx& c = g_ctx.d[i];
                 CU(cudaSetDevice(c.dev));
-                unsigned long long v[2];
-                CU(cudaMemcpy(v, c.d_counters, sizeof v, cudaMemcpyDeviceToHost));
-                CU(cudaMemset(c.d_counters, 0, sizeof v));
-                stats->primary_rays += v[0];
-                stats->shadow_rays += v[1];
+                uint64_t p, sh;
+                rc = take_ray_counters(c, c.stream, &p, &sh);
+                if (rc) return rc;
+                stats->primary_rays += p;
+                stats->shadow_rays += sh;
             }
             CU(cudaSetDevice(g_ctx.d[0].dev));
         }
@@ -1171,12 +1154,10 @@ int c2rt_render_pixel(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings
     if (rc) return rc;
     FrameParams fp;
     fill_params(fp, cam, set, s, 0);
-    fp.counters = c.d_counters;
-    fp.lut = c.d_lut;
+    set_bands(fp, c, 0, 1, TILE_H, false);
     fp.count_rays = 0;
     CU(launch_pixel(fp, s->mode, x, y, c.d_pixel, c.stream));
-    PixelOutHost o;
-    if (pixel_out_size() != sizeof o) return fail(C2RT_ERR_CUDA, "internal: PixelOut layout mismatch");
+    PixelOut o;
     CU(cudaMemcpyAsync(&o, c.d_pixel, sizeof o, cudaMemcpyDeviceToHost, c.stream));
     CU(cudaStreamSynchronize(c.stream));
     rgb[0] = o.rgb[0]; rgb[1] = o.rgb[1]; rgb[2] = o.rgb[2];

@@ -37,7 +37,7 @@ struct DevNode {
 struct DevGeom {
     double p[4];      // plane: y, limit | sphere: c.xyz, R | cube: c.xyz, side
     int type, left, right;
-    int pad;          // CSG depth: 0 primitive, 1 CSG of primitives, >1 nested (or forced literal: -1)
+    int depth;        // CSG depth: 0 primitive, 1 CSG of primitives, >1 nested (or forced literal: -1)
 };
 
 struct DevShader {
@@ -95,12 +95,14 @@ struct FrameParams {
     double inv_w, inv_h;
     double tap_d[5][3];               // ray-direction offset of AA tap k: du * kx/W + dv * ky/H (renderer.d:235-247)
     double focal_plane_dist, disc_multiplier;
-    float disc_multiplier_f, pad_disc;   // FP32 copy (the lens sample, render_kernel.cu gen_ray)
     double stereo_sep;                // camera.stereoSeparation (0 = off)
     unsigned long long seed;
     uint32_t W, H;                    // output size
     int aa, dof;
-    uint32_t num_samples, max_trace_depth;
+    uint32_t num_samples;
+    // frame number of the done_flags signalling (below).  It sits here so that every 4-byte field keeps its offset mod 8:
+    // ptxas reads adjacent 8-byte-aligned pairs of them with one 64-bit constant load (LDC.64 / LDCU.64)
+    uint32_t frame_no;
     float ambient[3];
     int count_rays;
     uint32_t prepass_bucket;          // > 0: prepassOnly frame (16x16-block preview inside buckets of this size)
@@ -108,15 +110,14 @@ struct FrameParams {
     float gi_fill;
     // interleaved row bands
     uint32_t rank, n_ranks, tiles_per_band, compact;
-    uint32_t tile_row0;               // first local tile row of this launch (frames are launched in chunks to overlap the D2H copy)
+    uint32_t tile_row0;               // first local tile row of this launch (one launch per band, c2rt_api.cu render_bands)
     // per-node bounding spheres (x, y, z, radius; radius < 0: unbounded) in GLOBAL memory for the per-warp node masks, whose
     // lanes each test a different node (render_kernel.cu camera_mask / shadow_mask)
     const float4* bounds;
     // frame-complete signalling folded into the kernel (render_frame_kernel epilogue); done_flags == nullptr: off
     uint32_t* done_flags;             // in rank 0's memory: [r] = last frame number rank r completed, [n_ranks] = wait time-outs
     uint32_t* done_counter;           // this device: CTAs of the current launch that have finished
-    uint32_t frame_no, pad_frame;
-    // MODE_SOLO frames (render_kernel.cu isect_plane_solo): solo_fast = the frame is regular (camera — the whole lens under
+    // MODE_SOLO frames (render_kernel.cu solo_plane_test): solo_fast = the frame is regular (camera — the whole lens under
     // DOF / stereo — off the plane, light on the camera's side, moderate magnitudes: c2rt_api.cu fill_params); the kernels
     // without the sampling loop only run such frames, the sampling kernels branch on it.  Then: side of the plane the camera is
     // on (+1 above, -1 below), the sign bit a ray's d.y must NOT have xor'ed in (0x80000000 above the plane: d.y must be
@@ -157,29 +158,42 @@ constexpr bool plane_only(int mode) { return (mode & (MODE_BOUNDED | MODE_GENERI
 
 // Scene classes whose rays go through per-warp node masks (render_kernel.cu camera_mask / shadow_mask): every scene class
 // but the plane-only ones.  Camera rays get a mask only when they all start at the camera position (no DOF / stereo
-// sampling loop); shadow rays always do.  -DC2RT_NO_WARP_MASK builds the kernels with all-node masks (A/B tuning aid).
+// sampling loop); shadow rays always do.
 #ifdef __CUDACC__
 __host__ __device__
 #endif
-constexpr bool camera_masked(int mode) {
-#ifdef C2RT_NO_WARP_MASK
-    return false && mode;
-#else
-    return !plane_only(mode) && !(mode & MODE_SAMPLING);
-#endif
-}
+constexpr bool camera_masked(int mode) { return !plane_only(mode) && !(mode & MODE_SAMPLING); }
 
-// CTA tile: 4 warps of 8x4 pixels each.  16x8 (2x2 warps) by default; -DC2RT_TILE_W=32 -DC2RT_TILE_H=4 lays the warps side by
-// side (384 contiguous bytes per tile row instead of 192: tuning aid for the NVLink band stores, profiles/r2_tile_shape.log)
-#ifndef C2RT_TILE_W
-#define C2RT_TILE_W 16
-#endif
-#ifndef C2RT_TILE_H
-#define C2RT_TILE_H 8
-#endif
-constexpr int TILE_W = C2RT_TILE_W;
-constexpr int TILE_H = C2RT_TILE_H;
+// CTA tile: 4 warps of 8x4 pixels each, 2x2 warps (32x4 was measured and not kept: profiles/r2_tile_shape.log)
+constexpr int TILE_W = 16;
+constexpr int TILE_H = 8;
 static_assert(TILE_W % 8 == 0 && TILE_H % 4 == 0 && TILE_W * TILE_H == 128, "a CTA tile is four 8x4 warp patches");
 constexpr int BLOCK_THREADS = TILE_W * TILE_H;
+
+// The pinned RNG of DOF sampling (c2rt.h c2rt_rng_u31): the kernel's lens samples and the exported function are this one
+// definition; the oracle keeps an independent copy (oracle/orc_scene.hpp rng_u31) that the tests compare it with.
+// Counter-based: four rounds of the 32-bit "lowbias32" finaliser over (seed, pixel) / (tap, sample) / draw.
+// The pixel and sample rounds do not depend on `draw`, so a compiler hoists them out of the draw sequence.
+#ifdef __CUDACC__
+__host__ __device__ __forceinline__
+#endif
+constexpr uint32_t rng_u31(uint64_t seed, uint32_t px, uint32_t py, uint32_t tap, uint32_t sample, uint32_t draw) {
+    uint32_t h = (uint32_t)seed ^ ((uint32_t)(seed >> 32) * 0x9E3779B9u) ^ (px * 0x85EBCA6Bu);
+    h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
+    h ^= py * 0xC2B2AE35u;
+    h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
+    h ^= tap * 0x27D4EB2Fu + sample * 0x165667B1u;
+    h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
+    h += draw * 0x9E3779B9u;
+    h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
+    return h >> 1;
+}
+
+// renderer.d:46-57 renderPixel: what render_pixel_kernel writes for c2rt_render_pixel
+struct PixelOut {
+    float rgb[3];
+    int node;
+    double dist, p[3], n[3], u, v;
+};
 
 }  // namespace c2rt

@@ -178,7 +178,7 @@ def test_palette_quad_bitmaps_equal_float4_texels(name, size, over, monkeypatch)
                                             ("zaphod.sdl", (161, 107), {"num_samples": 3})])   # DOF: the whole lens is checked
 def test_regular_one_plane_frames_equal_the_general_kernel(name, size, over, monkeypatch):
     """One-plane frames with a fixed camera off the plane and the light on its side run on kernels that take the camera's
-    side, its height and 'the plane cannot shadow itself' as frame constants (render_kernel.cu isect_plane_solo, c2rt_api.cu
+    side, its height and 'the plane cannot shadow itself' as frame constants (render_kernel.cu solo_plane_test, c2rt_api.cu
     fill_params).  Those are shortcuts, not approximations: the frame must be BIT-identical to the one the general kernel of
     the scene class renders (C2RT_NO_SOLO_FAST=1, read per frame), ray counts included."""
     g = c2.HostScene(os.path.join(SC, name))
