@@ -8,8 +8,8 @@ any attribute of :mod:`chess2rt_b200.api` raises if the libraries have not been 
 (``python -m chess2rt_b200.build``).
 """
 _API_NAMES = (
-    "C2rtError", "HostScene", "Stats", "band_rows_owned", "device_count", "init", "lib", "host_lib", "render_device",
-    "read_ray_counters", "deinterleave", "measure_fma_peak", "srgb_table", "rng_u31", "shutdown",
+    "C2rtError", "HostScene", "HitPlanes", "Stats", "band_rows_owned", "device_count", "init", "lib", "host_lib", "render_device",
+    "render_hits_device", "read_ray_counters", "deinterleave", "measure_fma_peak", "srgb_table", "rng_u31", "shutdown",
 )
 
 

@@ -57,6 +57,10 @@ class Hit(C.Structure):
                 ("normal", C.c_double * 3), ("u", C.c_double), ("v", C.c_double)]
 
 
+class HitPlanes(C.Structure):
+    _fields_ = [("node", C.c_void_p), ("dist", C.c_void_p), ("normal", C.c_void_p), ("uv", C.c_void_p)]
+
+
 class SceneDesc(C.Structure):
     _fields_ = [
         ("struct_size", C.c_uint32), ("abi_version", C.c_uint32),
@@ -82,7 +86,7 @@ class SceneDesc(C.Structure):
 C_ABI_SYMBOLS = [
     "c2rt_init", "c2rt_shutdown", "c2rt_abi_version", "c2rt_device_count", "c2rt_last_error",
     "c2rt_scene_create", "c2rt_scene_destroy", "c2rt_render", "c2rt_cancel", "c2rt_render_device", "c2rt_read_ray_counters",
-    "c2rt_deinterleave", "c2rt_render_pixel", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
+    "c2rt_deinterleave", "c2rt_render_pixel", "c2rt_render_hits", "c2rt_render_hits_device", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
     "c2rt_frame_alloc", "c2rt_frame_free", "c2rt_frame_export", "c2rt_frame_import", "c2rt_frame_unimport", "c2rt_frame_memset", "c2rt_frame_download", "c2rt_pin_host_buffer", "c2rt_unpin_host_buffer", "c2rt_gate",
     "c2rt_measure_fma_peak", "c2rt_selftest_device_pool",
 ]
@@ -102,6 +106,9 @@ lib.c2rt_deinterleave.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32
                                   C.c_uint32, C.c_void_p]
 lib.c2rt_render_pixel.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.c_int, C.c_int,
                                   C.POINTER(C.c_float), C.POINTER(Hit)]
+lib.c2rt_render_hits.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.POINTER(HitPlanes), C.POINTER(Stats)]
+lib.c2rt_render_hits_device.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.POINTER(Band), C.POINTER(HitPlanes),
+                                        C.c_void_p, C.POINTER(Stats)]
 lib.c2rt_band_rows_owned.argtypes = [C.c_uint32] * 4
 lib.c2rt_band_rows_owned.restype = C.c_uint32
 lib.c2rt_rng_u31.argtypes = [C.c_uint64] + [C.c_uint32] * 5
@@ -139,6 +146,7 @@ host_lib.c2rt_host_device_scene.argtypes = [C.c_void_p]
 host_lib.c2rt_host_device_scene.restype = C.c_void_p
 host_lib.c2rt_host_render.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.POINTER(Stats)]
 host_lib.c2rt_host_render_pixel.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(Hit)]
+host_lib.c2rt_host_render_hits.argtypes = [C.c_void_p, C.POINTER(HitPlanes), C.c_uint64, C.POINTER(Stats)]
 host_lib.c2rt_host_camera_rotate.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_double]
 host_lib.c2rt_host_camera_rotate.restype = None
 host_lib.c2rt_host_camera_move.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_double]
@@ -276,6 +284,24 @@ class HostScene:
         return np.array(list(rgb), np.float32), hit
 
 
+    def render_hits(self, planes=("node", "dist", "normal", "uv"), seed=0):
+        """renderPixel's hit record for every pixel (c2rt_render_hits) -> ({plane: array}, Stats).  Planes: node [H, W] int32
+        (-1 = miss), dist [H, W] float32 (+inf for a miss), normal [H, W, 3] and uv [H, W, 2] float32 (0 for a miss)."""
+        w, h = self.frame_size
+        out = {name: np.empty((h, w) + shape, dtype) for name, (dtype, shape) in HIT_PLANES.items() if name in planes}
+        unknown = set(planes) - set(HIT_PLANES)
+        if unknown:
+            raise ValueError(f"unknown hit planes {sorted(unknown)}")
+        p = HitPlanes(*(out[name].ctypes.data if name in out else None for name in HIT_PLANES))
+        st = Stats()
+        _check_host(host_lib.c2rt_host_render_hits(self._h, C.byref(p), seed, C.byref(st)))
+        return out, st
+
+
+# the planes of a hit frame: element type and per-pixel shape, in c2rt_hit_planes order
+HIT_PLANES = {"node": (np.int32, ()), "dist": (np.float32, ()), "normal": (np.float32, (3,)), "uv": (np.float32, (2,))}
+
+
 def save_bmp(argb, pad_rows=False):
     """saveBmp (imageio/bmp.d:195-237) of a packed uint32 plane [H, W] -> bytes."""
     a = np.ascontiguousarray(argb, np.uint32)
@@ -293,6 +319,14 @@ def render_device(scene_handle, cam, settings, d_rgb_ptr, d_argb_ptr=None, band=
     """c2rt_render_device: device pointers (ints), async on `stream` (int cudaStream_t or None)."""
     b = C.byref(band) if band is not None else None
     _check(lib.c2rt_render_device(scene_handle, C.byref(cam), C.byref(settings), b, d_rgb_ptr, d_argb_ptr, stream, None))
+
+
+def render_hits_device(scene_handle, cam, settings, node=None, dist=None, normal=None, uv=None, band=None, stream=None):
+    """c2rt_render_hits_device: plane device pointers (ints, e.g. a torch tensor's data_ptr(); None = not wanted), async on
+    `stream` (int cudaStream_t or None)."""
+    b = C.byref(band) if band is not None else None
+    p = HitPlanes(node, dist, normal, uv)
+    _check(lib.c2rt_render_hits_device(scene_handle, C.byref(cam), C.byref(settings), b, C.byref(p), stream, None))
 
 
 def read_ray_counters(scene_handle, stream=None):

@@ -26,6 +26,7 @@ namespace c2rt {
 cudaError_t upload_scene(const DevScene& s, cudaStream_t st);
 cudaError_t launch_frame(const FrameParams& fp, int mode, uint32_t local_tile_rows, cudaStream_t st);
 cudaError_t launch_pixel(const FrameParams& fp, int mode, int x, int y, PixelOut* d_out, cudaStream_t st);
+cudaError_t launch_hits(const FrameParams& fp, int mode, uint32_t local_tile_rows, const c2rt_hit_planes& out, cudaStream_t st);
 cudaError_t launch_deinterleave(const void* src, void* dst, uint32_t row_words, uint32_t height, uint32_t n_ranks,
                                 uint32_t band_rows, uint32_t rows_pad, cudaStream_t st);
 cudaError_t launch_fma_peak(bool fp64, int blocks, int threads, int iters, void* d_out, cudaStream_t st);
@@ -69,7 +70,8 @@ struct DeviceCtx {
     PixelOut* d_pixel = nullptr;
     float* d_rgb = nullptr;
     uint32_t* d_argb = nullptr;
-    size_t rgb_cap = 0, argb_cap = 0;
+    uint32_t* d_hits = nullptr;   // the four planes of a c2rt_render_hits frame, one after the other
+    size_t rgb_cap = 0, argb_cap = 0, hits_cap = 0;
 };
 
 struct Context {
@@ -185,6 +187,7 @@ void destroy_device(DeviceCtx& c) {
     cudaFree(c.d_pixel);
     cudaFree(c.d_rgb);
     cudaFree(c.d_argb);
+    cudaFree(c.d_hits);
     c = DeviceCtx();
 }
 
@@ -863,11 +866,24 @@ int grow_buffer(T*& buf, size_t& cap, size_t elems) {
     return C2RT_OK;
 }
 
-// Device slot i's share of an n-device c2rt_render frame: its bands (frame_band_rows) render into the slot's compact
-// buffer, which holds only its own rows in order (the whole frame when n == 1), and each band is copied to its rows of
-// the caller's host frame on copy_stream once its launch has finished.  Returns when the copies are complete.
+// c2rt_render_pixel and the hit frames refuse GI frames with one rule and one message
+const char* const kGiPickMessage = "pixel pick on a GI frame: the reference's lastTracingResult is the last random path segment";
+
+int check_hit_args(const c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, const c2rt_hit_planes* planes) {
+    int rc = check_frame_args(s, cam, set);
+    if (rc) return rc;
+    if (!planes || (!planes->node && !planes->dist && !planes->normal && !planes->uv))
+        return fail(C2RT_ERR_INVALID_ARG, "every hit plane is null");
+    if (set->gi_enabled && !cam->dof) return fail(C2RT_ERR_UNSUPPORTED, kGiPickMessage);
+    return C2RT_OK;
+}
+
+// Device slot i's share of an n-device frame: its bands (frame_band_rows) render into the slot's compact buffers, which hold
+// only its own rows in order (the whole frame when n == 1), and each band is copied to its rows of the caller's host planes
+// on copy_stream once its launch has finished.  A colour frame (c2rt_render: rgb, argb) or, with `hits`, a hit frame
+// (c2rt_render_hits: its host planes).  Returns when the copies are complete.
 int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb,
-                 uint32_t* launches_out, float* kernel_ms_out) {
+                 const c2rt_hit_planes* hits, uint32_t* launches_out, float* kernel_ms_out) {
     const uint32_t W = set->frame_width, H = set->frame_height;
     const uint32_t brows = frame_band_rows(n, H, W);
     DeviceCtx& c = g_ctx.d[i];
@@ -875,13 +891,36 @@ int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt
     FrameParams fp;
     fill_params(fp, cam, set, s, i);
     set_bands(fp, c, (uint32_t)i, (uint32_t)n, brows, true);
-    fp.cancel = c.d_cancel;
     const size_t need = (size_t)c2rt_band_rows_owned(H, fp.rank, fp.n_ranks, brows) * W;
-    int rc = rgb ? grow_buffer(c.d_rgb, c.rgb_cap, need * 3) : C2RT_OK;
-    if (rc == C2RT_OK && argb) rc = grow_buffer(c.d_argb, c.argb_cap, need);
-    if (rc) return rc;
-    fp.rgb = rgb ? c.d_rgb : nullptr;
-    fp.argb = argb ? c.d_argb : nullptr;
+    // the output planes: host destination, device buffer, 4-byte words per pixel
+    struct Plane {
+        void* host;
+        uint32_t* dev;
+        uint32_t words;
+    } planes[4] = {};
+    c2rt_hit_planes d_hits = {};
+    int rc = C2RT_OK;
+    if (hits) {
+        rc = grow_buffer(c.d_hits, c.hits_cap, need * 7);
+        if (rc) return rc;
+        planes[0] = {hits->node, c.d_hits, 1};
+        planes[1] = {hits->dist, c.d_hits + need, 1};
+        planes[2] = {hits->normal, c.d_hits + need * 2, 3};
+        planes[3] = {hits->uv, c.d_hits + need * 5, 2};
+        d_hits.node = hits->node ? (int32_t*)planes[0].dev : nullptr;
+        d_hits.dist = hits->dist ? (float*)planes[1].dev : nullptr;
+        d_hits.normal = hits->normal ? (float*)planes[2].dev : nullptr;
+        d_hits.uv = hits->uv ? (float*)planes[3].dev : nullptr;
+    } else {
+        fp.cancel = c.d_cancel;
+        rc = rgb ? grow_buffer(c.d_rgb, c.rgb_cap, need * 3) : C2RT_OK;
+        if (rc == C2RT_OK && argb) rc = grow_buffer(c.d_argb, c.argb_cap, need);
+        if (rc) return rc;
+        fp.rgb = rgb ? c.d_rgb : nullptr;
+        fp.argb = argb ? c.d_argb : nullptr;
+        planes[0] = {rgb, (uint32_t*)c.d_rgb, 3};
+        planes[1] = {argb, c.d_argb, 1};
+    }
     CU(cudaEventRecord(c.e0, c.stream));
     uint32_t local_row = 0, b = 0;
     for (uint32_t y0 = (uint32_t)i * brows; y0 < H; y0 += (uint32_t)n * brows, b++) {
@@ -892,15 +931,15 @@ int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt
             c.band_done.push_back(e);
         }
         fp.tile_row0 = b * fp.tiles_per_band;
-        CU(launch_frame(fp, s->mode, (rows + TILE_H - 1) / TILE_H, c.stream));
+        const uint32_t tile_rows = (rows + TILE_H - 1) / TILE_H;
+        if (hits) CU(launch_hits(fp, s->mode, tile_rows, d_hits, c.stream));
+        else CU(launch_frame(fp, s->mode, tile_rows, c.stream));
         CU(cudaEventRecord(c.band_done[b], c.stream));
         CU(cudaStreamWaitEvent(c.copy_stream, c.band_done[b], 0));
-        if (rgb)
-            CU(cudaMemcpyAsync(rgb + (size_t)y0 * W * 3, c.d_rgb + (size_t)local_row * W * 3, (size_t)rows * W * 3 * sizeof(float),
-                               cudaMemcpyDeviceToHost, c.copy_stream));
-        if (argb)
-            CU(cudaMemcpyAsync(argb + (size_t)y0 * W, c.d_argb + (size_t)local_row * W, (size_t)rows * W * sizeof(uint32_t),
-                               cudaMemcpyDeviceToHost, c.copy_stream));
+        for (const Plane& p : planes)
+            if (p.host)
+                CU(cudaMemcpyAsync((uint32_t*)p.host + (size_t)y0 * W * p.words, p.dev + (size_t)local_row * W * p.words,
+                                   (size_t)rows * W * p.words * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.copy_stream));
         local_row += rows;
     }
     CU(cudaEventRecord(c.e1, c.stream));
@@ -1080,10 +1119,10 @@ int c2rt_render(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set,
     std::string errs[C2RT_MAX_GPUS];
     if (n > 1)
         g_pool.run([&](int w) {
-            rcs[w + 1] = render_bands(w + 1, n, s, cam, set, rgb, argb, &ls[w + 1], &kms[w + 1]);
+            rcs[w + 1] = render_bands(w + 1, n, s, cam, set, rgb, argb, nullptr, &ls[w + 1], &kms[w + 1]);
             if (rcs[w + 1]) errs[w + 1] = g_err;
         });
-    rcs[0] = render_bands(0, n, s, cam, set, rgb, argb, &ls[0], &kms[0]);
+    rcs[0] = render_bands(0, n, s, cam, set, rgb, argb, nullptr, &ls[0], &kms[0]);
     if (rcs[0]) errs[0] = g_err;
     if (n > 1) g_pool.wait();
     uint32_t launches = 0;
@@ -1141,8 +1180,7 @@ int c2rt_render_pixel(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings
     int rc = check_frame_args(s, cam, set);
     if (rc) return rc;
     if (!rgb) return fail(C2RT_ERR_INVALID_ARG, "rgb is null");
-    if (set->gi_enabled && !cam->dof)
-        return fail(C2RT_ERR_UNSUPPORTED, "pixel pick on a GI frame: the reference's lastTracingResult is the last random path segment");
+    if (set->gi_enabled && !cam->dof) return fail(C2RT_ERR_UNSUPPORTED, kGiPickMessage);
     if (x < 0 || y < 0 || (uint32_t)x >= set->frame_width || (uint32_t)y >= set->frame_height)
         return fail(C2RT_ERR_INVALID_ARG, "pixel (%d,%d) outside the %ux%u frame", x, y, set->frame_width, set->frame_height);
     std::lock_guard<std::mutex> g(g_mu);
@@ -1167,6 +1205,84 @@ int c2rt_render_pixel(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings
         hit->dist = o.dist;
         for (int k = 0; k < 3; k++) { hit->p[k] = o.p[k]; hit->normal[k] = o.n[k]; }
         hit->u = o.u; hit->v = o.v;
+    }
+    return C2RT_OK;
+}
+
+int c2rt_render_hits(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, const c2rt_hit_planes* planes, c2rt_stats* stats) {
+    auto t0 = std::chrono::steady_clock::now();
+    int rc = check_hit_args(s, cam, set, planes);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> g(g_mu);
+    rc = ensure_init_locked();
+    if (rc) return rc;
+    if (s->n_dev != g_ctx.n) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
+    const int n = g_ctx.n;
+    for (int i = 0; i < n; i++) {   // (as in c2rt_render: residency first, on this thread)
+        if (g_ctx.d[i].uploaded_scene == s->id) continue;
+        CU(cudaSetDevice(g_ctx.d[i].dev));
+        rc = make_resident(s, i, g_ctx.d[i].stream);
+        if (rc) return rc;
+    }
+    int rcs[C2RT_MAX_GPUS] = {};
+    uint32_t ls[C2RT_MAX_GPUS] = {};
+    float kms[C2RT_MAX_GPUS] = {};
+    std::string errs[C2RT_MAX_GPUS];
+    if (n > 1)
+        g_pool.run([&](int w) {
+            rcs[w + 1] = render_bands(w + 1, n, s, cam, set, nullptr, nullptr, planes, &ls[w + 1], &kms[w + 1]);
+            if (rcs[w + 1]) errs[w + 1] = g_err;
+        });
+    rcs[0] = render_bands(0, n, s, cam, set, nullptr, nullptr, planes, &ls[0], &kms[0]);
+    if (rcs[0]) errs[0] = g_err;
+    if (n > 1) g_pool.wait();
+    uint32_t launches = 0;
+    double kernel_ms = 0;
+    for (int i = 0; i < n; i++) {
+        if (rcs[i]) { g_err = errs[i]; return rcs[i]; }
+        launches += ls[i];
+        if (kms[i] > kernel_ms) kernel_ms = kms[i];
+    }
+    CU(cudaSetDevice(g_ctx.d[0].dev));
+    if (stats) {
+        memset(stats, 0, sizeof *stats);
+        stats->kernel_ms = kernel_ms;
+        stats->n_gpus = (uint32_t)n;
+        stats->launches = launches;
+        stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    return C2RT_OK;
+}
+
+int c2rt_render_hits_device(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, const c2rt_band* band,
+                            const c2rt_hit_planes* planes, void* stream, c2rt_stats* stats) {
+    int rc = check_hit_args(s, cam, set, planes);
+    if (rc) return rc;
+    if (band && band->done_flags) return fail(C2RT_ERR_INVALID_ARG, "hit frames have no frame-complete signalling: done_flags must be null");
+    std::lock_guard<std::mutex> g(g_mu);
+    if (!g_ctx.inited) return fail(C2RT_ERR_NOT_INITIALISED, "c2rt_init has not been called");
+    int dev = -1;
+    CU(cudaGetDevice(&dev));
+    DeviceCtx* c = find_device(dev);
+    if (!c) return fail(C2RT_ERR_INVALID_ARG, "current device %d is not part of the c2rt context", dev);
+    int di = (int)(c - g_ctx.d);
+    if (di >= s->n_dev) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = make_resident(s, di, st);
+    if (rc) return rc;
+    const c2rt_band whole = {0, 1, TILE_H, 0, nullptr, 0, 0};   // no band: the whole frame on one rank
+    const c2rt_band& b = band ? *band : whole;
+    if (b.n_ranks == 0 || b.rank >= b.n_ranks || b.band_rows == 0 || b.band_rows % TILE_H != 0)
+        return fail(C2RT_ERR_INVALID_ARG, "bad band (rank %u of %u, band_rows %u; band_rows must be a multiple of %d)", b.rank,
+                    b.n_ranks, b.band_rows, TILE_H);
+    FrameParams fp;
+    fill_params(fp, cam, set, s, di);
+    set_bands(fp, *c, b.rank, b.n_ranks, b.band_rows, b.compact != 0);
+    CU(launch_hits(fp, s->mode, local_tile_rows(fp.H, b.rank, b.n_ranks, b.band_rows), *planes, st));
+    if (stats) {
+        memset(stats, 0, sizeof *stats);
+        stats->n_gpus = 1;
+        stats->launches = 1;
     }
     return C2RT_OK;
 }

@@ -111,6 +111,24 @@ int c2rt_host_render(c2rt_host_scene* h, float* rgb, uint32_t* argb, uint64_t se
     }
 }
 
+// renderPixel's hit record for every pixel into caller-owned HOST planes (c2rt_render_hits; `seed`: DOF / stereo frames)
+int c2rt_host_render_hits(c2rt_host_scene* h, const c2rt_hit_planes* planes, uint64_t seed, c2rt_stats* stats) {
+    try {
+        Scene& sc = *h->scene;
+        sc.beginFrame();
+        c2rt_camera cam = flattenCamera(sc.camera);
+        c2rt_settings set = flattenSettings(sc.settings, seed, false);
+        c2rt_scene* dev = c2rt_host_device_scene(h);
+        if (!dev) return C2RT_ERR_CUDA;
+        int rc = c2rt_render_hits(dev, &cam, &set, planes, stats);
+        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
+        return rc;
+    } catch (const std::exception& e) {
+        g_host_err = e.what();
+        return C2RT_ERR_INVALID_ARG;
+    }
+}
+
 // renderPixel(scene, output, x, y) (renderer.d:46-57)
 int c2rt_host_render_pixel(c2rt_host_scene* h, int x, int y, float rgb[3], c2rt_hit* hit) {
     try {

@@ -5,11 +5,14 @@
 //
 //   chess2rt_headless --file scenes/lecture5.sdl --out out.bmp [--pfm out.pfm] [--width W --height H]
 //                     [--gpus N] [--no-dof] [--no-aa] [--seed S] [--repeat K] [--pad-rows] [--orbit K]
+//                     [--depth d.pfm] [--ids ids.pgm]
 // --out writes the BMP the reference's Bitmap.saveImage would (bitmap.d:84-103 -> bmp.d:195-237, rows unpadded: only
 // widths with 3 W % 4 == 0 give a file other readers accept); --pad-rows writes the valid file for any width.
 // --orbit K: the interactive loop without a window — K frames, the camera turned by 360 / K degrees of yaw before each
 // (Camera.rotate, camera.d:211-229, what the arrow keys do: raytracer_demo.d:268-340), scene resident on the GPU, only the
 // camera / settings blocks go down and only the packed ARGB plane comes back (what SDL2Gui.draw blits, sdl2_gui.d:139-155).
+// --depth / --ids: renderPixel's hit distance / node of every pixel (one c2rt_render_hits call after the last frame), as a
+// one-channel PFM (bottom row first, +inf for a miss) / a 16-bit binary PGM (node + 1, 0 for a miss).
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -24,11 +27,11 @@ static void usage() {
     fprintf(stderr,
             "usage: chess2rt_headless --file <scene.sdl|scene.json> [--out img.bmp] [--pfm img.pfm]\n"
             "                         [--width W --height H] [--gpus N] [--no-dof] [--no-aa] [--seed S] [--repeat K]\n"
-            "                         [--pad-rows] [--orbit K]\n");
+            "                         [--pad-rows] [--orbit K] [--depth d.pfm] [--ids ids.pgm]\n");
 }
 
 int main(int argc, char** argv) {
-    std::string file, out, pfm;
+    std::string file, out, pfm, depth, ids;
     uint32_t width = 0, height = 0;
     int gpus = 1, repeat = 1, orbit = 0;
     bool noDof = false, noAA = false, padRows = false;
@@ -45,6 +48,8 @@ int main(int argc, char** argv) {
         if ((v = val("--file"))) file = v;
         else if ((v = val("--out"))) out = v;
         else if ((v = val("--pfm"))) pfm = v;
+        else if ((v = val("--depth"))) depth = v;
+        else if ((v = val("--ids"))) ids = v;
         else if ((v = val("--width"))) width = (uint32_t)atoi(v);
         else if ((v = val("--height"))) height = (uint32_t)atoi(v);
         else if ((v = val("--gpus"))) gpus = atoi(v);
@@ -103,6 +108,34 @@ int main(int argc, char** argv) {
             f << "PF\n" << W << " " << H << "\n-1.0\n";
             for (uint32_t y = H; y-- > 0;) f.write((const char*)&screen.pixels[(size_t)W * y], (std::streamsize)W * sizeof(Color));
             printf("wrote %s\n", pfm.c_str());
+        }
+        if (!depth.empty() || !ids.empty()) {
+            HitPlanes hits;
+            if (!depth.empty()) hits.dist.resize((size_t)W * H);
+            if (!ids.empty()) hits.node.resize((size_t)W * H);
+            Renderer renderer(*scene, screen);
+            renderer.options = opt;
+            renderer.renderHits(hits);
+            if (!depth.empty()) {  // one-channel float, bottom row first (PFM convention), little endian
+                std::ofstream f(depth, std::ios::binary);
+                f << "Pf\n" << W << " " << H << "\n-1.0\n";
+                for (uint32_t y = H; y-- > 0;) f.write((const char*)&hits.dist[(size_t)W * y], (std::streamsize)W * sizeof(float));
+                printf("wrote %s\n", depth.c_str());
+            }
+            if (!ids.empty()) {  // 16-bit binary PGM: most significant byte first, top row first
+                std::ofstream f(ids, std::ios::binary);
+                f << "P5\n" << W << " " << H << "\n65535\n";
+                std::vector<uint8_t> row((size_t)W * 2);
+                for (uint32_t y = 0; y < H; y++) {
+                    for (uint32_t x = 0; x < W; x++) {
+                        const uint32_t v = (uint32_t)(hits.node[(size_t)W * y + x] + 1);
+                        row[2 * x] = (uint8_t)(v >> 8);
+                        row[2 * x + 1] = (uint8_t)v;
+                    }
+                    f.write((const char*)row.data(), (std::streamsize)row.size());
+                }
+                printf("wrote %s\n", ids.c_str());
+            }
         }
         if (orbit > 0) {
             RenderOptions io = opt;

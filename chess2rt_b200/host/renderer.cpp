@@ -60,6 +60,22 @@ void Renderer::renderRT() {
     if (rc != C2RT_OK && !cancelled) raise(rc);
 }
 
+void Renderer::renderHits(HitPlanes& planes) {
+    const size_t n = (size_t)scene_.settings.frameWidth * scene_.settings.frameHeight;
+    if ((!planes.node.empty() && planes.node.size() != n) || (!planes.dist.empty() && planes.dist.size() != n) ||
+        (!planes.normal.empty() && planes.normal.size() != 3 * n) || (!planes.uv.empty() && planes.uv.size() != 2 * n))
+        throw RTException("hit plane size does not match settings.frameWidth x frameHeight");
+    c2rt_camera cam = flattenCamera(scene_.camera);
+    c2rt_settings set = flattenSettings(scene_.settings, options.rngSeed, false);
+    c2rt_hit_planes p;
+    p.node = planes.node.empty() ? nullptr : planes.node.data();
+    p.dist = planes.dist.empty() ? nullptr : planes.dist.data();
+    p.normal = planes.normal.empty() ? nullptr : planes.normal.data();
+    p.uv = planes.uv.empty() ? nullptr : planes.uv.data();
+    int rc = c2rt_render_hits(device(), &cam, &set, &p, &lastStats);
+    if (rc != C2RT_OK) raise(rc);
+}
+
 void requestStop(std::atomic<bool>* isStopRequested) {
     if (isStopRequested) isStopRequested->store(true);
     c2rt_cancel();

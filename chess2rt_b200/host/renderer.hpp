@@ -33,11 +33,21 @@ struct RenderOptions {        // knobs the reference does not have
     bool argbOnly = false;    // interactive hosts that only blit `argb` (sdl2_gui.d:139-155): the float frame is neither written nor copied
 };
 
+// renderPixel's hit record for every pixel of the frame (c2rt_render_hits): structure of arrays, row-major, top row first.
+// renderHits fills the planes that are not empty; a non-empty plane must hold exactly W * H records.
+struct HitPlanes {
+    std::vector<int32_t> node;   // [W*H] closestNode, -1 = miss
+    std::vector<float> dist;     // [W*H] hit distance, +inf for a miss
+    std::vector<float> normal;   // [W*H*3] unit geometric normal, 0 for a miss
+    std::vector<float> uv;       // [W*H*2] u, v, 0 for a miss
+};
+
 struct Renderer {
     Renderer(const Scene& scene, Image<Color>& output, std::atomic<bool>* isRendering = nullptr,
              const std::atomic<bool>* isStopRequested = nullptr);
 
     void renderRT();                               // renderer.d:83-189
+    void renderHits(HitPlanes& planes);            // no counterpart: renderPixelNoAA's hit record for every pixel, no colour
     Color renderPixelNoAA(int x, int y);           // renderer.d:223-228 (also records lastTracingResult)
 
     TraceResult lastTracingResult;

@@ -261,6 +261,28 @@ int c2rt_deinterleave(const void* gathered, void* frame, uint32_t width, uint32_
 int c2rt_render_pixel(c2rt_scene* scene, const c2rt_camera* camera, const c2rt_settings* settings,
                       int x, int y, float rgb[3], c2rt_hit* hit);
 
+/* Hit buffers: for every pixel of the frame, the hit record that the renderPixel replacement above returns for that pixel
+ * (the un-antialiased ray at the pixel corner; on DOF / stereo frames sample 0 of the left eye with the pinned generator),
+ * floating-point fields rounded to FP32.  Structure of arrays, row-major, top row first; every plane may be NULL.
+ * No colour is computed.  aa_enabled, prepass_only and count_rays are ignored; the ray counters and the cancel flag are
+ * neither read nor changed.  GI frames are refused with C2RT_ERR_UNSUPPORTED, as the pixel pick refuses them. */
+typedef struct c2rt_hit_planes {
+    int32_t* node;     /* [W*H] closestNode, -1 = miss */
+    float* dist;       /* [W*H] hit distance, +inf for a miss */
+    float* normal;     /* [W*H*3] unit geometric normal, 0 for a miss */
+    float* uv;         /* [W*H*2] u, v, 0 for a miss */
+} c2rt_hit_planes;
+
+/* Blocking, into caller-owned HOST planes.  With n_gpus > 1 the frame is split into the same interleaved row bands as the
+ * colour frame, and every device copies its own rows.  stats (nullable): kernel_ms, total_ms, n_gpus, launches. */
+int c2rt_render_hits(c2rt_scene* scene, const c2rt_camera* camera, const c2rt_settings* settings,
+                     const c2rt_hit_planes* host_planes, c2rt_stats* stats);
+/* The same into DEVICE planes of the current device, async on `stream`, with the band and scene-residency rules of the
+ * colour frame's device call (band NULL = the whole frame; compact 0 or 1).  band->done_flags must be NULL: hit frames
+ * have no frame-complete signalling.  stats (nullable) gets launches only. */
+int c2rt_render_hits_device(c2rt_scene* scene, const c2rt_camera* camera, const c2rt_settings* settings,
+                            const c2rt_band* band, const c2rt_hit_planes* device_planes, void* stream, c2rt_stats* stats);
+
 /* Number of rows rank `rank` owns in a frame of `height` rows. */
 uint32_t c2rt_band_rows_owned(uint32_t height, uint32_t rank, uint32_t n_ranks, uint32_t band_rows);
 
