@@ -796,6 +796,8 @@ void fill_params(FrameParams& fp, const c2rt_camera* cam, const c2rt_settings* s
         // the same value for every sx >= 0, so d.y is constant along a row.  Tested on the value the kernel uses, not on the
         // camera's roll: the corners reach the ABI from any host.
         fp.solo_rows = fp.solo_fast && fp.du[1] == 0.0;
+        // the same for d.z = fma(dv.z, sy, fma(du.z, sx, ul_rel.z)) + tap_d.z: a camera without yaw or roll has du.z == 0
+        fp.solo_zrows = fp.solo_rows && fp.du[2] == 0.0;
     }
 }
 

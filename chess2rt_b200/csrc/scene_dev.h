@@ -133,6 +133,9 @@ struct FrameParams {
     uint32_t* argb;
     unsigned long long* counters;     // [0] primary, [1] shadow
     const uint8_t* lut;               // 4097-entry sRGB table
+    // solo_zrows: a solo_rows frame with du.z == 0 as well (no yaw): a camera ray's d.z, its hit point's z and what depends on
+    // it alone are constants of the (row, AA tap) too (render_kernel.cu RowZ).  Last, so that every other field keeps its offset.
+    uint32_t solo_zrows;
 };
 
 // Kernel specialisations by scene class (chosen at scene-create time, c2rt_api.cu):
