@@ -240,10 +240,17 @@ int ensure_init_locked() {
     return init_locked(1, &dev);
 }
 
-DeviceCtx* find_device(int dev) {
+// The context slot of the caller's current device (the entry points that work on the caller's device and stream)
+int current_device_locked(DeviceCtx*& c) {
+    if (!g_ctx.inited) return fail(C2RT_ERR_NOT_INITIALISED, "c2rt_init has not been called");
+    int dev = -1;
+    CU(cudaGetDevice(&dev));
     for (int i = 0; i < g_ctx.n; i++)
-        if (g_ctx.d[i].dev == dev) return &g_ctx.d[i];
-    return nullptr;
+        if (g_ctx.d[i].dev == dev) {
+            c = &g_ctx.d[i];
+            return C2RT_OK;
+        }
+    return fail(C2RT_ERR_INVALID_ARG, "current device %d is not part of the c2rt context", dev);
 }
 
 }  // namespace
@@ -952,6 +959,63 @@ int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt
     return C2RT_OK;
 }
 
+// A frame on every context device (c2rt_render, c2rt_render_hits; lock held): the scene made resident everywhere first, on this
+// thread (make_resident patches the shared host copy of the scene block per device), then render_bands for device 0 on this
+// thread and for device w + 1 on pool worker w.  Every device copies its bands to the host frame over its own PCIe link: the
+// host copy of a float frame is the slow part, so N links beat one.  Returns the first failing device's status and message,
+// or the launches of all devices and the longest kernel time, with device 0 current again.
+int render_devices_locked(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb,
+                          const c2rt_hit_planes* hits, uint32_t& launches, double& kernel_ms) {
+    const int n = g_ctx.n;
+    for (int i = 0; i < n; i++) {
+        if (g_ctx.d[i].uploaded_scene == s->id) continue;
+        CU(cudaSetDevice(g_ctx.d[i].dev));
+        const int rc = make_resident(s, i, g_ctx.d[i].stream);
+        if (rc) return rc;
+    }
+    int rcs[C2RT_MAX_GPUS] = {};
+    uint32_t ls[C2RT_MAX_GPUS] = {};
+    float kms[C2RT_MAX_GPUS] = {};
+    std::string errs[C2RT_MAX_GPUS];
+    if (n > 1)
+        g_pool.run([&](int w) {
+            rcs[w + 1] = render_bands(w + 1, n, s, cam, set, rgb, argb, hits, &ls[w + 1], &kms[w + 1]);
+            if (rcs[w + 1]) errs[w + 1] = g_err;
+        });
+    rcs[0] = render_bands(0, n, s, cam, set, rgb, argb, hits, &ls[0], &kms[0]);
+    if (rcs[0]) errs[0] = g_err;
+    if (n > 1) g_pool.wait();
+    launches = 0;
+    kernel_ms = 0;
+    for (int i = 0; i < n; i++) {
+        if (rcs[i]) { g_err = errs[i]; return rcs[i]; }
+        launches += ls[i];
+        if (kms[i] > kernel_ms) kernel_ms = kms[i];
+    }
+    CU(cudaSetDevice(g_ctx.d[0].dev));
+    return C2RT_OK;
+}
+
+// The set-up of a launch on the caller's device and stream (c2rt_render_device, c2rt_render_hits_device; lock held): `c` is the
+// current device's slot, the scene is made resident there on `st`, `b` is the band (null `band`: the whole frame on one rank)
+// and `fp` the frame's parameters for that band.
+int device_band_locked(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, const c2rt_band* band, cudaStream_t st,
+                       DeviceCtx*& c, c2rt_band& b, FrameParams& fp) {
+    int rc = current_device_locked(c);
+    if (rc) return rc;
+    const int di = (int)(c - g_ctx.d);
+    if (di >= s->n_dev) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
+    rc = make_resident(s, di, st);
+    if (rc) return rc;
+    b = band ? *band : c2rt_band{0, 1, TILE_H, 0, nullptr, 0, 0};
+    if (b.n_ranks == 0 || b.rank >= b.n_ranks || b.band_rows == 0 || b.band_rows % TILE_H != 0)
+        return fail(C2RT_ERR_INVALID_ARG, "bad band (rank %u of %u, band_rows %u; band_rows must be a multiple of %d)", b.rank,
+                    b.n_ranks, b.band_rows, TILE_H);
+    fill_params(fp, cam, set, s, di);
+    set_bands(fp, *c, b.rank, b.n_ranks, b.band_rows, b.compact != 0);
+    return C2RT_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1040,24 +1104,12 @@ int c2rt_render_device(c2rt_scene* s, const c2rt_camera* cam, const c2rt_setting
     if (!d_rgb) return fail(C2RT_ERR_INVALID_ARG, "d_rgb is null");
     if (set->prepass_only && !set->prepass_enabled) return C2RT_OK;  // renderer.d:110,129-130: nothing is drawn
     std::lock_guard<std::mutex> g(g_mu);
-    if (!g_ctx.inited) return fail(C2RT_ERR_NOT_INITIALISED, "c2rt_init has not been called");
-    int dev = -1;
-    CU(cudaGetDevice(&dev));
-    DeviceCtx* c = find_device(dev);
-    if (!c) return fail(C2RT_ERR_INVALID_ARG, "current device %d is not part of the c2rt context", dev);
-    int di = (int)(c - g_ctx.d);
-    if (di >= s->n_dev) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
-    cudaStream_t st = (cudaStream_t)stream;
-    rc = make_resident(s, di, st);
-    if (rc) return rc;
-    const c2rt_band whole = {0, 1, TILE_H, 0, nullptr, 0, 0};   // no band: the whole frame on one rank
-    const c2rt_band& b = band ? *band : whole;
-    if (b.n_ranks == 0 || b.rank >= b.n_ranks || b.band_rows == 0 || b.band_rows % TILE_H != 0)
-        return fail(C2RT_ERR_INVALID_ARG, "bad band (rank %u of %u, band_rows %u; band_rows must be a multiple of %d)", b.rank,
-                    b.n_ranks, b.band_rows, TILE_H);
+    const cudaStream_t st = (cudaStream_t)stream;
+    DeviceCtx* c;
+    c2rt_band b;
     FrameParams fp;
-    fill_params(fp, cam, set, s, di);
-    set_bands(fp, *c, b.rank, b.n_ranks, b.band_rows, b.compact != 0);
+    rc = device_band_locked(s, cam, set, band, st, c, b, fp);
+    if (rc) return rc;
     if (b.done_flags) {
         if (b.n_ranks > 32) return fail(C2RT_ERR_INVALID_ARG, "done_flags: at most 32 ranks");
         fp.frame_no = b.frame_no;
@@ -1083,11 +1135,9 @@ int c2rt_render_device(c2rt_scene* s, const c2rt_camera* cam, const c2rt_setting
 
 int c2rt_read_ray_counters(c2rt_scene*, void* stream, uint64_t* primary, uint64_t* shadow) {
     std::lock_guard<std::mutex> g(g_mu);
-    if (!g_ctx.inited) return fail(C2RT_ERR_NOT_INITIALISED, "c2rt_init has not been called");
-    int dev = -1;
-    CU(cudaGetDevice(&dev));
-    DeviceCtx* c = find_device(dev);
-    if (!c) return fail(C2RT_ERR_INVALID_ARG, "current device %d is not part of the c2rt context", dev);
+    DeviceCtx* c;
+    const int rc = current_device_locked(c);
+    if (rc) return rc;
     return take_ray_counters(*c, (cudaStream_t)stream, primary, shadow);
 }
 
@@ -1105,43 +1155,17 @@ int c2rt_render(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set,
     if (rc) return rc;
     if (s->n_dev != g_ctx.n) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
     take_cancel_request();   // a cancel that arrived while no frame was in progress cancels nothing
-    const int n = g_ctx.n;
-    // scene residency first, on this thread: make_resident patches the shared host copy of the scene block per device
-    for (int i = 0; i < n; i++) {
-        if (g_ctx.d[i].uploaded_scene == s->id) continue;
-        CU(cudaSetDevice(g_ctx.d[i].dev));
-        rc = make_resident(s, i, g_ctx.d[i].stream);
-        if (rc) return rc;
-    }
-    // Every device renders its bands and copies them to the host frame over its own PCIe link: the host copy of a float
-    // frame is the slow part, so N links beat one.  Worker w of the pool drives device w + 1, this thread drives device 0.
-    int rcs[C2RT_MAX_GPUS] = {};
-    uint32_t ls[C2RT_MAX_GPUS] = {};
-    float kms[C2RT_MAX_GPUS] = {};
-    std::string errs[C2RT_MAX_GPUS];
-    if (n > 1)
-        g_pool.run([&](int w) {
-            rcs[w + 1] = render_bands(w + 1, n, s, cam, set, rgb, argb, nullptr, &ls[w + 1], &kms[w + 1]);
-            if (rcs[w + 1]) errs[w + 1] = g_err;
-        });
-    rcs[0] = render_bands(0, n, s, cam, set, rgb, argb, nullptr, &ls[0], &kms[0]);
-    if (rcs[0]) errs[0] = g_err;
-    if (n > 1) g_pool.wait();
-    uint32_t launches = 0;
-    double kernel_ms = 0;
-    for (int i = 0; i < n; i++) {
-        if (rcs[i]) { g_err = errs[i]; return rcs[i]; }
-        launches += ls[i];
-        if (kms[i] > kernel_ms) kernel_ms = kms[i];
-    }
-    CU(cudaSetDevice(g_ctx.d[0].dev));
+    uint32_t launches;
+    double kernel_ms;
+    rc = render_devices_locked(s, cam, set, rgb, argb, nullptr, launches, kernel_ms);
+    if (rc) return rc;
     if (stats) {
         memset(stats, 0, sizeof *stats);
         stats->kernel_ms = kernel_ms;
-        stats->n_gpus = (uint32_t)n;
+        stats->n_gpus = (uint32_t)g_ctx.n;
         stats->launches = launches;
         if (set->count_rays) {
-            for (int i = 0; i < n; i++) {
+            for (int i = 0; i < g_ctx.n; i++) {
                 DeviceCtx& c = g_ctx.d[i];
                 CU(cudaSetDevice(c.dev));
                 uint64_t p, sh;
@@ -1219,37 +1243,14 @@ int c2rt_render_hits(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings*
     rc = ensure_init_locked();
     if (rc) return rc;
     if (s->n_dev != g_ctx.n) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
-    const int n = g_ctx.n;
-    for (int i = 0; i < n; i++) {   // (as in c2rt_render: residency first, on this thread)
-        if (g_ctx.d[i].uploaded_scene == s->id) continue;
-        CU(cudaSetDevice(g_ctx.d[i].dev));
-        rc = make_resident(s, i, g_ctx.d[i].stream);
-        if (rc) return rc;
-    }
-    int rcs[C2RT_MAX_GPUS] = {};
-    uint32_t ls[C2RT_MAX_GPUS] = {};
-    float kms[C2RT_MAX_GPUS] = {};
-    std::string errs[C2RT_MAX_GPUS];
-    if (n > 1)
-        g_pool.run([&](int w) {
-            rcs[w + 1] = render_bands(w + 1, n, s, cam, set, nullptr, nullptr, planes, &ls[w + 1], &kms[w + 1]);
-            if (rcs[w + 1]) errs[w + 1] = g_err;
-        });
-    rcs[0] = render_bands(0, n, s, cam, set, nullptr, nullptr, planes, &ls[0], &kms[0]);
-    if (rcs[0]) errs[0] = g_err;
-    if (n > 1) g_pool.wait();
-    uint32_t launches = 0;
-    double kernel_ms = 0;
-    for (int i = 0; i < n; i++) {
-        if (rcs[i]) { g_err = errs[i]; return rcs[i]; }
-        launches += ls[i];
-        if (kms[i] > kernel_ms) kernel_ms = kms[i];
-    }
-    CU(cudaSetDevice(g_ctx.d[0].dev));
+    uint32_t launches;
+    double kernel_ms;
+    rc = render_devices_locked(s, cam, set, nullptr, nullptr, planes, launches, kernel_ms);
+    if (rc) return rc;
     if (stats) {
         memset(stats, 0, sizeof *stats);
         stats->kernel_ms = kernel_ms;
-        stats->n_gpus = (uint32_t)n;
+        stats->n_gpus = (uint32_t)g_ctx.n;
         stats->launches = launches;
         stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     }
@@ -1262,24 +1263,12 @@ int c2rt_render_hits_device(c2rt_scene* s, const c2rt_camera* cam, const c2rt_se
     if (rc) return rc;
     if (band && band->done_flags) return fail(C2RT_ERR_INVALID_ARG, "hit frames have no frame-complete signalling: done_flags must be null");
     std::lock_guard<std::mutex> g(g_mu);
-    if (!g_ctx.inited) return fail(C2RT_ERR_NOT_INITIALISED, "c2rt_init has not been called");
-    int dev = -1;
-    CU(cudaGetDevice(&dev));
-    DeviceCtx* c = find_device(dev);
-    if (!c) return fail(C2RT_ERR_INVALID_ARG, "current device %d is not part of the c2rt context", dev);
-    int di = (int)(c - g_ctx.d);
-    if (di >= s->n_dev) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
-    cudaStream_t st = (cudaStream_t)stream;
-    rc = make_resident(s, di, st);
-    if (rc) return rc;
-    const c2rt_band whole = {0, 1, TILE_H, 0, nullptr, 0, 0};   // no band: the whole frame on one rank
-    const c2rt_band& b = band ? *band : whole;
-    if (b.n_ranks == 0 || b.rank >= b.n_ranks || b.band_rows == 0 || b.band_rows % TILE_H != 0)
-        return fail(C2RT_ERR_INVALID_ARG, "bad band (rank %u of %u, band_rows %u; band_rows must be a multiple of %d)", b.rank,
-                    b.n_ranks, b.band_rows, TILE_H);
+    const cudaStream_t st = (cudaStream_t)stream;
+    DeviceCtx* c;
+    c2rt_band b;
     FrameParams fp;
-    fill_params(fp, cam, set, s, di);
-    set_bands(fp, *c, b.rank, b.n_ranks, b.band_rows, b.compact != 0);
+    rc = device_band_locked(s, cam, set, band, st, c, b, fp);
+    if (rc) return rc;
     CU(launch_hits(fp, s->mode, local_tile_rows(fp.H, b.rank, b.n_ranks, b.band_rows), *planes, st));
     if (stats) {
         memset(stats, 0, sizeof *stats);

@@ -303,6 +303,27 @@ def test_errors(ctx):
         g.render_hits(planes=("depth",))
 
 
+@pytest.mark.gpu
+def test_both_device_entry_points_refuse_a_malformed_band_alike(ctx):
+    import torch
+    g = scene(os.path.join(SC, "lecture4.sdl"), (64, 48))
+    handle = g.device_scene()
+    cam, st = g.frame_blocks()
+    rgb = torch.zeros((48, 64, 3), device="cuda")
+    node = torch.zeros((48, 64), dtype=torch.int32, device="cuda")
+    p = api.HitPlanes(node.data_ptr(), None, None, None)
+    # no ranks, a rank beyond them, empty bands, bands of a partial tile
+    for rank, n_ranks, band_rows in [(0, 0, 8), (2, 2, 8), (0, 1, 0), (1, 2, 12)]:
+        band = api.Band(rank, n_ranks, band_rows, 0)
+        assert api.lib.c2rt_render_device(handle, C.byref(cam), C.byref(st), C.byref(band), rgb.data_ptr(), None, None, None) == -1
+        colour = api.lib.c2rt_last_error().decode()
+        assert colour == f"bad band (rank {rank} of {n_ranks}, band_rows {band_rows}; band_rows must be a multiple of 8)"
+        assert api.lib.c2rt_render_hits_device(handle, C.byref(cam), C.byref(st), C.byref(band), C.byref(p), None, None) == -1
+        assert api.lib.c2rt_last_error().decode() == colour
+    torch.cuda.synchronize()
+    assert (rgb.cpu().numpy() == 0).all() and (node.cpu().numpy() == 0).all()
+
+
 def _read_pfm1(path):
     magic, dims, scale, body = open(path, "rb").read().split(b"\n", 3)
     w, h = map(int, dims.split())
