@@ -61,6 +61,10 @@ class HitPlanes(C.Structure):
     _fields_ = [("node", C.c_void_p), ("dist", C.c_void_p), ("normal", C.c_void_p), ("uv", C.c_void_p)]
 
 
+class RayHits(C.Structure):
+    _fields_ = [("node", C.c_void_p), ("dist", C.c_void_p), ("p", C.c_void_p), ("normal", C.c_void_p), ("uv", C.c_void_p)]
+
+
 class SceneDesc(C.Structure):
     _fields_ = [
         ("struct_size", C.c_uint32), ("abi_version", C.c_uint32),
@@ -86,7 +90,8 @@ class SceneDesc(C.Structure):
 C_ABI_SYMBOLS = [
     "c2rt_init", "c2rt_shutdown", "c2rt_abi_version", "c2rt_device_count", "c2rt_last_error",
     "c2rt_scene_create", "c2rt_scene_destroy", "c2rt_render", "c2rt_cancel", "c2rt_render_device", "c2rt_read_ray_counters",
-    "c2rt_deinterleave", "c2rt_render_pixel", "c2rt_render_hits", "c2rt_render_hits_device", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
+    "c2rt_deinterleave", "c2rt_render_pixel", "c2rt_render_hits", "c2rt_render_hits_device",
+    "c2rt_trace_rays", "c2rt_trace_rays_device", "c2rt_test_visibility", "c2rt_test_visibility_device", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
     "c2rt_frame_alloc", "c2rt_frame_free", "c2rt_frame_export", "c2rt_frame_import", "c2rt_frame_unimport", "c2rt_frame_memset", "c2rt_frame_download", "c2rt_pin_host_buffer", "c2rt_unpin_host_buffer", "c2rt_gate",
     "c2rt_measure_fma_peak", "c2rt_selftest_device_pool",
 ]
@@ -109,6 +114,12 @@ lib.c2rt_render_pixel.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Setti
 lib.c2rt_render_hits.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.POINTER(HitPlanes), C.POINTER(Stats)]
 lib.c2rt_render_hits_device.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.POINTER(Band), C.POINTER(HitPlanes),
                                         C.c_void_p, C.POINTER(Stats)]
+lib.c2rt_trace_rays.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.POINTER(RayHits), C.POINTER(Stats)]
+lib.c2rt_trace_rays_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.POINTER(RayHits), C.c_void_p,
+                                       C.POINTER(Stats)]
+lib.c2rt_test_visibility.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Stats)]
+lib.c2rt_test_visibility_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.POINTER(Stats)]
 lib.c2rt_band_rows_owned.argtypes = [C.c_uint32] * 4
 lib.c2rt_band_rows_owned.restype = C.c_uint32
 lib.c2rt_rng_u31.argtypes = [C.c_uint64] + [C.c_uint32] * 5
@@ -147,6 +158,8 @@ host_lib.c2rt_host_device_scene.restype = C.c_void_p
 host_lib.c2rt_host_render.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.POINTER(Stats)]
 host_lib.c2rt_host_render_pixel.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(Hit)]
 host_lib.c2rt_host_render_hits.argtypes = [C.c_void_p, C.POINTER(HitPlanes), C.c_uint64, C.POINTER(Stats)]
+host_lib.c2rt_host_trace_rays.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.POINTER(RayHits), C.POINTER(Stats)]
+host_lib.c2rt_host_test_visibility.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Stats)]
 host_lib.c2rt_host_camera_rotate.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_double]
 host_lib.c2rt_host_camera_rotate.restype = None
 host_lib.c2rt_host_camera_move.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_double]
@@ -297,6 +310,44 @@ class HostScene:
         _check_host(host_lib.c2rt_host_render_hits(self._h, C.byref(p), seed, C.byref(st)))
         return out, st
 
+    def trace_rays(self, origins, dirs, planes=("node", "dist", "p", "normal", "uv")):
+        """The closest hit of every ray (origins[i], normalize(dirs[i])) (c2rt_trace_rays) -> ({plane: array}, Stats).  origins
+        and dirs: [n, 3] float64.  Planes: node [n] int32 (-1 = miss), dist [n] (+inf for a miss), p, normal [n, 3] and uv
+        [n, 2] float64 (0 for a miss)."""
+        o, d = _points(origins), _points(dirs)
+        if o.shape != d.shape:
+            raise ValueError(f"origins {o.shape} and dirs {d.shape} differ in shape")
+        unknown = set(planes) - set(RAY_PLANES)
+        if unknown:
+            raise ValueError(f"unknown ray planes {sorted(unknown)}")
+        n = len(o)
+        out = {name: np.empty((n,) + shape, dtype) for name, (dtype, shape) in RAY_PLANES.items() if name in planes}
+        p = RayHits(*(out[name].ctypes.data if name in out else None for name in RAY_PLANES))
+        st = Stats()
+        _check_host(host_lib.c2rt_host_trace_rays(self._h, n, o.ctypes.data, d.ctypes.data, C.byref(p), C.byref(st)))
+        return out, st
+
+    def test_visibility(self, frm, to):
+        """testVisibility(frm[i], to[i]) for every i (c2rt_test_visibility) -> (bool [n] array, Stats).  frm, to: [n, 3]."""
+        f, t = _points(frm), _points(to)
+        if f.shape != t.shape:
+            raise ValueError(f"frm {f.shape} and to {t.shape} differ in shape")
+        vis = np.empty(len(f), np.uint8)
+        st = Stats()
+        _check_host(host_lib.c2rt_host_test_visibility(self._h, len(f), f.ctypes.data, t.ctypes.data, vis.ctypes.data, C.byref(st)))
+        return vis.astype(bool), st
+
+
+def _points(a):
+    a = np.ascontiguousarray(a, np.float64)
+    if a.ndim != 2 or a.shape[1] != 3:
+        raise ValueError(f"expected an [n, 3] array of points, got shape {a.shape}")
+    return a
+
+
+# the planes of a ray query: element type and per-ray shape, in c2rt_ray_hits order
+RAY_PLANES = {"node": (np.int32, ()), "dist": (np.float64, ()), "p": (np.float64, (3,)), "normal": (np.float64, (3,)),
+              "uv": (np.float64, (2,))}
 
 # the planes of a hit frame: element type and per-pixel shape, in c2rt_hit_planes order
 HIT_PLANES = {"node": (np.int32, ()), "dist": (np.float32, ()), "normal": (np.float32, (3,)), "uv": (np.float32, (2,))}
@@ -327,6 +378,18 @@ def render_hits_device(scene_handle, cam, settings, node=None, dist=None, normal
     b = C.byref(band) if band is not None else None
     p = HitPlanes(node, dist, normal, uv)
     _check(lib.c2rt_render_hits_device(scene_handle, C.byref(cam), C.byref(settings), b, C.byref(p), stream, None))
+
+
+def trace_rays_device(scene_handle, n, d_origins, d_dirs, node=None, dist=None, p=None, normal=None, uv=None, stream=None):
+    """c2rt_trace_rays_device: [n*3] float64 inputs and the output planes as device pointers (ints, e.g. a torch tensor's
+    data_ptr(); None = not wanted), async on `stream` (int cudaStream_t or None)."""
+    out = RayHits(node, dist, p, normal, uv)
+    _check(lib.c2rt_trace_rays_device(scene_handle, n, d_origins, d_dirs, C.byref(out), stream, None))
+
+
+def test_visibility_device(scene_handle, n, d_from, d_to, d_visible, stream=None):
+    """c2rt_test_visibility_device: [n*3] float64 inputs and the [n] uint8 output as device pointers, async on `stream`."""
+    _check(lib.c2rt_test_visibility_device(scene_handle, n, d_from, d_to, d_visible, stream, None))
 
 
 def read_ray_counters(scene_handle, stream=None):

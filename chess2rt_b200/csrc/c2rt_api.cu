@@ -27,6 +27,8 @@ cudaError_t upload_scene(const DevScene& s, cudaStream_t st);
 cudaError_t launch_frame(const FrameParams& fp, int mode, uint32_t local_tile_rows, cudaStream_t st);
 cudaError_t launch_pixel(const FrameParams& fp, int mode, int x, int y, PixelOut* d_out, cudaStream_t st);
 cudaError_t launch_hits(const FrameParams& fp, int mode, uint32_t local_tile_rows, const c2rt_hit_planes& out, cudaStream_t st);
+cudaError_t launch_rays(const RayParams& rp, int mode, cudaStream_t st);
+cudaError_t launch_visibility(const RayParams& rp, int mode, cudaStream_t st);
 cudaError_t launch_deinterleave(const void* src, void* dst, uint32_t row_words, uint32_t height, uint32_t n_ranks,
                                 uint32_t band_rows, uint32_t rows_pad, cudaStream_t st);
 cudaError_t launch_fma_peak(bool fp64, int blocks, int threads, int iters, void* d_out, cudaStream_t st);
@@ -71,7 +73,8 @@ struct DeviceCtx {
     float* d_rgb = nullptr;
     uint32_t* d_argb = nullptr;
     uint32_t* d_hits = nullptr;   // the four planes of a c2rt_render_hits frame, one after the other
-    size_t rgb_cap = 0, argb_cap = 0, hits_cap = 0;
+    double* d_rays = nullptr;     // a c2rt_trace_rays / c2rt_test_visibility chunk: its inputs, then its output planes
+    size_t rgb_cap = 0, argb_cap = 0, hits_cap = 0, rays_cap = 0;
 };
 
 struct Context {
@@ -188,6 +191,7 @@ void destroy_device(DeviceCtx& c) {
     cudaFree(c.d_rgb);
     cudaFree(c.d_argb);
     cudaFree(c.d_hits);
+    cudaFree(c.d_rays);
     c = DeviceCtx();
 }
 
@@ -964,8 +968,10 @@ int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt
 // thread and for device w + 1 on pool worker w.  Every device copies its bands to the host frame over its own PCIe link: the
 // host copy of a float frame is the slow part, so N links beat one.  Returns the first failing device's status and message,
 // or the launches of all devices and the longest kernel time, with device 0 current again.
-int render_devices_locked(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb,
-                          const c2rt_hit_planes* hits, uint32_t& launches, double& kernel_ms) {
+// work(i, &launches_i, &kernel_ms_i) runs device slot i's share of a call (the frame calls: render_bands; the ray queries:
+// ray_chunk).
+template <class Work>
+int run_devices_locked(c2rt_scene* s, Work&& work, uint32_t& launches, double& kernel_ms) {
     const int n = g_ctx.n;
     for (int i = 0; i < n; i++) {
         if (g_ctx.d[i].uploaded_scene == s->id) continue;
@@ -979,10 +985,10 @@ int render_devices_locked(c2rt_scene* s, const c2rt_camera* cam, const c2rt_sett
     std::string errs[C2RT_MAX_GPUS];
     if (n > 1)
         g_pool.run([&](int w) {
-            rcs[w + 1] = render_bands(w + 1, n, s, cam, set, rgb, argb, hits, &ls[w + 1], &kms[w + 1]);
+            rcs[w + 1] = work(w + 1, &ls[w + 1], &kms[w + 1]);
             if (rcs[w + 1]) errs[w + 1] = g_err;
         });
-    rcs[0] = render_bands(0, n, s, cam, set, rgb, argb, hits, &ls[0], &kms[0]);
+    rcs[0] = work(0, &ls[0], &kms[0]);
     if (rcs[0]) errs[0] = g_err;
     if (n > 1) g_pool.wait();
     launches = 0;
@@ -993,6 +999,152 @@ int render_devices_locked(c2rt_scene* s, const c2rt_camera* cam, const c2rt_sett
         if (kms[i] > kernel_ms) kernel_ms = kms[i];
     }
     CU(cudaSetDevice(g_ctx.d[0].dev));
+    return C2RT_OK;
+}
+int render_devices_locked(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb,
+                          const c2rt_hit_planes* hits, uint32_t& launches, double& kernel_ms) {
+    return run_devices_locked(
+        s, [&](int i, uint32_t* l, float* ms) { return render_bands(i, g_ctx.n, s, cam, set, rgb, argb, hits, l, ms); }, launches,
+        kernel_ms);
+}
+
+// ---- ray queries (c2rt_trace_rays, c2rt_test_visibility)
+// Argument checks, before any device is touched (c2rt.h): returns C2RT_OK with `noop` set for n == 0.
+int check_ray_args(const c2rt_scene* s, size_t n, const void* a, const void* b, bool any_out, bool& noop) {
+    noop = false;
+    if (!s) return fail(C2RT_ERR_INVALID_ARG, "scene is null");
+    if (!any_out) return fail(C2RT_ERR_INVALID_ARG, "every ray-query output is null");
+    if (n > (size_t)INT32_MAX) return fail(C2RT_ERR_LIMIT, "%zu ray queries: at most 2^31 - 1 per call", n);
+    if (n == 0) { noop = true; return C2RT_OK; }
+    if (!a || !b) return fail(C2RT_ERR_INVALID_ARG, "a ray-query input array is null");
+    return C2RT_OK;
+}
+bool any_ray_output(const c2rt_ray_hits* o) { return o && (o->node || o->dist || o->p || o->normal || o->uv); }
+
+// The queries [first, first + count) of device slot i in an n-device call: contiguous chunks of whole CTAs
+void ray_chunk_range(size_t total, int i, int n, size_t& first, size_t& count) {
+    const size_t ctas = (total + BLOCK_THREADS - 1) / BLOCK_THREADS, per = (ctas + n - 1) / n * BLOCK_THREADS;
+    first = std::min(total, (size_t)i * per);
+    count = std::min(total - first, per);
+}
+
+// Device slot i's chunk of a blocking ray-query call: inputs up, one launch, outputs down (every copy on the slot's stream,
+// from and to the caller's host arrays).  `hits` null: a visibility call into `visible`.
+int ray_chunk(int i, int n_dev, c2rt_scene* s, size_t total, const double* a, const double* b, const c2rt_ray_hits* hits,
+              uint8_t* visible, uint32_t* launches_out, float* kernel_ms_out) {
+    DeviceCtx& c = g_ctx.d[i];
+    CU(cudaSetDevice(c.dev));
+    size_t first, m;
+    ray_chunk_range(total, i, n_dev, first, m);
+    *launches_out = 0;
+    *kernel_ms_out = 0.f;
+    if (m == 0) return C2RT_OK;
+    // device layout, each plane at a multiple of the CTA-rounded chunk (16-byte aligned): a, b, then
+    // dist, p, normal, uv, node (closest hit) or visible (visibility)
+    const size_t mp = (m + BLOCK_THREADS - 1) / BLOCK_THREADS * BLOCK_THREADS;
+    int rc = grow_buffer(c.d_rays, c.rays_cap, mp * (hits ? 16 : 7));
+    if (rc) return rc;
+    double* d = c.d_rays;
+    RayParams rp;
+    memset(&rp, 0, sizeof rp);
+    rp.a = d; rp.b = d + 3 * mp;
+    rp.bounds = s->d_bounds[i];
+    rp.n = (uint32_t)m;
+    struct Out {
+        void* host;
+        void* dev;
+        size_t bytes;
+    } outs[5] = {};
+    if (hits) {
+        rp.hits.dist = hits->dist ? d + 6 * mp : nullptr;
+        rp.hits.p = hits->p ? d + 7 * mp : nullptr;
+        rp.hits.normal = hits->normal ? d + 10 * mp : nullptr;
+        rp.hits.uv = hits->uv ? d + 13 * mp : nullptr;
+        rp.hits.node = hits->node ? (int32_t*)(d + 15 * mp) : nullptr;
+        outs[0] = {hits->dist ? hits->dist + first : nullptr, rp.hits.dist, m * sizeof(double)};
+        outs[1] = {hits->p ? hits->p + 3 * first : nullptr, rp.hits.p, 3 * m * sizeof(double)};
+        outs[2] = {hits->normal ? hits->normal + 3 * first : nullptr, rp.hits.normal, 3 * m * sizeof(double)};
+        outs[3] = {hits->uv ? hits->uv + 2 * first : nullptr, rp.hits.uv, 2 * m * sizeof(double)};
+        outs[4] = {hits->node ? hits->node + first : nullptr, rp.hits.node, m * sizeof(int32_t)};
+    } else {
+        rp.visible = (uint8_t*)(d + 6 * mp);
+        outs[0] = {visible + first, rp.visible, m};
+    }
+    CU(cudaMemcpyAsync((void*)rp.a, a + 3 * first, 3 * m * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    CU(cudaMemcpyAsync((void*)rp.b, b + 3 * first, 3 * m * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    CU(cudaEventRecord(c.e0, c.stream));
+    if (hits) CU(launch_rays(rp, s->mode, c.stream));
+    else CU(launch_visibility(rp, s->mode, c.stream));
+    CU(cudaEventRecord(c.e1, c.stream));
+    for (const Out& o : outs)
+        if (o.host) CU(cudaMemcpyAsync(o.host, o.dev, o.bytes, cudaMemcpyDeviceToHost, c.stream));
+    CU(cudaStreamSynchronize(c.stream));
+    CU(cudaEventElapsedTime(kernel_ms_out, c.e0, c.e1));
+    *launches_out = 1;
+    return C2RT_OK;
+}
+
+// The blocking form of both queries (lock not held): checks, then every device's chunk (run_devices_locked)
+int rays_host(c2rt_scene* s, size_t n, const double* a, const double* b, const c2rt_ray_hits* hits, uint8_t* visible,
+              c2rt_stats* stats) {
+    const auto t0 = std::chrono::steady_clock::now();
+    bool noop;
+    int rc = check_ray_args(s, n, a, b, hits ? any_ray_output(hits) : visible != nullptr, noop);
+    if (rc) return rc;
+    if (stats) memset(stats, 0, sizeof *stats);
+    if (noop) return C2RT_OK;
+    std::lock_guard<std::mutex> g(g_mu);
+    rc = ensure_init_locked();
+    if (rc) return rc;
+    if (s->n_dev != g_ctx.n) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
+    uint32_t launches;
+    double kernel_ms;
+    rc = run_devices_locked(
+        s, [&](int i, uint32_t* l, float* ms) { return ray_chunk(i, g_ctx.n, s, n, a, b, hits, visible, l, ms); }, launches,
+        kernel_ms);
+    if (rc) return rc;
+    if (stats) {
+        stats->kernel_ms = kernel_ms;
+        stats->n_gpus = (uint32_t)g_ctx.n;
+        stats->launches = launches;
+        stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    return C2RT_OK;
+}
+
+// The device form of both queries: the caller's current device and stream, device arrays
+int rays_device(c2rt_scene* s, size_t n, const double* a, const double* b, const c2rt_ray_hits* hits, uint8_t* visible,
+                void* stream, c2rt_stats* stats) {
+    bool noop;
+    int rc = check_ray_args(s, n, a, b, hits ? any_ray_output(hits) : visible != nullptr, noop);
+    if (rc) return rc;
+    if (stats) memset(stats, 0, sizeof *stats);
+    if (noop) return C2RT_OK;
+    std::lock_guard<std::mutex> g(g_mu);
+    const cudaStream_t st = (cudaStream_t)stream;
+    DeviceCtx* c;
+    rc = current_device_locked(c);
+    if (rc) return rc;
+    const int di = (int)(c - g_ctx.d);
+    if (di >= s->n_dev) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
+    rc = make_resident(s, di, st);
+    if (rc) return rc;
+    RayParams rp;
+    memset(&rp, 0, sizeof rp);
+    rp.a = a; rp.b = b;
+    rp.bounds = s->d_bounds[di];
+    rp.n = (uint32_t)n;
+    if (hits) {
+        rp.hits = *hits;
+        CU(launch_rays(rp, s->mode, st));
+    } else {
+        rp.visible = visible;
+        CU(launch_visibility(rp, s->mode, st));
+    }
+    if (stats) {
+        stats->n_gpus = 1;
+        stats->launches = 1;
+    }
     return C2RT_OK;
 }
 
@@ -1276,6 +1428,27 @@ int c2rt_render_hits_device(c2rt_scene* s, const c2rt_camera* cam, const c2rt_se
         stats->launches = 1;
     }
     return C2RT_OK;
+}
+
+int c2rt_trace_rays(c2rt_scene* s, size_t n, const double* origins, const double* dirs, const c2rt_ray_hits* host_out,
+                    c2rt_stats* stats) {
+    if (!host_out) return fail(C2RT_ERR_INVALID_ARG, "every ray-query output is null");
+    return rays_host(s, n, origins, dirs, host_out, nullptr, stats);
+}
+
+int c2rt_trace_rays_device(c2rt_scene* s, size_t n, const double* d_origins, const double* d_dirs, const c2rt_ray_hits* device_out,
+                           void* stream, c2rt_stats* stats) {
+    if (!device_out) return fail(C2RT_ERR_INVALID_ARG, "every ray-query output is null");
+    return rays_device(s, n, d_origins, d_dirs, device_out, nullptr, stream, stats);
+}
+
+int c2rt_test_visibility(c2rt_scene* s, size_t n, const double* from, const double* to, uint8_t* visible, c2rt_stats* stats) {
+    return rays_host(s, n, from, to, nullptr, visible, stats);
+}
+
+int c2rt_test_visibility_device(c2rt_scene* s, size_t n, const double* d_from, const double* d_to, uint8_t* d_visible, void* stream,
+                                c2rt_stats* stats) {
+    return rays_device(s, n, d_from, d_to, nullptr, d_visible, stream, stats);
 }
 
 int c2rt_deinterleave(const void* gathered, void* frame, uint32_t width, uint32_t height, uint32_t elem_words, uint32_t n_ranks,

@@ -192,6 +192,17 @@ constexpr uint32_t rng_u31(uint64_t seed, uint32_t px, uint32_t py, uint32_t tap
     return h >> 1;
 }
 
+// One launch of ray queries (c2rt.h c2rt_trace_rays / c2rt_test_visibility; render_kernel.cu ray_query_kernel,
+// visibility_kernel): n queries of two [n*3] FP64 input arrays (origins / dirs, or from / to) in device memory
+struct RayParams {
+    const double* a;          // origins | from
+    const double* b;          // dirs | to
+    c2rt_ray_hits hits;       // closest-hit outputs (each nullable)
+    uint8_t* visible;         // visibility output
+    const float4* bounds;     // the scene's node bounding spheres on this device (FrameParams.bounds)
+    uint32_t n;
+};
+
 // renderer.d:46-57 renderPixel: what render_pixel_kernel writes for c2rt_render_pixel
 struct PixelOut {
     float rgb[3];

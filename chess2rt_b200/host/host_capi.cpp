@@ -129,6 +129,35 @@ int c2rt_host_render_hits(c2rt_host_scene* h, const c2rt_hit_planes* planes, uin
     }
 }
 
+// the closest hit of n caller-supplied rays into caller-owned HOST arrays (c2rt_trace_rays)
+int c2rt_host_trace_rays(c2rt_host_scene* h, size_t n, const double* origins, const double* dirs, const c2rt_ray_hits* out,
+                         c2rt_stats* stats) {
+    try {
+        c2rt_scene* dev = c2rt_host_device_scene(h);
+        if (!dev) return C2RT_ERR_CUDA;
+        int rc = c2rt_trace_rays(dev, n, origins, dirs, out, stats);
+        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
+        return rc;
+    } catch (const std::exception& e) {
+        g_host_err = e.what();
+        return C2RT_ERR_INVALID_ARG;
+    }
+}
+
+// testVisibility(from[i], to[i]) for n pairs into a caller-owned HOST array (c2rt_test_visibility)
+int c2rt_host_test_visibility(c2rt_host_scene* h, size_t n, const double* from, const double* to, uint8_t* visible, c2rt_stats* stats) {
+    try {
+        c2rt_scene* dev = c2rt_host_device_scene(h);
+        if (!dev) return C2RT_ERR_CUDA;
+        int rc = c2rt_test_visibility(dev, n, from, to, visible, stats);
+        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
+        return rc;
+    } catch (const std::exception& e) {
+        g_host_err = e.what();
+        return C2RT_ERR_INVALID_ARG;
+    }
+}
+
 // renderPixel(scene, output, x, y) (renderer.d:46-57)
 int c2rt_host_render_pixel(c2rt_host_scene* h, int x, int y, float rgb[3], c2rt_hit* hit) {
     try {

@@ -76,6 +76,40 @@ void Renderer::renderHits(HitPlanes& planes) {
     if (rc != C2RT_OK) raise(rc);
 }
 
+namespace {
+std::vector<double> flattenVectors(const std::vector<Vector>& v) {
+    std::vector<double> out(v.size() * 3);
+    for (size_t i = 0; i < v.size(); i++) { out[3 * i] = v[i].x; out[3 * i + 1] = v[i].y; out[3 * i + 2] = v[i].z; }
+    return out;
+}
+}  // namespace
+
+void Renderer::traceRays(const std::vector<Vector>& orig, const std::vector<Vector>& dir, RayHits& hits) {
+    const size_t n = orig.size();
+    if (dir.size() != n) throw RTException("traceRays: as many directions as origins are needed");
+    if ((!hits.node.empty() && hits.node.size() != n) || (!hits.dist.empty() && hits.dist.size() != n) ||
+        (!hits.p.empty() && hits.p.size() != 3 * n) || (!hits.normal.empty() && hits.normal.size() != 3 * n) ||
+        (!hits.uv.empty() && hits.uv.size() != 2 * n))
+        throw RTException("ray hit plane size does not match the number of rays");
+    const std::vector<double> o = flattenVectors(orig), d = flattenVectors(dir);
+    c2rt_ray_hits p;
+    p.node = hits.node.empty() ? nullptr : hits.node.data();
+    p.dist = hits.dist.empty() ? nullptr : hits.dist.data();
+    p.p = hits.p.empty() ? nullptr : hits.p.data();
+    p.normal = hits.normal.empty() ? nullptr : hits.normal.data();
+    p.uv = hits.uv.empty() ? nullptr : hits.uv.data();
+    int rc = c2rt_trace_rays(device(), n, o.data(), d.data(), &p, &lastStats);
+    if (rc != C2RT_OK) raise(rc);
+}
+
+void Renderer::testVisibility(const std::vector<Vector>& from, const std::vector<Vector>& to, std::vector<uint8_t>& visible) {
+    if (to.size() != from.size()) throw RTException("testVisibility: as many `to` points as `from` points are needed");
+    const std::vector<double> f = flattenVectors(from), t = flattenVectors(to);
+    visible.resize(from.size());
+    int rc = c2rt_test_visibility(device(), from.size(), f.data(), t.data(), visible.data(), &lastStats);
+    if (rc != C2RT_OK) raise(rc);
+}
+
 void requestStop(std::atomic<bool>* isStopRequested) {
     if (isStopRequested) isStopRequested->store(true);
     c2rt_cancel();

@@ -42,6 +42,16 @@ struct HitPlanes {
     std::vector<float> uv;       // [W*H*2] u, v, 0 for a miss
 };
 
+// The closest-hit records of caller-supplied rays (c2rt_trace_rays): one entry per ray, structure of arrays.  traceRays fills
+// the planes that are not empty; a non-empty plane must hold exactly as many records as there are rays.
+struct RayHits {
+    std::vector<int32_t> node;   // [n] closestNode, -1 = miss
+    std::vector<double> dist;    // [n] distance along the unit direction, +inf for a miss
+    std::vector<double> p;       // [n*3] world-space hit point, 0 for a miss
+    std::vector<double> normal;  // [n*3] unit geometric normal, 0 for a miss
+    std::vector<double> uv;      // [n*2] u, v, 0 for a miss
+};
+
 struct Renderer {
     Renderer(const Scene& scene, Image<Color>& output, std::atomic<bool>* isRendering = nullptr,
              const std::atomic<bool>* isStopRequested = nullptr);
@@ -49,6 +59,10 @@ struct Renderer {
     void renderRT();                               // renderer.d:83-189
     void renderHits(HitPlanes& planes);            // no counterpart: renderPixelNoAA's hit record for every pixel, no colour
     Color renderPixelNoAA(int x, int y);           // renderer.d:223-228 (also records lastTracingResult)
+    // renderer.d:325-376's closest-hit loop on (orig[i], normalize(dir[i])) for every i (c2rt_trace_rays)
+    void traceRays(const std::vector<Vector>& orig, const std::vector<Vector>& dir, RayHits& hits);
+    // scene.d:62-78 testVisibility(from[i], to[i]) for every i: visible[i] = 1 or 0 (c2rt_test_visibility)
+    void testVisibility(const std::vector<Vector>& from, const std::vector<Vector>& to, std::vector<uint8_t>& visible);
 
     TraceResult lastTracingResult;
     c2rt_stats lastStats{};

@@ -283,6 +283,42 @@ int c2rt_render_hits(c2rt_scene* scene, const c2rt_camera* camera, const c2rt_se
 int c2rt_render_hits_device(c2rt_scene* scene, const c2rt_camera* camera, const c2rt_settings* settings,
                             const c2rt_band* band, const c2rt_hit_planes* device_planes, void* stream, c2rt_stats* stats);
 
+/* Ray queries: the reference's two scene queries for rays the caller chooses, n queries per call, one thread each.
+ *   c2rt_trace_rays       the closest-hit loop of trace / renderPixel (renderer.d:325-376) on the ray (origin, normalize(dir)):
+ *                         the walk starts at dist = 1e99, visits the nodes in scene order, and the last node that reports a hit
+ *                         wins.  The direction is normalised on the device in FP64, as camera rays are.
+ *   c2rt_test_visibility  Scene.testVisibility(from, to) (scene.d:62-78): the ray from `from` towards normalize(to - from) is
+ *                         occluded iff some node, planes included, hits it at a distance <= |to - from|.
+ * A query is traced only when its six coordinates are finite and the squared length of its direction (dir, or to - from) is
+ * positive and finite in FP64.  Any other query (a zero direction, from == to, a NaN or an infinity) is a miss, or visible = 1.
+ * Each result depends on the scene and that one query only: not on the other queries, their order, n or the devices.
+ * No camera, settings or GI rule applies; the ray counters and the cancel flag are neither read nor changed; the scene is
+ * made resident on the device by the residency rule of the frame calls.
+ * n == 0 is a no-op.  A null scene, all outputs null, or a null input with n > 0 is C2RT_ERR_INVALID_ARG; n > 2^31 - 1 is
+ * C2RT_ERR_LIMIT.  These checks come before any device is touched.
+ * Speed: the 32 consecutive queries of a warp share one node mask, so batches whose runs of 32 queries are close in origin
+ * and direction (e.g. 8x4 pixel patches of a camera) skip most nodes; incoherent batches walk every node. */
+typedef struct c2rt_ray_hits {   /* every pointer may be NULL; at least one must not be */
+    int32_t* node;     /* [n]   closest node, -1 = miss */
+    double* dist;      /* [n]   distance along the unit direction, +inf for a miss */
+    double* p;         /* [n*3] world-space hit point, 0 for a miss */
+    double* normal;    /* [n*3] unit geometric normal as c2rt_hit reports it (CsgDiff flip applied, not face-forwarded), 0 for a miss */
+    double* uv;        /* [n*2] u, v, 0 for a miss */
+} c2rt_ray_hits;
+
+/* Blocking, HOST arrays ([n*3] doubles each in, host_out planes out).  With n_gpus > 1 the queries are split into n_gpus
+ * contiguous chunks of whole CTAs; every device uploads its chunk, runs it and copies its results back over its own link.
+ * stats (nullable): kernel_ms, total_ms, n_gpus, launches. */
+int c2rt_trace_rays(c2rt_scene* scene, size_t n, const double* origins, const double* dirs, const c2rt_ray_hits* host_out,
+                    c2rt_stats* stats);
+/* The same on DEVICE arrays of the current device, async on `stream`.  stats (nullable) gets launches only. */
+int c2rt_trace_rays_device(c2rt_scene* scene, size_t n, const double* d_origins, const double* d_dirs,
+                           const c2rt_ray_hits* device_out, void* stream, c2rt_stats* stats);
+/* visible[i] = 1 when nothing occludes the segment from[i] -> to[i], 0 when something does.  Host / device forms as above. */
+int c2rt_test_visibility(c2rt_scene* scene, size_t n, const double* from, const double* to, uint8_t* visible, c2rt_stats* stats);
+int c2rt_test_visibility_device(c2rt_scene* scene, size_t n, const double* d_from, const double* d_to, uint8_t* d_visible,
+                                void* stream, c2rt_stats* stats);
+
 /* Number of rows rank `rank` owns in a frame of `height` rows. */
 uint32_t c2rt_band_rows_owned(uint32_t height, uint32_t rank, uint32_t n_ranks, uint32_t band_rows);
 
