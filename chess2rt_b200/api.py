@@ -91,7 +91,8 @@ C_ABI_SYMBOLS = [
     "c2rt_init", "c2rt_shutdown", "c2rt_abi_version", "c2rt_device_count", "c2rt_last_error",
     "c2rt_scene_create", "c2rt_scene_destroy", "c2rt_render", "c2rt_cancel", "c2rt_render_device", "c2rt_read_ray_counters",
     "c2rt_deinterleave", "c2rt_render_pixel", "c2rt_render_hits", "c2rt_render_hits_device",
-    "c2rt_trace_rays", "c2rt_trace_rays_device", "c2rt_test_visibility", "c2rt_test_visibility_device", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
+    "c2rt_trace_rays", "c2rt_trace_rays_device", "c2rt_test_visibility", "c2rt_test_visibility_device",
+    "c2rt_shade_rays", "c2rt_shade_rays_device", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
     "c2rt_frame_alloc", "c2rt_frame_free", "c2rt_frame_export", "c2rt_frame_import", "c2rt_frame_unimport", "c2rt_frame_memset", "c2rt_frame_download", "c2rt_pin_host_buffer", "c2rt_unpin_host_buffer", "c2rt_gate",
     "c2rt_measure_fma_peak", "c2rt_selftest_device_pool",
 ]
@@ -120,6 +121,10 @@ lib.c2rt_trace_rays_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_v
 lib.c2rt_test_visibility.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Stats)]
 lib.c2rt_test_visibility_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.POINTER(Stats)]
+lib.c2rt_shade_rays.argtypes = [C.c_void_p, C.POINTER(C.c_float), C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.POINTER(Stats)]
+lib.c2rt_shade_rays_device.argtypes = [C.c_void_p, C.POINTER(C.c_float), C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.POINTER(Stats)]
 lib.c2rt_band_rows_owned.argtypes = [C.c_uint32] * 4
 lib.c2rt_band_rows_owned.restype = C.c_uint32
 lib.c2rt_rng_u31.argtypes = [C.c_uint64] + [C.c_uint32] * 5
@@ -160,6 +165,7 @@ host_lib.c2rt_host_render_pixel.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POIN
 host_lib.c2rt_host_render_hits.argtypes = [C.c_void_p, C.POINTER(HitPlanes), C.c_uint64, C.POINTER(Stats)]
 host_lib.c2rt_host_trace_rays.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.POINTER(RayHits), C.POINTER(Stats)]
 host_lib.c2rt_host_test_visibility.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Stats)]
+host_lib.c2rt_host_shade_rays.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Stats)]
 host_lib.c2rt_host_camera_rotate.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_double]
 host_lib.c2rt_host_camera_rotate.restype = None
 host_lib.c2rt_host_camera_move.argtypes = [C.c_void_p, C.c_double, C.c_double, C.c_double]
@@ -337,6 +343,21 @@ class HostScene:
         _check_host(host_lib.c2rt_host_test_visibility(self._h, len(f), f.ctypes.data, t.ctypes.data, vis.ctypes.data, C.byref(st)))
         return vis.astype(bool), st
 
+    def shade_rays(self, origins, dirs, argb=False):
+        """trace((origins[i], normalize(dirs[i]))) at depth 0 with the scene file's ambientLightColor (c2rt_shade_rays) ->
+        (rgb [n, 3] float32, argb [n] uint32 (Color.toRGB32) or None, Stats).  origins and dirs: [n, 3] float64.  An untraced
+        query (a non-finite coordinate, a zero direction) is (0, 0, 0) and 0."""
+        o, d = _points(origins), _points(dirs)
+        if o.shape != d.shape:
+            raise ValueError(f"origins {o.shape} and dirs {d.shape} differ in shape")
+        n = len(o)
+        rgb = np.empty((n, 3), np.float32)
+        a = np.empty(n, np.uint32) if argb else None
+        st = Stats()
+        _check_host(host_lib.c2rt_host_shade_rays(self._h, n, o.ctypes.data, d.ctypes.data, rgb.ctypes.data,
+                                                  a.ctypes.data if a is not None else None, C.byref(st)))
+        return rgb, a, st
+
 
 def _points(a):
     a = np.ascontiguousarray(a, np.float64)
@@ -390,6 +411,13 @@ def trace_rays_device(scene_handle, n, d_origins, d_dirs, node=None, dist=None, 
 def test_visibility_device(scene_handle, n, d_from, d_to, d_visible, stream=None):
     """c2rt_test_visibility_device: [n*3] float64 inputs and the [n] uint8 output as device pointers, async on `stream`."""
     _check(lib.c2rt_test_visibility_device(scene_handle, n, d_from, d_to, d_visible, stream, None))
+
+
+def shade_rays_device(scene_handle, n, d_origins, d_dirs, ambient, d_rgb=None, d_argb=None, stream=None):
+    """c2rt_shade_rays_device: [n*3] float64 inputs, the [n*3] float32 rgb and [n] uint32 argb outputs as device pointers (ints;
+    None = not wanted), `ambient` three floats on the host, async on `stream` (int cudaStream_t or None)."""
+    amb = (C.c_float * 3)(*ambient)
+    _check(lib.c2rt_shade_rays_device(scene_handle, amb, n, d_origins, d_dirs, d_rgb, d_argb, stream, None))
 
 
 def read_ray_counters(scene_handle, stream=None):

@@ -29,6 +29,7 @@ cudaError_t launch_pixel(const FrameParams& fp, int mode, int x, int y, PixelOut
 cudaError_t launch_hits(const FrameParams& fp, int mode, uint32_t local_tile_rows, const c2rt_hit_planes& out, cudaStream_t st);
 cudaError_t launch_rays(const RayParams& rp, int mode, cudaStream_t st);
 cudaError_t launch_visibility(const RayParams& rp, int mode, cudaStream_t st);
+cudaError_t launch_shade_rays(const RayParams& rp, const FrameParams& fp, int mode, cudaStream_t st);
 cudaError_t launch_deinterleave(const void* src, void* dst, uint32_t row_words, uint32_t height, uint32_t n_ranks,
                                 uint32_t band_rows, uint32_t rows_pad, cudaStream_t st);
 cudaError_t launch_fma_peak(bool fp64, int blocks, int threads, int iters, void* d_out, cudaStream_t st);
@@ -73,7 +74,7 @@ struct DeviceCtx {
     float* d_rgb = nullptr;
     uint32_t* d_argb = nullptr;
     uint32_t* d_hits = nullptr;   // the four planes of a c2rt_render_hits frame, one after the other
-    double* d_rays = nullptr;     // a c2rt_trace_rays / c2rt_test_visibility chunk: its inputs, then its output planes
+    double* d_rays = nullptr;     // a c2rt_trace_rays / c2rt_test_visibility / c2rt_shade_rays chunk: its inputs, then its output planes
     size_t rgb_cap = 0, argb_cap = 0, hits_cap = 0, rays_cap = 0;
 };
 
@@ -1008,7 +1009,20 @@ int render_devices_locked(c2rt_scene* s, const c2rt_camera* cam, const c2rt_sett
         kernel_ms);
 }
 
-// ---- ray queries (c2rt_trace_rays, c2rt_test_visibility)
+// ---- ray queries (c2rt_trace_rays, c2rt_test_visibility, c2rt_shade_rays)
+// The outputs of one ray-query call, in host or device memory: closest-hit planes, visibility bytes, or colours
+struct RayOut {
+    const c2rt_ray_hits* hits = nullptr;   // c2rt_trace_rays
+    uint8_t* visible = nullptr;            // c2rt_test_visibility
+    const float* ambient = nullptr;        // c2rt_shade_rays (a host pointer in both forms): rgb [n*3] / argb [n], each nullable
+    float* rgb = nullptr;
+    uint32_t* argb = nullptr;
+    bool any() const {
+        if (hits) return hits->node || hits->dist || hits->p || hits->normal || hits->uv;
+        return ambient ? (rgb || argb) : visible != nullptr;
+    }
+};
+
 // Argument checks, before any device is touched (c2rt.h): returns C2RT_OK with `noop` set for n == 0.
 int check_ray_args(const c2rt_scene* s, size_t n, const void* a, const void* b, bool any_out, bool& noop) {
     noop = false;
@@ -1019,7 +1033,17 @@ int check_ray_args(const c2rt_scene* s, size_t n, const void* a, const void* b, 
     if (!a || !b) return fail(C2RT_ERR_INVALID_ARG, "a ray-query input array is null");
     return C2RT_OK;
 }
-bool any_ray_output(const c2rt_ray_hits* o) { return o && (o->node || o->dist || o->p || o->normal || o->uv); }
+
+// The shading parameters of a c2rt_shade_rays launch on device slot c: the ambient term and the node bounds trace_warp reads at
+// depth 0, the sRGB table and the output planes; no camera, band, counter or cancel flag (all 0)
+void shade_params(FrameParams& fp, const c2rt_scene* s, const DeviceCtx& c, int di, const float* ambient, float* rgb, uint32_t* argb) {
+    memset(&fp, 0, sizeof fp);
+    for (int k = 0; k < 3; k++) fp.ambient[k] = ambient[k];
+    fp.bounds = s->d_bounds[di];
+    fp.lut = c.d_lut;
+    fp.rgb = rgb;
+    fp.argb = argb;
+}
 
 // The queries [first, first + count) of device slot i in an n-device call: contiguous chunks of whole CTAs
 void ray_chunk_range(size_t total, int i, int n, size_t& first, size_t& count) {
@@ -1029,9 +1053,9 @@ void ray_chunk_range(size_t total, int i, int n, size_t& first, size_t& count) {
 }
 
 // Device slot i's chunk of a blocking ray-query call: inputs up, one launch, outputs down (every copy on the slot's stream,
-// from and to the caller's host arrays).  `hits` null: a visibility call into `visible`.
-int ray_chunk(int i, int n_dev, c2rt_scene* s, size_t total, const double* a, const double* b, const c2rt_ray_hits* hits,
-              uint8_t* visible, uint32_t* launches_out, float* kernel_ms_out) {
+// from and to the caller's host arrays `out`).
+int ray_chunk(int i, int n_dev, c2rt_scene* s, size_t total, const double* a, const double* b, const RayOut& out,
+              uint32_t* launches_out, float* kernel_ms_out) {
     DeviceCtx& c = g_ctx.d[i];
     CU(cudaSetDevice(c.dev));
     size_t first, m;
@@ -1040,9 +1064,9 @@ int ray_chunk(int i, int n_dev, c2rt_scene* s, size_t total, const double* a, co
     *kernel_ms_out = 0.f;
     if (m == 0) return C2RT_OK;
     // device layout, each plane at a multiple of the CTA-rounded chunk (16-byte aligned): a, b, then
-    // dist, p, normal, uv, node (closest hit) or visible (visibility)
+    // dist, p, normal, uv, node (closest hit), visible (visibility) or rgb, argb (colour)
     const size_t mp = (m + BLOCK_THREADS - 1) / BLOCK_THREADS * BLOCK_THREADS;
-    int rc = grow_buffer(c.d_rays, c.rays_cap, mp * (hits ? 16 : 7));
+    int rc = grow_buffer(c.d_rays, c.rays_cap, mp * (out.hits ? 16 : out.ambient ? 8 : 7));
     if (rc) return rc;
     double* d = c.d_rays;
     RayParams rp;
@@ -1050,12 +1074,13 @@ int ray_chunk(int i, int n_dev, c2rt_scene* s, size_t total, const double* a, co
     rp.a = d; rp.b = d + 3 * mp;
     rp.bounds = s->d_bounds[i];
     rp.n = (uint32_t)m;
+    FrameParams fp;
     struct Out {
         void* host;
         void* dev;
         size_t bytes;
     } outs[5] = {};
-    if (hits) {
+    if (const c2rt_ray_hits* hits = out.hits) {
         rp.hits.dist = hits->dist ? d + 6 * mp : nullptr;
         rp.hits.p = hits->p ? d + 7 * mp : nullptr;
         rp.hits.normal = hits->normal ? d + 10 * mp : nullptr;
@@ -1066,14 +1091,21 @@ int ray_chunk(int i, int n_dev, c2rt_scene* s, size_t total, const double* a, co
         outs[2] = {hits->normal ? hits->normal + 3 * first : nullptr, rp.hits.normal, 3 * m * sizeof(double)};
         outs[3] = {hits->uv ? hits->uv + 2 * first : nullptr, rp.hits.uv, 2 * m * sizeof(double)};
         outs[4] = {hits->node ? hits->node + first : nullptr, rp.hits.node, m * sizeof(int32_t)};
+    } else if (out.ambient) {
+        float* rgb = (float*)(d + 6 * mp);
+        uint32_t* argb = (uint32_t*)(rgb + 3 * mp);
+        shade_params(fp, s, c, i, out.ambient, out.rgb ? rgb : nullptr, out.argb ? argb : nullptr);
+        outs[0] = {out.rgb ? out.rgb + 3 * first : nullptr, rgb, 3 * m * sizeof(float)};
+        outs[1] = {out.argb ? out.argb + first : nullptr, argb, m * sizeof(uint32_t)};
     } else {
         rp.visible = (uint8_t*)(d + 6 * mp);
-        outs[0] = {visible + first, rp.visible, m};
+        outs[0] = {out.visible + first, rp.visible, m};
     }
     CU(cudaMemcpyAsync((void*)rp.a, a + 3 * first, 3 * m * sizeof(double), cudaMemcpyHostToDevice, c.stream));
     CU(cudaMemcpyAsync((void*)rp.b, b + 3 * first, 3 * m * sizeof(double), cudaMemcpyHostToDevice, c.stream));
     CU(cudaEventRecord(c.e0, c.stream));
-    if (hits) CU(launch_rays(rp, s->mode, c.stream));
+    if (out.hits) CU(launch_rays(rp, s->mode, c.stream));
+    else if (out.ambient) CU(launch_shade_rays(rp, fp, s->mode, c.stream));
     else CU(launch_visibility(rp, s->mode, c.stream));
     CU(cudaEventRecord(c.e1, c.stream));
     for (const Out& o : outs)
@@ -1084,12 +1116,11 @@ int ray_chunk(int i, int n_dev, c2rt_scene* s, size_t total, const double* a, co
     return C2RT_OK;
 }
 
-// The blocking form of both queries (lock not held): checks, then every device's chunk (run_devices_locked)
-int rays_host(c2rt_scene* s, size_t n, const double* a, const double* b, const c2rt_ray_hits* hits, uint8_t* visible,
-              c2rt_stats* stats) {
+// The blocking form of every query (lock not held): checks, then every device's chunk (run_devices_locked)
+int rays_host(c2rt_scene* s, size_t n, const double* a, const double* b, const RayOut& out, c2rt_stats* stats) {
     const auto t0 = std::chrono::steady_clock::now();
     bool noop;
-    int rc = check_ray_args(s, n, a, b, hits ? any_ray_output(hits) : visible != nullptr, noop);
+    int rc = check_ray_args(s, n, a, b, out.any(), noop);
     if (rc) return rc;
     if (stats) memset(stats, 0, sizeof *stats);
     if (noop) return C2RT_OK;
@@ -1100,8 +1131,7 @@ int rays_host(c2rt_scene* s, size_t n, const double* a, const double* b, const c
     uint32_t launches;
     double kernel_ms;
     rc = run_devices_locked(
-        s, [&](int i, uint32_t* l, float* ms) { return ray_chunk(i, g_ctx.n, s, n, a, b, hits, visible, l, ms); }, launches,
-        kernel_ms);
+        s, [&](int i, uint32_t* l, float* ms) { return ray_chunk(i, g_ctx.n, s, n, a, b, out, l, ms); }, launches, kernel_ms);
     if (rc) return rc;
     if (stats) {
         stats->kernel_ms = kernel_ms;
@@ -1112,11 +1142,10 @@ int rays_host(c2rt_scene* s, size_t n, const double* a, const double* b, const c
     return C2RT_OK;
 }
 
-// The device form of both queries: the caller's current device and stream, device arrays
-int rays_device(c2rt_scene* s, size_t n, const double* a, const double* b, const c2rt_ray_hits* hits, uint8_t* visible,
-                void* stream, c2rt_stats* stats) {
+// The device form of every query: the caller's current device and stream, device arrays
+int rays_device(c2rt_scene* s, size_t n, const double* a, const double* b, const RayOut& out, void* stream, c2rt_stats* stats) {
     bool noop;
-    int rc = check_ray_args(s, n, a, b, hits ? any_ray_output(hits) : visible != nullptr, noop);
+    int rc = check_ray_args(s, n, a, b, out.any(), noop);
     if (rc) return rc;
     if (stats) memset(stats, 0, sizeof *stats);
     if (noop) return C2RT_OK;
@@ -1134,11 +1163,15 @@ int rays_device(c2rt_scene* s, size_t n, const double* a, const double* b, const
     rp.a = a; rp.b = b;
     rp.bounds = s->d_bounds[di];
     rp.n = (uint32_t)n;
-    if (hits) {
-        rp.hits = *hits;
+    if (out.hits) {
+        rp.hits = *out.hits;
         CU(launch_rays(rp, s->mode, st));
+    } else if (out.ambient) {
+        FrameParams fp;
+        shade_params(fp, s, *c, di, out.ambient, out.rgb, out.argb);
+        CU(launch_shade_rays(rp, fp, s->mode, st));
     } else {
-        rp.visible = visible;
+        rp.visible = out.visible;
         CU(launch_visibility(rp, s->mode, st));
     }
     if (stats) {
@@ -1433,22 +1466,50 @@ int c2rt_render_hits_device(c2rt_scene* s, const c2rt_camera* cam, const c2rt_se
 int c2rt_trace_rays(c2rt_scene* s, size_t n, const double* origins, const double* dirs, const c2rt_ray_hits* host_out,
                     c2rt_stats* stats) {
     if (!host_out) return fail(C2RT_ERR_INVALID_ARG, "every ray-query output is null");
-    return rays_host(s, n, origins, dirs, host_out, nullptr, stats);
+    RayOut out;
+    out.hits = host_out;
+    return rays_host(s, n, origins, dirs, out, stats);
 }
 
 int c2rt_trace_rays_device(c2rt_scene* s, size_t n, const double* d_origins, const double* d_dirs, const c2rt_ray_hits* device_out,
                            void* stream, c2rt_stats* stats) {
     if (!device_out) return fail(C2RT_ERR_INVALID_ARG, "every ray-query output is null");
-    return rays_device(s, n, d_origins, d_dirs, device_out, nullptr, stream, stats);
+    RayOut out;
+    out.hits = device_out;
+    return rays_device(s, n, d_origins, d_dirs, out, stream, stats);
 }
 
 int c2rt_test_visibility(c2rt_scene* s, size_t n, const double* from, const double* to, uint8_t* visible, c2rt_stats* stats) {
-    return rays_host(s, n, from, to, nullptr, visible, stats);
+    RayOut out;
+    out.visible = visible;
+    return rays_host(s, n, from, to, out, stats);
 }
 
 int c2rt_test_visibility_device(c2rt_scene* s, size_t n, const double* d_from, const double* d_to, uint8_t* d_visible, void* stream,
                                 c2rt_stats* stats) {
-    return rays_device(s, n, d_from, d_to, nullptr, d_visible, stream, stats);
+    RayOut out;
+    out.visible = d_visible;
+    return rays_device(s, n, d_from, d_to, out, stream, stats);
+}
+
+int c2rt_shade_rays(c2rt_scene* s, const float ambient[3], size_t n, const double* origins, const double* dirs, float* rgb,
+                    uint32_t* argb, c2rt_stats* stats) {
+    if (s && !ambient) return fail(C2RT_ERR_INVALID_ARG, "ambient is null");
+    RayOut out;
+    out.ambient = ambient;
+    out.rgb = rgb;
+    out.argb = argb;
+    return rays_host(s, n, origins, dirs, out, stats);
+}
+
+int c2rt_shade_rays_device(c2rt_scene* s, const float ambient[3], size_t n, const double* d_origins, const double* d_dirs,
+                           float* d_rgb, uint32_t* d_argb, void* stream, c2rt_stats* stats) {
+    if (s && !ambient) return fail(C2RT_ERR_INVALID_ARG, "ambient is null");
+    RayOut out;
+    out.ambient = ambient;
+    out.rgb = d_rgb;
+    out.argb = d_argb;
+    return rays_device(s, n, d_origins, d_dirs, out, stream, stats);
 }
 
 int c2rt_deinterleave(const void* gathered, void* frame, uint32_t width, uint32_t height, uint32_t elem_words, uint32_t n_ranks,

@@ -192,8 +192,8 @@ constexpr uint32_t rng_u31(uint64_t seed, uint32_t px, uint32_t py, uint32_t tap
     return h >> 1;
 }
 
-// One launch of ray queries (c2rt.h c2rt_trace_rays / c2rt_test_visibility; render_kernel.cu ray_query_kernel,
-// visibility_kernel): n queries of two [n*3] FP64 input arrays (origins / dirs, or from / to) in device memory
+// One launch of ray queries (c2rt.h c2rt_trace_rays / c2rt_test_visibility / c2rt_shade_rays; render_kernel.cu ray_query_kernel,
+// visibility_kernel, shade_ray_kernel): n queries of two [n*3] FP64 input arrays (origins / dirs, or from / to) in device memory
 struct RayParams {
     const double* a;          // origins | from
     const double* b;          // dirs | to

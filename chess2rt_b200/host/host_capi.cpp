@@ -158,6 +158,24 @@ int c2rt_host_test_visibility(c2rt_host_scene* h, size_t n, const double* from, 
     }
 }
 
+// trace(ray) at depth 0 for n caller-supplied rays into caller-owned HOST arrays (c2rt_shade_rays; rgb / argb nullable), with
+// the scene file's ambientLightColor
+int c2rt_host_shade_rays(c2rt_host_scene* h, size_t n, const double* origins, const double* dirs, float* rgb, uint32_t* argb,
+                         c2rt_stats* stats) {
+    try {
+        const Color& amb = h->scene->settings.ambientLightColor;
+        const float ambient[3] = {amb.r, amb.g, amb.b};
+        c2rt_scene* dev = c2rt_host_device_scene(h);
+        if (!dev) return C2RT_ERR_CUDA;
+        int rc = c2rt_shade_rays(dev, ambient, n, origins, dirs, rgb, argb, stats);
+        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
+        return rc;
+    } catch (const std::exception& e) {
+        g_host_err = e.what();
+        return C2RT_ERR_INVALID_ARG;
+    }
+}
+
 // renderPixel(scene, output, x, y) (renderer.d:46-57)
 int c2rt_host_render_pixel(c2rt_host_scene* h, int x, int y, float rgb[3], c2rt_hit* hit) {
     try {

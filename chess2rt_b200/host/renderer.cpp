@@ -110,6 +110,21 @@ void Renderer::testVisibility(const std::vector<Vector>& from, const std::vector
     if (rc != C2RT_OK) raise(rc);
 }
 
+void Renderer::shadeRays(const std::vector<Vector>& orig, const std::vector<Vector>& dir, std::vector<Color>& out,
+                         std::vector<uint32_t>* argb) {
+    static_assert(sizeof(Color) == 3 * sizeof(float), "a Color[] is the rgb plane of c2rt_shade_rays");
+    const size_t n = orig.size();
+    if (dir.size() != n) throw RTException("shadeRays: as many directions as origins are needed");
+    const std::vector<double> o = flattenVectors(orig), d = flattenVectors(dir);
+    const Color& amb = scene_.settings.ambientLightColor;
+    const float ambient[3] = {amb.r, amb.g, amb.b};
+    out.resize(n);
+    if (argb) argb->resize(n);
+    int rc = c2rt_shade_rays(device(), ambient, n, o.data(), d.data(), reinterpret_cast<float*>(out.data()),
+                             argb ? argb->data() : nullptr, &lastStats);
+    if (rc != C2RT_OK) raise(rc);
+}
+
 void requestStop(std::atomic<bool>* isStopRequested) {
     if (isStopRequested) isStopRequested->store(true);
     c2rt_cancel();

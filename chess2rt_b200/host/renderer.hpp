@@ -63,6 +63,10 @@ struct Renderer {
     void traceRays(const std::vector<Vector>& orig, const std::vector<Vector>& dir, RayHits& hits);
     // scene.d:62-78 testVisibility(from[i], to[i]) for every i: visible[i] = 1 or 0 (c2rt_test_visibility)
     void testVisibility(const std::vector<Vector>& from, const std::vector<Vector>& to, std::vector<uint8_t>& visible);
+    // renderer.d:325-376 trace((orig[i], normalize(dir[i]))) at depth 0 for every i, with the scene's ambientLightColor
+    // (c2rt_shade_rays): out[i] is the colour; argb (optional) gets Color.toRGB32 of it
+    void shadeRays(const std::vector<Vector>& orig, const std::vector<Vector>& dir, std::vector<Color>& out,
+                   std::vector<uint32_t>* argb = nullptr);
 
     TraceResult lastTracingResult;
     c2rt_stats lastStats{};

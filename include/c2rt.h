@@ -319,6 +319,29 @@ int c2rt_test_visibility(c2rt_scene* scene, size_t n, const double* from, const 
 int c2rt_test_visibility_device(c2rt_scene* scene, size_t n, const double* d_from, const double* d_to, uint8_t* d_visible,
                                 void* stream, c2rt_stats* stats);
 
+/* Shaded ray queries: the colour Renderer.trace returns (renderer.d:325-376) for the ray (origin, normalize(dir)), depth 0 —
+ * the closest hit shaded by its Lambert or Phong shader with one shadow ray per lit light and the ambient term, or
+ * env_lookup(dir) for a miss (black, or the C2RT_ENV_CUBEMAP extension).  The shading is the colour frames' own code.
+ *   rgb   [n*3] FP32, laid out like Color[n] (nullable)
+ *   argb  [n]   Color.toRGB32 through the sRGB table (c2rt_srgb_table), bit-exact as in frames (nullable; not both null)
+ *   ambient  GlobalSettings.ambientLightColor, a HOST pointer in both forms: the only setting trace reads at depth 0.  GI does
+ *            not apply: this is trace, not pathtrace.
+ * A query is traced under the rule of c2rt_trace_rays; an untraced query gives rgb (0, 0, 0) and argb 0.  Each result depends
+ * on the scene, ambient and that one query only: not on the other queries, their order, n or the devices.  No camera, AA,
+ * DOF or stereo applies (the caller supplies the rays); the ray counters and the cancel flag are neither read nor changed; the
+ * scene is made resident by the residency rule of the frame calls.
+ * n == 0 is a no-op that zeroes stats.  A null scene, a null ambient, both outputs null, or a null input with n > 0 is
+ * C2RT_ERR_INVALID_ARG; n > 2^31 - 1 is C2RT_ERR_LIMIT.  These checks come before any device is touched.
+ * Speed: as for c2rt_trace_rays, runs of 32 queries close in origin and direction (a camera's 8x4 pixel patches, rows of a
+ * panorama) skip most nodes for the camera ray; shadow rays get their own per-warp node mask. */
+/* Blocking, HOST arrays; with n_gpus > 1 the queries are split into contiguous chunks of whole CTAs, as c2rt_trace_rays does.
+ * stats (nullable): kernel_ms, total_ms, n_gpus, launches. */
+int c2rt_shade_rays(c2rt_scene* scene, const float ambient[3], size_t n, const double* origins, const double* dirs, float* rgb,
+                    uint32_t* argb, c2rt_stats* stats);
+/* The same on DEVICE arrays of the current device, async on `stream`.  stats (nullable) gets launches only. */
+int c2rt_shade_rays_device(c2rt_scene* scene, const float ambient[3], size_t n, const double* d_origins, const double* d_dirs,
+                           float* d_rgb, uint32_t* d_argb, void* stream, c2rt_stats* stats);
+
 /* Number of rows rank `rank` owns in a frame of `height` rows. */
 uint32_t c2rt_band_rows_owned(uint32_t height, uint32_t rank, uint32_t n_ranks, uint32_t band_rows);
 
