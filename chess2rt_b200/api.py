@@ -89,7 +89,7 @@ class SceneDesc(C.Structure):
 # every symbol include/c2rt.h declares (tests/test_abi.py checks the library exports them all)
 C_ABI_SYMBOLS = [
     "c2rt_init", "c2rt_shutdown", "c2rt_abi_version", "c2rt_device_count", "c2rt_last_error",
-    "c2rt_scene_create", "c2rt_scene_destroy", "c2rt_render", "c2rt_cancel", "c2rt_render_device", "c2rt_read_ray_counters",
+    "c2rt_scene_create", "c2rt_scene_destroy", "c2rt_scene_set_nodes", "c2rt_render", "c2rt_cancel", "c2rt_render_device", "c2rt_read_ray_counters",
     "c2rt_deinterleave", "c2rt_render_pixel", "c2rt_render_hits", "c2rt_render_hits_device",
     "c2rt_trace_rays", "c2rt_trace_rays_device", "c2rt_test_visibility", "c2rt_test_visibility_device",
     "c2rt_shade_rays", "c2rt_shade_rays_device", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
@@ -104,6 +104,8 @@ lib.c2rt_init.argtypes = [C.c_int, C.POINTER(C.c_int)]
 lib.c2rt_scene_create.argtypes = [C.POINTER(SceneDesc), C.POINTER(C.c_void_p)]
 lib.c2rt_scene_destroy.argtypes = [C.c_void_p]
 lib.c2rt_scene_destroy.restype = None
+lib.c2rt_scene_set_nodes.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p]
 lib.c2rt_render.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.c_void_p, C.c_void_p, C.POINTER(Stats)]
 lib.c2rt_render_device.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.POINTER(Band), C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.POINTER(Stats)]
@@ -156,6 +158,8 @@ host_lib.c2rt_host_scene_override.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_
 host_lib.c2rt_host_scene_override.restype = None
 host_lib.c2rt_host_scene_desc.argtypes = [C.c_void_p]
 host_lib.c2rt_host_scene_desc.restype = C.POINTER(SceneDesc)
+host_lib.c2rt_host_scene_node_index.argtypes = [C.c_void_p, C.c_char_p]
+host_lib.c2rt_host_scene_place_node.argtypes = [C.c_void_p, C.c_int, C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p]
 host_lib.c2rt_host_frame_blocks.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.POINTER(Camera), C.POINTER(Settings)]
 host_lib.c2rt_host_frame_blocks.restype = None
 host_lib.c2rt_host_device_scene.argtypes = [C.c_void_p]
@@ -264,6 +268,25 @@ class HostScene:
         if not p:
             raise C2rtError(-1, host_lib.c2rt_host_last_error().decode())
         return p
+
+    def node_index(self, name):
+        """The index of the node the scene file names `name` (its place in the description's node arrays)."""
+        i = host_lib.c2rt_host_scene_node_index(self._h, str(name).encode())
+        if i < 0:
+            raise KeyError(f"no node named {name!r}")
+        return i
+
+    def place_node(self, node, geometry=None, scale=None, rotate=None, translate=None):
+        """As if the node's entry in the scene file had been edited: `geometry` (a geometry name; None keeps it) and the keys
+        scale / rotate / translate (three numbers each; None: the key is absent).  The node's Transform is reset and the keys
+        are applied as the loader applies them.  `node` is a node name or index.  The flat description and any uploaded scene
+        follow (c2rt_scene_set_nodes), so the next frame shows the edit.  A bad node or geometry name changes nothing."""
+        i = self.node_index(node) if isinstance(node, str) else int(node)
+        for v, name in zip((scale, rotate, translate), ("scale", "rotate", "translate")):
+            if v is not None and len(v) != 3:
+                raise ValueError(f"{name} needs three numbers, got {len(v)}")
+        vecs = [None if v is None else (C.c_double * 3)(*[float(x) for x in v]) for v in (scale, rotate, translate)]
+        _check_host(host_lib.c2rt_host_scene_place_node(self._h, i, None if geometry is None else str(geometry).encode(), *vecs))
 
     def frame_blocks(self, seed=0, count_rays=False):
         cam, st = Camera(), Settings()
@@ -385,6 +408,25 @@ def save_bmp(argb, pad_rows=False):
 
 def cancel():
     _check(lib.c2rt_cancel())
+
+
+def scene_set_nodes(scene_handle, nodes, geom=None, transform=None, inverse=None, inverse_t=None, offset=None):
+    """c2rt_scene_set_nodes on an uploaded scene (a handle from HostScene.device_scene or c2rt_scene_create): entry i sets node
+    nodes[i]'s geometry index geom[i] and / or its transform[i], inverse[i], inverse_t[i] (3x3, row-major) and offset[i].  geom
+    None keeps the geometries; the four transform arrays are given together or not at all."""
+    ids = np.ascontiguousarray(nodes, np.uint32).reshape(-1)
+    n = len(ids)
+    g = None if geom is None else np.ascontiguousarray(geom, np.int32).reshape(-1)
+    if g is not None and len(g) != n:
+        raise ValueError(f"geom has {len(g)} entries for {n} nodes")
+    tf = []
+    for a, per in ((transform, 9), (inverse, 9), (inverse_t, 9), (offset, 3)):
+        a = None if a is None else np.ascontiguousarray(a, np.float64).reshape(-1)
+        if a is not None and len(a) != per * n:
+            raise ValueError(f"a transform array has {len(a)} elements, {per * n} expected")
+        tf.append(a)
+    ptr = lambda a: None if a is None else a.ctypes.data  # noqa: E731
+    _check(lib.c2rt_scene_set_nodes(scene_handle, n, ptr(ids), ptr(g), *[ptr(a) for a in tf]))
 
 
 def render_device(scene_handle, cam, settings, d_rgb_ptr, d_argb_ptr=None, band=None, stream=None):

@@ -260,27 +260,33 @@ int current_device_locked(DeviceCtx*& c) {
 
 }  // namespace
 
-struct c2rt_scene {
-    uint64_t id;
-    DevScene host;                       // constant block; record arrays copied in from the vectors below when they fit
+// The part of a scene that derive_records writes: the node records, the scene class, and the shader / texture order (MODE_SOLO
+// swaps the node's shader and its texture into record 0).  c2rt_scene_set_nodes edits and derives a copy of it, then commits it.
+struct SceneRecords {
     std::vector<DevNode> nodes;          // the scene's records (texel pointers patched per device at upload)
-    std::vector<DevGeom> geoms;
     std::vector<DevShader> shaders;
     std::vector<DevTex> textures;
+    std::vector<size_t> tex_offset;      // per texture, in texels (general-form bitmaps only)
+    std::vector<long long> quad_offset, pal_offset;   // per texture; -1 = general form
+    int mode;                            // kernel specialisation (render_kernel.cu MODE_*)
+};
+
+struct c2rt_scene : SceneRecords {
+    uint64_t id;
+    DevScene host;                       // constant block; record arrays copied in from the vectors when they fit
+    std::vector<DevGeom> geoms;
     bool big = false;                    // beyond the constant block: the records go to global memory (MODE_BIG)
+    bool no_solo = false;                // C2RT_NO_SOLO at creation (test hook: no MODE_SOLO)
     void* d_records[C2RT_MAX_GPUS][4];   // big scenes, per context device: nodes, geoms, shaders, textures
     std::vector<float4> texels;          // bitmaps in the general form, float4 per texel
-    std::vector<size_t> tex_offset;      // per texture, in texels (general-form bitmaps only)
     float4* d_texels[C2RT_MAX_GPUS];     // per context device
     // bitmaps with <= 256 distinct colours (scene_dev.h DevTex::quads): index quads + 256-entry palettes
     std::vector<uint32_t> quads;
     std::vector<float4> palettes;
-    std::vector<long long> quad_offset, pal_offset;   // per texture; -1 = general form
     uint32_t* d_quads[C2RT_MAX_GPUS];
     float4* d_palettes[C2RT_MAX_GPUS];
     float4* d_bounds[C2RT_MAX_GPUS];     // per context device: node bounding spheres for the per-warp masks (FrameParams.bounds)
     int n_dev;
-    int mode;                            // kernel specialisation (render_kernel.cu MODE_*)
 };
 
 namespace {
@@ -309,10 +315,10 @@ Bound union_bound(const Bound& l, const Bound& r) {
 // child is itself a CSG the reference's walk is quirky (a nested child's crossings toggle the wrong flag,
 // entry-only crossing lists flip the initial parity: tests/scenes/nested.sdl) and a hit may be reported on
 // ANY leaf surface: the bound is then the union over all leaves.
-Bound bound_of(const c2rt_scene_desc* d, int gi) {
+Bound bound_of(const std::vector<DevGeom>& geoms, int gi) {
     Bound b{};
-    const double* p = d->geom_params + 4 * gi;
-    const int type = d->geom_type[gi];
+    const double* p = geoms[gi].p;
+    const int type = geoms[gi].type;
     if (type == C2RT_GEOM_SPHERE) {
         b.finite = std::isfinite(p[3]);
         b.c[0] = p[0]; b.c[1] = p[1]; b.c[2] = p[2];
@@ -322,9 +328,9 @@ Bound bound_of(const c2rt_scene_desc* d, int gi) {
         b.c[0] = p[0]; b.c[1] = p[1]; b.c[2] = p[2];
         b.r = fabs(p[3]) * 0.5 * sqrt(3.0);
     } else if (type >= C2RT_GEOM_CSG_UNION) {
-        const int li = d->geom_left[gi], ri = d->geom_right[gi];
-        Bound l = bound_of(d, li), r = bound_of(d, ri);
-        const bool nested = d->geom_type[li] >= C2RT_GEOM_CSG_UNION || d->geom_type[ri] >= C2RT_GEOM_CSG_UNION;
+        const int li = geoms[gi].left, ri = geoms[gi].right;
+        Bound l = bound_of(geoms, li), r = bound_of(geoms, ri);
+        const bool nested = geoms[li].type >= C2RT_GEOM_CSG_UNION || geoms[ri].type >= C2RT_GEOM_CSG_UNION;
         if (nested || type == C2RT_GEOM_CSG_UNION) b = union_bound(l, r);
         else if (type == C2RT_GEOM_CSG_INTER) {
             if (l.finite && r.finite) b = l.r <= r.r ? l : r;
@@ -393,6 +399,8 @@ void build_bitmap(c2rt_scene* s, const DevTex& t, const float* src, int slot) {
         for (uint64_t k = 0; k < n; k++) dst[k] = make_float4(src[3 * k], src[3 * k + 1], src[3 * k + 2], 0.f);
     }
 }
+
+void derive_records(const c2rt_scene& s, SceneRecords& rec);
 
 int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
     if (!d) return fail(C2RT_ERR_INVALID_ARG, "scene description is null");
@@ -528,9 +536,42 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
         memcpy(nd.Minv, d->node_inverse + 9 * i, 9 * sizeof(double));
         memcpy(nd.MinvT, d->node_inverse_t + 9 * i, 9 * sizeof(double));
         memcpy(nd.off, d->node_offset + 3 * i, 3 * sizeof(double));
-        nd.flags = 0;
+    }
+    const char* no_solo = getenv("C2RT_NO_SOLO");   // test hook: keep one-plane scenes on the general plane-only kernel
+    s->no_solo = no_solo && no_solo[0] == '1';
+    derive_records(*s, *s);
+    return C2RT_OK;
+}
+
+// The node bounding spheres of FrameParams.bounds / RayParams.bounds, one float4 per node (radius -1: unbounded)
+std::vector<float4> node_bounds(const SceneRecords& r) {
+    std::vector<float4> bounds(std::max<size_t>(1, r.nodes.size()));
+    for (size_t k = 0; k < r.nodes.size(); k++) {
+        const DevNode& nd = r.nodes[k];
+        bounds[k] = (nd.flags & NODE_UNBOUNDED) ? make_float4(0.f, 0.f, 0.f, -1.f) : make_float4(nd.bcf[0], nd.bcf[1], nd.bcf[2], nd.brf);
+    }
+    return bounds;
+}
+
+// Everything that follows from the raw node fields (geom, shader, M, Minv, MinvT, off) of r.nodes: per node the bound, its FP32
+// form for the cull, NODE_IDENTITY / NODE_UNBOUNDED, kind and wp; then the scene class r.mode with MODE_SOLO's swap.  It reads
+// the scene's geometry records, its light count and the decisions taken at creation (big, no_solo), and no description, so
+// c2rt_scene_create (r is the scene itself) and c2rt_scene_set_nodes (r is the edit's copy) derive alike.
+void derive_records(const c2rt_scene& s, SceneRecords& rec) {
+    const int n_nodes = (int)rec.nodes.size();
+    for (int i = 0; i < n_nodes; i++) {
+        // only the raw fields carry over: a node that changes class keeps nothing of its old derived fields
+        const DevNode raw = rec.nodes[i];
+        DevNode& nd = rec.nodes[i];
+        memset(&nd, 0, sizeof nd);
+        nd.geom = raw.geom;
+        nd.shader = raw.shader;
+        memcpy(nd.M, raw.M, sizeof nd.M);
+        memcpy(nd.Minv, raw.Minv, sizeof nd.Minv);
+        memcpy(nd.MinvT, raw.MinvT, sizeof nd.MinvT);
+        memcpy(nd.off, raw.off, sizeof nd.off);
         if (is_identity(nd.M) && is_identity(nd.Minv) && is_identity(nd.MinvT)) nd.flags |= NODE_IDENTITY;
-        Bound b = bound_of(d, nd.geom);
+        Bound b = bound_of(s.geoms, nd.geom);
         if (b.finite) {
             // world centre = c*M + offset; radius scaled by an upper bound of |M|_2
             double cx = b.c[0] * nd.M[0] + b.c[1] * nd.M[3] + b.c[2] * nd.M[6] + nd.off[0];
@@ -572,7 +613,7 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
         // diagonal scale (Node "scale", zaphod.sdl): such a plane is the world plane y = y0 * sy + off.y, its
         // object-space uv (geometry.d:54-55) are the world offsets times 1/sx, 1/sz
         nd.kind = KIND_GENERIC;
-        const DevGeom& g = s->geoms[nd.geom];
+        const DevGeom& g = s.geoms[nd.geom];
         nd.wp[1] = 1.0; nd.wp[2] = 1.0;
         if (g.type == C2RT_GEOM_PLANE && std::isnan(g.p[1])) {   // bounded planes (limit set) keep the generic path
             bool diag = nd.M[0] > 0 && nd.M[4] > 0 && nd.M[8] > 0;
@@ -592,37 +633,36 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
             nd.wp[3] = g.p[3];
         }
     }
-    s->mode = 0;
-    for (uint32_t i = 0; i < d->n_nodes; i++) {
-        if (!(s->nodes[i].flags & NODE_UNBOUNDED)) s->mode |= MODE_BOUNDED;
-        if (s->nodes[i].kind == KIND_GENERIC) s->mode |= MODE_GENERIC;
-        const DevGeom& ng = s->geoms[s->nodes[i].geom];
+    rec.mode = 0;
+    for (int i = 0; i < n_nodes; i++) {
+        if (!(rec.nodes[i].flags & NODE_UNBOUNDED)) rec.mode |= MODE_BOUNDED;
+        if (rec.nodes[i].kind == KIND_GENERIC) rec.mode |= MODE_GENERIC;
+        const DevGeom& ng = s.geoms[rec.nodes[i].geom];
         // (MODE_NESTED implies the generic, bounded kernel)
-        if (ng.type >= C2RT_GEOM_CSG_UNION && ng.depth != 1) s->mode |= MODE_NESTED | MODE_GENERIC | MODE_BOUNDED;
+        if (ng.type >= C2RT_GEOM_CSG_UNION && ng.depth != 1) rec.mode |= MODE_NESTED | MODE_GENERIC | MODE_BOUNDED;
     }
     // MODE_SOLO: exactly one node, a world-space plane, and exactly one light.  The node's shader and that shader's
-    // texture are swapped into record 0 so the kernel addresses every scene constant statically.
-    const char* no_solo = getenv("C2RT_NO_SOLO");   // test hook: keep such scenes on the general plane-only kernel
-    if (!s->big && s->mode == 0 && h.n_nodes == 1 && h.n_lights == 1 && s->nodes[0].kind == KIND_PLANE_W && !(no_solo && no_solo[0] == '1')) {
-        const int si = s->nodes[0].shader;
-        std::swap(s->shaders[0], s->shaders[si]);
-        s->nodes[0].shader = 0;
-        const int ti = s->shaders[0].tex;
+    // texture are swapped into record 0 so the kernel addresses every scene constant statically.  On records this swap
+    // has already been applied to (node 0's shader is 0, its texture 0) it changes nothing.
+    if (!s.big && rec.mode == 0 && n_nodes == 1 && s.host.n_lights == 1 && rec.nodes[0].kind == KIND_PLANE_W && !s.no_solo) {
+        const int si = rec.nodes[0].shader;
+        std::swap(rec.shaders[0], rec.shaders[si]);
+        rec.nodes[0].shader = 0;
+        const int ti = rec.shaders[0].tex;
         if (ti >= 0) {
-            std::swap(s->textures[0], s->textures[ti]);
-            std::swap(s->tex_offset[0], s->tex_offset[ti]);
-            std::swap(s->quad_offset[0], s->quad_offset[ti]);
-            std::swap(s->pal_offset[0], s->pal_offset[ti]);
-            for (int k = 0; k < h.n_shaders; k++) {
-                if (s->shaders[k].tex == 0) s->shaders[k].tex = ti;
-                else if (s->shaders[k].tex == ti) s->shaders[k].tex = 0;
+            std::swap(rec.textures[0], rec.textures[ti]);
+            std::swap(rec.tex_offset[0], rec.tex_offset[ti]);
+            std::swap(rec.quad_offset[0], rec.quad_offset[ti]);
+            std::swap(rec.pal_offset[0], rec.pal_offset[ti]);
+            for (DevShader& sh : rec.shaders) {
+                if (sh.tex == 0) sh.tex = ti;
+                else if (sh.tex == ti) sh.tex = 0;
             }
         }
-        s->mode = MODE_SOLO | ((s->shaders[0].tex >= 0 ? 1 + s->textures[0].type : 0) << MODE_TEX_SHIFT) |
-                  (s->shaders[0].type == C2RT_SHADER_PHONG ? MODE_PHONG : 0);
+        rec.mode = MODE_SOLO | ((rec.shaders[0].tex >= 0 ? 1 + rec.textures[0].type : 0) << MODE_TEX_SHIFT) |
+                   (rec.shaders[0].type == C2RT_SHADER_PHONG ? MODE_PHONG : 0);
     }
-    if (s->big) s->mode = (s->mode & MODE_NESTED) | MODE_BOUNDED | MODE_GENERIC | MODE_BIG;   // the general kernels only
-    return C2RT_OK;
+    if (s.big) rec.mode = (rec.mode & MODE_NESTED) | MODE_BOUNDED | MODE_GENERIC | MODE_BIG;   // the general kernels only
 }
 
 int upload_to_devices(c2rt_scene* s) {
@@ -631,11 +671,7 @@ int upload_to_devices(c2rt_scene* s) {
         s->d_texels[i] = nullptr; s->d_bounds[i] = nullptr; s->d_quads[i] = nullptr; s->d_palettes[i] = nullptr;
         for (int k = 0; k < 4; k++) s->d_records[i][k] = nullptr;
     }
-    std::vector<float4> bounds((size_t)std::max(1, s->host.n_nodes));
-    for (int k = 0; k < s->host.n_nodes; k++) {
-        const DevNode& nd = s->nodes[k];
-        bounds[k] = (nd.flags & NODE_UNBOUNDED) ? make_float4(0.f, 0.f, 0.f, -1.f) : make_float4(nd.bcf[0], nd.bcf[1], nd.bcf[2], nd.brf);
-    }
+    const std::vector<float4> bounds = node_bounds(*s);
     for (int i = 0; i < g_ctx.n; i++) {
         CU(cudaSetDevice(g_ctx.d[i].dev));
         CU(cudaMalloc(&s->d_bounds[i], bounds.size() * sizeof(float4)));
@@ -1280,6 +1316,51 @@ void c2rt_scene_destroy(c2rt_scene* s) {
         if (g_ctx.d[i].uploaded_scene == s->id) g_ctx.d[i].uploaded_scene = 0;
     }
     delete s;
+}
+
+int c2rt_scene_set_nodes(c2rt_scene* s, size_t n, const uint32_t* nodes, const int32_t* geom, const double* transform,
+                         const double* inverse, const double* inverse_t, const double* offset) {
+    if (!s) return fail(C2RT_ERR_INVALID_ARG, "scene is null");
+    const int n_tf = (transform != nullptr) + (inverse != nullptr) + (inverse_t != nullptr) + (offset != nullptr);
+    if (n_tf != 0 && n_tf != 4)
+        return fail(C2RT_ERR_INVALID_ARG, "transform, inverse, inverse_t and offset are given together or all null (%d of 4 given)", n_tf);
+    if (!geom && n_tf == 0) return fail(C2RT_ERR_INVALID_ARG, "nothing to edit: geom and the transform arrays are all null");
+    if (n == 0) return C2RT_OK;
+    if (!nodes) return fail(C2RT_ERR_INVALID_ARG, "nodes is null");
+    for (size_t k = 0; k < n; k++) {
+        if (nodes[k] >= s->nodes.size())
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: node index %u out of range (%zu nodes)", k, nodes[k], s->nodes.size());
+        if (geom && (geom[k] < 0 || (size_t)geom[k] >= s->geoms.size()))
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: geometry index %d out of range (%zu geometries)", k, geom[k], s->geoms.size());
+    }
+    std::lock_guard<std::mutex> g(g_mu);
+    if (s->n_dev != g_ctx.n) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
+    // the edit and its derivation on a copy; nothing of the scene changes before the devices are idle
+    SceneRecords work = *s;
+    for (size_t k = 0; k < n; k++) {
+        DevNode& nd = work.nodes[nodes[k]];
+        if (geom) nd.geom = geom[k];
+        if (transform) {
+            memcpy(nd.M, transform + 9 * k, sizeof nd.M);
+            memcpy(nd.Minv, inverse + 9 * k, sizeof nd.Minv);
+            memcpy(nd.MinvT, inverse_t + 9 * k, sizeof nd.MinvT);
+            memcpy(nd.off, offset + 3 * k, sizeof nd.off);
+        }
+    }
+    derive_records(*s, work);
+    // kernels in flight on any stream of these devices read the bounds (and the scene block): wait for them, then rewrite the
+    // bounds in place.  The scene block, or the global records of a big scene, is re-uploaded by make_resident at the next use
+    // on each device: the scene gets a new id, which no device holds.
+    const std::vector<float4> bounds = node_bounds(work);
+    for (int i = 0; i < s->n_dev; i++) {
+        CU(cudaSetDevice(g_ctx.d[i].dev));
+        CU(cudaDeviceSynchronize());
+        CU(cudaMemcpy(s->d_bounds[i], bounds.data(), bounds.size() * sizeof(float4), cudaMemcpyHostToDevice));
+    }
+    CU(cudaSetDevice(g_ctx.d[0].dev));
+    static_cast<SceneRecords&>(*s) = std::move(work);
+    s->id = g_ctx.next_scene_id++;
+    return C2RT_OK;
 }
 
 int c2rt_render_device(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, const c2rt_band* band, float* d_rgb,

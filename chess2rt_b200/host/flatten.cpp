@@ -12,9 +12,9 @@ int indexOf(const std::vector<std::unique_ptr<T>>& v, const T* p) {
     return -1;
 }
 
-void pushMatrix(std::vector<double>& dst, const Matrix& m) {
+void putMatrix(double dst[9], const Matrix& m) {
     for (int r = 0; r < 3; r++)
-        for (int c = 0; c < 3; c++) dst.push_back(m.c[r][c]);
+        for (int c = 0; c < 3; c++) dst[3 * r + c] = m.c[r][c];
 }
 
 }  // namespace
@@ -149,17 +149,28 @@ FlatScene flatten(const Scene& scene) {
 
     // nodes
     for (auto& n : scene.nodes) {
-        int g = indexOf(scene.geometries, n->geom), s = indexOf(scene.shaders, n->shader);
-        if (g < 0 || s < 0) throw InvalidSceneException("node refers to a geometry / shader outside the scene");
-        f.node_geom.push_back(g);
-        f.node_shader.push_back(s);
-        pushMatrix(f.node_transform, n->transform.transform);
-        pushMatrix(f.node_inverse, n->transform.inverseTransform);
-        pushMatrix(f.node_inverse_t, n->transform.transposedInverse);
-        f.node_offset.push_back(n->transform.offset.x);
-        f.node_offset.push_back(n->transform.offset.y);
-        f.node_offset.push_back(n->transform.offset.z);
+        const FlatNode fn = flattenNode(scene, *n);
+        f.node_geom.push_back(fn.geom);
+        f.node_shader.push_back(fn.shader);
+        f.node_transform.insert(f.node_transform.end(), fn.transform, fn.transform + 9);
+        f.node_inverse.insert(f.node_inverse.end(), fn.inverse, fn.inverse + 9);
+        f.node_inverse_t.insert(f.node_inverse_t.end(), fn.inverse_t, fn.inverse_t + 9);
+        f.node_offset.insert(f.node_offset.end(), fn.offset, fn.offset + 3);
     }
+    return f;
+}
+
+FlatNode flattenNode(const Scene& scene, const Node& n) {
+    FlatNode f;
+    f.geom = indexOf(scene.geometries, n.geom);
+    f.shader = indexOf(scene.shaders, n.shader);
+    if (f.geom < 0 || f.shader < 0) throw InvalidSceneException("node refers to a geometry / shader outside the scene");
+    putMatrix(f.transform, n.transform.transform);
+    putMatrix(f.inverse, n.transform.inverseTransform);
+    putMatrix(f.inverse_t, n.transform.transposedInverse);
+    f.offset[0] = n.transform.offset.x;
+    f.offset[1] = n.transform.offset.y;
+    f.offset[2] = n.transform.offset.z;
     return f;
 }
 

@@ -35,7 +35,15 @@ struct FlatScene {
     c2rt_scene_desc desc() const;  // borrows the vectors above
 };
 
+// One node's entries of the node arrays (c2rt_scene_desc, c2rt_scene_set_nodes): geometry and shader index, the three
+// matrices row-major, the offset
+struct FlatNode {
+    int32_t geom, shader;
+    double transform[9], inverse[9], inverse_t[9], offset[3];
+};
+
 FlatScene flatten(const Scene& scene);                        // throws InvalidSceneException on dangling references
+FlatNode flattenNode(const Scene& scene, const Node& node);   // the same for one node
 c2rt_camera flattenCamera(const Camera& cam);                 // call after Camera.beginFrame
 c2rt_settings flattenSettings(const GlobalSettings& s, uint64_t rngSeed = 0, bool countRays = false);
 

@@ -1,7 +1,9 @@
 // C entry points over the C++ host mirror, for the Python harness (tests/, bench.py) — the same
 // calls the headless executable makes: load a scene file with the reference-compatible loader,
 // flatten it, render through libc2rt.so.  No torch types, no CPU rendering.
+#include <algorithm>
 #include <cstring>
+#include <string>
 
 #include "flatten.hpp"
 #include "renderer.hpp"
@@ -71,6 +73,73 @@ const c2rt_scene_desc* c2rt_host_scene_desc(c2rt_host_scene* h) {
         return nullptr;
     }
 }
+// index of the node the scene file names `name` (its place in c2rt_scene_desc's node arrays), -1 if there is none
+int c2rt_host_scene_node_index(const c2rt_host_scene* h, const char* name) {
+    const Scene& s = *h->scene;
+    auto it = name ? s.namedEntities.nodes.find(name) : s.namedEntities.nodes.end();
+    if (it == s.namedEntities.nodes.end()) return -1;
+    for (size_t i = 0; i < s.nodes.size(); i++)
+        if (s.nodes[i].get() == it->second) return (int)i;
+    return -1;
+}
+
+// As if the scene file's entry of node `node` had been edited: its geometry becomes the one named `geometry` (NULL: kept), its
+// Transform is reset and the given keys are applied the way the loader applies them (makeNode: scale, then rotate through
+// scale as the reference does, then translate; NULL: key absent).  The flat description and both uploaded scenes (the
+// render_device one and the Renderer's) follow with c2rt_scene_set_nodes.  A bad node index or geometry name changes nothing.
+int c2rt_host_scene_place_node(c2rt_host_scene* h, int node, const char* geometry, const double* scale, const double* rotate,
+                               const double* translate) {
+    try {
+        Scene& sc = *h->scene;
+        if (node < 0 || (size_t)node >= sc.nodes.size()) {
+            g_host_err = "place_node: node index " + std::to_string(node) + " out of range (" + std::to_string(sc.nodes.size()) + " nodes)";
+            return C2RT_ERR_INVALID_ARG;
+        }
+        const Geometry* g = nullptr;
+        if (geometry) {
+            auto it = sc.namedEntities.geometries.find(geometry);
+            if (it == sc.namedEntities.geometries.end()) {
+                g_host_err = std::string("place_node: no geometry named \"") + geometry + "\"";
+                return C2RT_ERR_INVALID_ARG;
+            }
+            g = it->second;
+        }
+        Node& nd = *sc.nodes[node];
+        if (g) nd.geom = g;
+        nd.transform.reset();
+        if (scale) nd.transform.scale(scale[0], scale[1], scale[2]);
+        if (rotate) nd.transform.scale(rotate[0], rotate[1], rotate[2]);   // sic: scene_loader.cpp makeNode, node.d:89-90
+        if (translate) nd.transform.translate(Vector(translate[0], translate[1], translate[2]));
+        const FlatNode f = flattenNode(sc, nd);
+        if (h->flat_valid) {   // in place: the pointers c2rt_host_scene_desc handed out stay valid
+            FlatScene& fl = h->flat;
+            fl.node_geom[node] = f.geom;
+            std::copy(f.transform, f.transform + 9, fl.node_transform.begin() + 9 * node);
+            std::copy(f.inverse, f.inverse + 9, fl.node_inverse.begin() + 9 * node);
+            std::copy(f.inverse_t, f.inverse_t + 9, fl.node_inverse_t.begin() + 9 * node);
+            std::copy(f.offset, f.offset + 3, fl.node_offset.begin() + 3 * node);
+        }
+        sc.nodesEdited({node});
+        if (h->device) {
+            const uint32_t id = (uint32_t)node;
+            int rc = c2rt_scene_set_nodes(h->device, 1, &id, &f.geom, f.transform, f.inverse, f.inverse_t, f.offset);
+            if (rc != C2RT_OK) {
+                g_host_err = std::string("libc2rt: ") + c2rt_last_error();
+                c2rt_scene_destroy(h->device);   // the next use re-creates it from the edited scene
+                h->device = nullptr;
+                return rc;
+            }
+        }
+        return 0;
+    } catch (const BackendException& e) {
+        g_host_err = e.what();
+        return e.status;
+    } catch (const std::exception& e) {
+        g_host_err = e.what();
+        return C2RT_ERR_INVALID_ARG;
+    }
+}
+
 // per-frame blocks: runs scene.beginFrame() first, like renderSceneAsync (renderer.d:31)
 void c2rt_host_frame_blocks(c2rt_host_scene* h, uint64_t seed, int count_rays, c2rt_camera* cam, c2rt_settings* set) {
     h->scene->beginFrame();

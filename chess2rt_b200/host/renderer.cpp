@@ -1,5 +1,6 @@
 #include "renderer.hpp"
 
+#include <algorithm>
 #include <cstring>
 
 namespace rt {
@@ -32,6 +33,30 @@ c2rt_scene* Renderer::device() {
         scene_.deviceScene = holder;
     }
     return static_cast<DeviceSceneHolder*>(scene_.deviceScene.get())->handle;
+}
+
+void Scene::nodesEdited(const std::vector<int>& indices) {
+    if (!deviceScene || indices.empty()) return;   // (no uploaded scene: the next frame flattens the whole scene)
+    const size_t n = indices.size();
+    std::vector<uint32_t> ids(n);
+    std::vector<int32_t> geom(n);
+    std::vector<double> m(9 * n), inv(9 * n), inv_t(9 * n), off(3 * n);
+    for (size_t k = 0; k < n; k++) {
+        if (indices[k] < 0 || (size_t)indices[k] >= nodes.size()) throw RTException("nodesEdited: node index out of range");
+        const FlatNode f = flattenNode(*this, *nodes[indices[k]]);
+        ids[k] = (uint32_t)indices[k];
+        geom[k] = f.geom;
+        std::copy(f.transform, f.transform + 9, m.begin() + 9 * k);
+        std::copy(f.inverse, f.inverse + 9, inv.begin() + 9 * k);
+        std::copy(f.inverse_t, f.inverse_t + 9, inv_t.begin() + 9 * k);
+        std::copy(f.offset, f.offset + 3, off.begin() + 3 * k);
+    }
+    c2rt_scene* handle = static_cast<DeviceSceneHolder*>(deviceScene.get())->handle;
+    int rc = c2rt_scene_set_nodes(handle, n, ids.data(), geom.data(), m.data(), inv.data(), inv_t.data(), off.data());
+    if (rc != C2RT_OK) {
+        invalidateDeviceScene();   // the next frame re-creates it from the edited scene
+        raise(rc);
+    }
 }
 
 void Renderer::renderRT() {

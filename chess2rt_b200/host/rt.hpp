@@ -272,9 +272,14 @@ public:
 
     // New with the CUDA backend: the uploaded (flattened) scene, created on first render and
     // reused by every later frame; see renderer.cpp.  Call invalidateDeviceScene() after
-    // editing geometry / shaders / textures / lights / nodes (camera and settings are per-frame).
+    // editing geometry / shaders / textures / lights, or adding / removing nodes (camera and
+    // settings are per-frame).  After changing only the geom or transform of existing nodes, call
+    // nodesEdited(indices) instead: it re-flattens those nodes and edits the uploaded scene in
+    // place (c2rt_scene_set_nodes) rather than re-creating it.  Throws BackendException on a
+    // library error, after dropping the uploaded scene.
     mutable std::shared_ptr<void> deviceScene;
     void invalidateDeviceScene() { deviceScene.reset(); }
+    void nodesEdited(const std::vector<int>& indices);
 };
 
 // rt/scene_loader.d:20-41

@@ -221,6 +221,23 @@ const char* c2rt_last_error(void);
 int c2rt_scene_create(const c2rt_scene_desc* desc, c2rt_scene** out);
 void c2rt_scene_destroy(c2rt_scene* scene);
 
+/* Node edits in place: moves a piece (its transform), captures it (moves it off the board), promotes it (its geometry index)
+ * without re-creating the scene.  Entry i edits node nodes[i]; the arrays have the layout of c2rt_scene_desc's node arrays
+ * ([n], [n*9], [n*9], [n*9], [n*3]).  geom == NULL keeps every edited node's geometry; the four transform arrays are given
+ * together, or all NULL to keep every edited node's transform; at least one of the two must be given.  Entries apply in array
+ * order, so a later entry for the same node wins.  Shaders, textures, lights, the environment, the node count and the node
+ * order stay as created.
+ * Afterwards every call on the scene (frames, _device frames, hit frames, the pixel pick, ray queries, visibility, shaded rays)
+ * gives the same result, bit for bit, as on a scene c2rt_scene_create built from the edited description, on every device.
+ * Errors: a null scene, nodes == NULL with n > 0, a node index >= n_nodes, a geometry index outside 0..n_geoms-1 or a partial
+ * set of transform arrays is C2RT_ERR_INVALID_ARG.  Every check runs before anything changes: on any of these errors the scene
+ * is unchanged.  n == 0 is a no-op.  A C2RT_ERR_CUDA leaves the scene fit only for c2rt_scene_destroy.
+ * Blocking: takes the library lock (so it waits for a c2rt_render running on another thread) and waits for all work on every
+ * context device, since kernels in flight read the scene.  The first frame after an edit, like a scene's first frame on a
+ * device, must be issued outside any CUDA stream capture, and a graph captured before the edit must not be replayed after it. */
+int c2rt_scene_set_nodes(c2rt_scene* scene, size_t n, const uint32_t* nodes, const int32_t* geom,
+                         const double* transform, const double* inverse, const double* inverse_t, const double* offset);
+
 /* Replaces Renderer.renderRT (renderer.d:83-189): blocking, one frame into caller-owned HOST
  * memory.  rgb: frame_width*frame_height*3 floats laid out as Image!Color.pixels
  * (row-major, top row first, imageio/image.d:45-54).  argb (nullable): one uint32 per pixel,
@@ -243,7 +260,9 @@ int c2rt_cancel(void);
  * d_rgb must be 16-byte aligned when frame_width is a multiple of 4 (bands are written with float4 stores).
  * A device holds ONE scene block at a time: rendering a different scene than the previous call on this device first waits
  * for all work on the device and re-uploads the block, so (i) frames of two scenes never overlap on one device and
- * (ii) the first frame of a scene on a device must be issued outside any CUDA stream capture (later ones may be captured). */
+ * (ii) the first frame of a scene on a device must be issued outside any CUDA stream capture (later ones may be captured).
+ * The same holds for the first frame after a c2rt_scene_set_nodes: the edit re-uploads the block, and a frame captured into a
+ * graph before the edit is not valid after it. */
 int c2rt_render_device(c2rt_scene* scene, const c2rt_camera* camera, const c2rt_settings* settings,
                        const c2rt_band* band, float* d_rgb, uint32_t* d_argb, void* stream, c2rt_stats* stats);
 
