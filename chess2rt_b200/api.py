@@ -94,7 +94,7 @@ C_ABI_SYMBOLS = [
     "c2rt_trace_rays", "c2rt_trace_rays_device", "c2rt_test_visibility", "c2rt_test_visibility_device",
     "c2rt_shade_rays", "c2rt_shade_rays_device", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
     "c2rt_frame_alloc", "c2rt_frame_free", "c2rt_frame_export", "c2rt_frame_import", "c2rt_frame_unimport", "c2rt_frame_memset", "c2rt_frame_download", "c2rt_pin_host_buffer", "c2rt_unpin_host_buffer", "c2rt_gate",
-    "c2rt_measure_fma_peak", "c2rt_selftest_device_pool",
+    "c2rt_measure_fma_peak", "c2rt_selftest_device_pool", "c2rt_selftest_scene_class",
 ]
 
 lib.c2rt_last_error.restype = C.c_char_p

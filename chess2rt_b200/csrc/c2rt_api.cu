@@ -14,6 +14,7 @@
 #include <condition_variable>
 #include <cstring>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -553,6 +554,17 @@ std::vector<float4> node_bounds(const SceneRecords& r) {
     return bounds;
 }
 
+// MODE_UPAT of a Procedure2 record: which u frequencies d[0..2] (the doubles sin_phase multiplies u by) are equal.  Judged by
+// their bits, as the kernel would compute them: a sine shared between two terms is the same value only when the two factors are
+// the same double (-0.0 and 0.0 are not).
+static int proc2_u_pattern(const DevTex& t) {
+    auto same = [&](int i, int j) { return memcmp(&t.d[i], &t.d[j], sizeof(double)) == 0; };
+    const int first1 = same(1, 0) ? 0 : 1, first2 = same(2, 0) ? 0 : same(2, 1) ? 1 : 2;
+    for (int p = UPAT_DISTINCT; p <= UPAT_ALL; p++)
+        if (upat_first(p, 1) == first1 && upat_first(p, 2) == first2) return p;
+    return UPAT_DISTINCT;   // (unreachable: first1 == 0 and first2 == 1 contradict each other)
+}
+
 // Everything that follows from the raw node fields (geom, shader, M, Minv, MinvT, off) of r.nodes: per node the bound, its FP32
 // form for the cull, NODE_IDENTITY / NODE_UNBOUNDED, kind and wp; then the scene class r.mode with MODE_SOLO's swap.  It reads
 // the scene's geometry records, its light count and the decisions taken at creation (big, no_solo), and no description, so
@@ -661,6 +673,8 @@ void derive_records(const c2rt_scene& s, SceneRecords& rec) {
         }
         rec.mode = MODE_SOLO | ((rec.shaders[0].tex >= 0 ? 1 + rec.textures[0].type : 0) << MODE_TEX_SHIFT) |
                    (rec.shaders[0].type == C2RT_SHADER_PHONG ? MODE_PHONG : 0);
+        if (rec.shaders[0].tex >= 0 && rec.textures[0].type == C2RT_TEX_PROCEDURE2)
+            rec.mode |= proc2_u_pattern(rec.textures[0]) << MODE_UPAT_SHIFT;
     }
     if (s.big) rec.mode = (rec.mode & MODE_NESTED) | MODE_BOUNDED | MODE_GENERIC | MODE_BIG;   // the general kernels only
 }
@@ -1689,6 +1703,13 @@ long long c2rt_selftest_device_pool(int workers, int rounds) {
         total += h.load();
     }
     return total / 2;
+}
+
+int c2rt_selftest_scene_class(const c2rt_scene_desc* desc) {
+    std::lock_guard<std::mutex> g(g_mu);
+    const std::unique_ptr<c2rt_scene> s(new c2rt_scene());   // built, never uploaded
+    const int rc = validate_and_build(desc, s.get());
+    return rc == C2RT_OK ? s->mode : rc;
 }
 
 int c2rt_measure_fma_peak(int fp64, double* tflops, double* sm_clock_mhz_est) {

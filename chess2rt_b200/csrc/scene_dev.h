@@ -153,6 +153,19 @@ constexpr int MODE_SOLO = 32, MODE_TEX_SHIFT = 6, MODE_TEX_MASK = 3 << MODE_TEX_
 //   MODE_BIG      the scene exceeds the constant block: node / geometry / shader / texture records in global memory
 //                 (DevScene::g_*), node masks of one 64-bit word per 64 nodes in shared memory (render_kernel.cu NodeMask)
 constexpr int MODE_BIG = 512;
+//   MODE_UPAT     MODE_SOLO with a Procedure2 texture: which of its three u frequencies are the same double
+//                 (c2rt_api.cu proc2_u_pattern), so that the straight-line tap of render_solo_kernel<..., ROWS_YZ> takes one sine
+//                 per distinct frequency (render_kernel.cu texture_uv); 0 (all distinct) for every other scene class.  Term i
+//                 reads the sine of term upat_first(pattern, i).
+constexpr int MODE_UPAT_SHIFT = 10, MODE_UPAT_MASK = 7 << MODE_UPAT_SHIFT;
+enum : int { UPAT_DISTINCT = 0, UPAT_01 = 1, UPAT_02 = 2, UPAT_12 = 3, UPAT_ALL = 4 };
+#ifdef __CUDACC__
+__host__ __device__
+#endif
+constexpr int upat_first(int upat, int i) {
+    return i == 0 ? 0 : i == 1 ? (upat == UPAT_01 || upat == UPAT_ALL ? 0 : 1)
+                               : (upat == UPAT_02 || upat == UPAT_ALL ? 0 : upat == UPAT_12 ? 1 : 2);
+}
 // every node is a world-space plane (KIND_PLANE_W): no bounded and no generic node exists
 #ifdef __CUDACC__
 __host__ __device__

@@ -409,6 +409,10 @@ int c2rt_measure_fma_peak(int fp64, double* tflops, double* sm_clock_mhz_est);
  * (== workers * rounds when nothing was lost or duplicated), negative on bad arguments. */
 long long c2rt_selftest_device_pool(int workers, int rounds);
 
+/* Test hook (no GPU needed): validates `desc` as c2rt_scene_create does and returns the kernel specialisation the scene
+ * would get (>= 0: the MODE_* bits of chess2rt_b200/csrc/scene_dev.h), or a negative C2RT_ERR_* code.  Nothing is uploaded. */
+int c2rt_selftest_scene_class(const c2rt_scene_desc* desc);
+
 #ifdef __cplusplus
 }
 #endif
