@@ -9,7 +9,8 @@ any attribute of :mod:`chess2rt_b200.api` raises if the libraries have not been 
 """
 _API_NAMES = (
     "C2rtError", "HostScene", "HitPlanes", "Stats", "band_rows_owned", "device_count", "init", "lib", "host_lib", "render_device",
-    "render_hits_device", "RayHits", "trace_rays_device", "test_visibility_device", "shade_rays_device", "scene_set_nodes", "read_ray_counters", "deinterleave", "measure_fma_peak", "srgb_table", "rng_u31", "shutdown",
+    "render_hits_device", "RayHits", "trace_rays_device", "test_visibility_device", "shade_rays_device", "scene_set_nodes", "scene_set_node_shaders", "scene_set_shaders",
+    "scene_set_textures", "scene_set_lights", "read_ray_counters", "deinterleave", "measure_fma_peak", "srgb_table", "rng_u31", "shutdown",
 )
 
 

@@ -89,7 +89,8 @@ class SceneDesc(C.Structure):
 # every symbol include/c2rt.h declares (tests/test_abi.py checks the library exports them all)
 C_ABI_SYMBOLS = [
     "c2rt_init", "c2rt_shutdown", "c2rt_abi_version", "c2rt_device_count", "c2rt_last_error",
-    "c2rt_scene_create", "c2rt_scene_destroy", "c2rt_scene_set_nodes", "c2rt_render", "c2rt_cancel", "c2rt_render_device", "c2rt_read_ray_counters",
+    "c2rt_scene_create", "c2rt_scene_destroy", "c2rt_scene_set_nodes", "c2rt_scene_set_node_shaders", "c2rt_scene_set_shaders",
+    "c2rt_scene_set_textures", "c2rt_scene_set_lights", "c2rt_render", "c2rt_cancel", "c2rt_render_device", "c2rt_read_ray_counters",
     "c2rt_deinterleave", "c2rt_render_pixel", "c2rt_render_hits", "c2rt_render_hits_device",
     "c2rt_trace_rays", "c2rt_trace_rays_device", "c2rt_test_visibility", "c2rt_test_visibility_device",
     "c2rt_shade_rays", "c2rt_shade_rays_device", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
@@ -106,6 +107,10 @@ lib.c2rt_scene_destroy.argtypes = [C.c_void_p]
 lib.c2rt_scene_destroy.restype = None
 lib.c2rt_scene_set_nodes.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_void_p]
+lib.c2rt_scene_set_node_shaders.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]
+lib.c2rt_scene_set_shaders.argtypes = [C.c_void_p, C.c_size_t] + [C.c_void_p] * 6
+lib.c2rt_scene_set_textures.argtypes = [C.c_void_p, C.c_size_t] + [C.c_void_p] * 3
+lib.c2rt_scene_set_lights.argtypes = [C.c_void_p, C.c_size_t] + [C.c_void_p] * 4
 lib.c2rt_render.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.c_void_p, C.c_void_p, C.POINTER(Stats)]
 lib.c2rt_render_device.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.POINTER(Band), C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.POINTER(Stats)]
@@ -160,6 +165,13 @@ host_lib.c2rt_host_scene_desc.argtypes = [C.c_void_p]
 host_lib.c2rt_host_scene_desc.restype = C.POINTER(SceneDesc)
 host_lib.c2rt_host_scene_node_index.argtypes = [C.c_void_p, C.c_char_p]
 host_lib.c2rt_host_scene_place_node.argtypes = [C.c_void_p, C.c_int, C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p]
+host_lib.c2rt_host_scene_index.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p]
+host_lib.c2rt_host_scene_name.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
+host_lib.c2rt_host_scene_name.restype = C.c_char_p
+host_lib.c2rt_host_scene_set_node_shader.argtypes = [C.c_void_p, C.c_int, C.c_char_p]
+host_lib.c2rt_host_scene_set_shader.argtypes = [C.c_void_p, C.c_int, C.c_char_p, C.c_void_p, C.c_char_p, C.c_void_p, C.c_void_p]
+host_lib.c2rt_host_scene_set_texture.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 8
+host_lib.c2rt_host_scene_set_light.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
 host_lib.c2rt_host_frame_blocks.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.POINTER(Camera), C.POINTER(Settings)]
 host_lib.c2rt_host_frame_blocks.restype = None
 host_lib.c2rt_host_device_scene.argtypes = [C.c_void_p]
@@ -288,6 +300,63 @@ class HostScene:
         vecs = [None if v is None else (C.c_double * 3)(*[float(x) for x in v]) for v in (scale, rotate, translate)]
         _check_host(host_lib.c2rt_host_scene_place_node(self._h, i, None if geometry is None else str(geometry).encode(), *vecs))
 
+    def index(self, section, entity):
+        """The index of an entity of `section` ("nodes", "shaders", "textures" or "lights"): its place in the description's
+        arrays.  `entity` is the name the scene file gives it, or an index (checked by the edit that takes it)."""
+        if not isinstance(entity, str):
+            return int(entity)
+        i = host_lib.c2rt_host_scene_index(self._h, section.encode(), entity.encode())
+        if i < 0:
+            raise KeyError(f"no {section[:-1]} named {entity!r}")
+        return i
+
+    def set_node_shader(self, node, shader):
+        """As if the node's `shader` key in the scene file named `shader` (a shader name or index): highlighting a piece and
+        back.  The flat description and any uploaded scene follow (c2rt_scene_set_node_shaders).  A bad name changes nothing."""
+        i = self.index("nodes", node)
+        _check_host(host_lib.c2rt_host_scene_set_node_shader(self._h, i, self._name("shaders", shader).encode()))
+
+    def set_shader(self, shader, kind=None, color=None, texture=..., exponent=None, strength=None):
+        """As if the shader's entry in the scene file had been edited.  kind ("Lambert" or "Phong"; None keeps the object)
+        replaces it with a fresh shader of that kind, with that kind's defaults; then the given keys apply as the loader applies
+        them: color (three numbers), texture (a texture name or index; None for no texture; omitted: kept), exponent and
+        strength (Phong keys, clamped as the loader clamps them).  `shader` is a name or index.  The flat description and any
+        uploaded scene follow (c2rt_scene_set_shaders).  A bad name, index, kind or key changes nothing."""
+        i = self.index("shaders", shader)
+        tex = None if texture is ... else ("" if texture is None else self._name("textures", texture))
+        _check_host(host_lib.c2rt_host_scene_set_shader(
+            self._h, i, None if kind is None else str(kind).encode(), _floats(color, 3, "color"),
+            None if tex is None else tex.encode(), _doubles(exponent, 1, "exponent"), _floats(strength, 1, "strength")))
+
+    def set_texture(self, texture, color1=None, color2=None, size=None, colorU=None, colorV=None, freqU=None, freqV=None,
+                    scaling=None):
+        """As if the texture's entry in the scene file had the given keys replaced (None: kept).  Checker: color1, color2 (three
+        numbers each), size; Procedure2: colorU, colorV (three colours), freqU, freqV (three numbers each); BitmapTexture:
+        scaling.  A texture keeps its kind and its bitmap.  `texture` is a name or index.  The flat description and any uploaded
+        scene follow (c2rt_scene_set_textures).  A bad name or index, or a key of another kind, changes nothing."""
+        i = self.index("textures", texture)
+        _check_host(host_lib.c2rt_host_scene_set_texture(
+            self._h, i, _floats(color1, 3, "color1"), _floats(color2, 3, "color2"), _doubles(size, 1, "size"),
+            _floats(colorU, 9, "colorU"), _floats(colorV, 9, "colorV"), _doubles(freqU, 3, "freqU"), _doubles(freqV, 3, "freqV"),
+            _floats(scaling, 1, "scaling")))
+
+    def set_light(self, light, pos=None, color=None, power=None):
+        """As if the light's entry in the scene file had the given keys replaced (None: kept): pos, color (three numbers each),
+        power.  `light` is a name or index.  The flat description and any uploaded scene follow (c2rt_scene_set_lights).  A bad
+        name or index changes nothing."""
+        i = self.index("lights", light)
+        _check_host(host_lib.c2rt_host_scene_set_light(self._h, i, _doubles(pos, 3, "pos"), _floats(color, 3, "color"),
+                                                       _floats(power, 1, "power")))
+
+    def _name(self, section, entity):
+        """The scene file's name of an entity given by name or index (the host mirror's edits take references by name)."""
+        if isinstance(entity, str):
+            return entity
+        p = host_lib.c2rt_host_scene_name(self._h, section.encode(), int(entity))
+        if p is None:
+            raise KeyError(f"{section[:-1]} {entity} does not exist or has no name")
+        return p.decode()
+
     def frame_blocks(self, seed=0, count_rays=False):
         cam, st = Camera(), Settings()
         host_lib.c2rt_host_frame_blocks(self._h, seed, int(count_rays), C.byref(cam), C.byref(st))
@@ -382,6 +451,24 @@ class HostScene:
         return rgb, a, st
 
 
+def _floats(v, n, what):
+    """None, or a C float array of the n numbers of v (a number when n == 1)."""
+    return _array(v, n, what, C.c_float)
+
+
+def _doubles(v, n, what):
+    return _array(v, n, what, C.c_double)
+
+
+def _array(v, n, what, ctype):
+    if v is None:
+        return None
+    vals = np.asarray(v, np.float64).reshape(-1)
+    if len(vals) != n:
+        raise ValueError(f"{what} needs {n} numbers, got {len(vals)}")
+    return C.cast((ctype * n)(*vals.tolist()), C.c_void_p)
+
+
 def _points(a):
     a = np.ascontiguousarray(a, np.float64)
     if a.ndim != 2 or a.shape[1] != 3:
@@ -427,6 +514,50 @@ def scene_set_nodes(scene_handle, nodes, geom=None, transform=None, inverse=None
         tf.append(a)
     ptr = lambda a: None if a is None else a.ctypes.data  # noqa: E731
     _check(lib.c2rt_scene_set_nodes(scene_handle, n, ptr(ids), ptr(g), *[ptr(a) for a in tf]))
+
+
+def _entries(a, n, per, dtype, what):
+    a = np.ascontiguousarray(a, dtype).reshape(-1)
+    if len(a) != per * n:
+        raise ValueError(f"{what} has {len(a)} elements, {per * n} expected")
+    return a
+
+
+def scene_set_node_shaders(scene_handle, nodes, shader):
+    """c2rt_scene_set_node_shaders on an uploaded scene: entry i points node nodes[i] at shader index shader[i] (description
+    indices, as in c2rt_scene_desc)."""
+    ids = np.ascontiguousarray(nodes, np.uint32).reshape(-1)
+    sh = _entries(shader, len(ids), 1, np.int32, "shader")
+    _check(lib.c2rt_scene_set_node_shaders(scene_handle, len(ids), ids.ctypes.data, sh.ctypes.data))
+
+
+def scene_set_shaders(scene_handle, shaders, type, color, texture, exponent, strength):
+    """c2rt_scene_set_shaders on an uploaded scene: entry i replaces shader shaders[i] with type[i] (C2RT_SHADER_*), color[i]
+    (three floats), texture[i] (a texture index, < 0: none), exponent[i] and strength[i]."""
+    ids = np.ascontiguousarray(shaders, np.uint32).reshape(-1)
+    n = len(ids)
+    arrs = [_entries(type, n, 1, np.int32, "type"), _entries(color, n, 3, np.float32, "color"),
+            _entries(texture, n, 1, np.int32, "texture"), _entries(exponent, n, 1, np.float64, "exponent"),
+            _entries(strength, n, 1, np.float32, "strength")]
+    _check(lib.c2rt_scene_set_shaders(scene_handle, n, ids.ctypes.data, *[a.ctypes.data for a in arrs]))
+
+
+def scene_set_textures(scene_handle, textures, colors, params):
+    """c2rt_scene_set_textures on an uploaded scene: entry i replaces texture textures[i]'s colors[i] (18 floats) and params[i]
+    (6 doubles), laid out as c2rt_scene_desc's tex_colors / tex_params; a bitmap reads params[i][0] (scaling) only."""
+    ids = np.ascontiguousarray(textures, np.uint32).reshape(-1)
+    n = len(ids)
+    c, p = _entries(colors, n, 18, np.float32, "colors"), _entries(params, n, 6, np.float64, "params")
+    _check(lib.c2rt_scene_set_textures(scene_handle, n, ids.ctypes.data, c.ctypes.data, p.ctypes.data))
+
+
+def scene_set_lights(scene_handle, lights, pos, color, power):
+    """c2rt_scene_set_lights on an uploaded scene: entry i replaces light lights[i]'s pos[i] (three doubles), color[i] (three
+    floats, not premultiplied) and power[i]."""
+    ids = np.ascontiguousarray(lights, np.uint32).reshape(-1)
+    n = len(ids)
+    arrs = [_entries(pos, n, 3, np.float64, "pos"), _entries(color, n, 3, np.float32, "color"), _entries(power, n, 1, np.float32, "power")]
+    _check(lib.c2rt_scene_set_lights(scene_handle, n, ids.ctypes.data, *[a.ctypes.data for a in arrs]))
 
 
 def render_device(scene_handle, cam, settings, d_rgb_ptr, d_argb_ptr=None, band=None, stream=None):

@@ -261,24 +261,39 @@ int current_device_locked(DeviceCtx*& c) {
 
 }  // namespace
 
-// The part of a scene that derive_records writes: the node records, the scene class, and the shader / texture order (MODE_SOLO
-// swaps the node's shader and its texture into record 0).  c2rt_scene_set_nodes edits and derives a copy of it, then commits it.
+// A scene's editable records in description order: the order of the c2rt_scene_desc arrays, which every index a caller passes
+// to the c2rt_scene_set_* calls refers to.  Nodes carry their raw fields only (geom, shader, M, Minv, MinvT, off); shaders,
+// textures and lights are what derive_shader / derive_texture / derive_light make of one description entry.  c2rt_scene_create
+// builds them, the edits change a copy of them, and derive_records makes the device records from them on every derive: the
+// device order (MODE_SOLO's swap) is never edited, so no record index reaches a caller.
+struct SceneSource {
+    std::vector<DevNode> nodes;
+    std::vector<DevShader> shaders;
+    std::vector<DevTex> textures;
+    std::vector<DevLight> lights;
+};
+
+// What derive_records makes of a SceneSource: the node records with everything that follows from their raw fields, the scene
+// class, and the shader / texture records in device order (MODE_SOLO swaps the node's shader and its texture into record 0).
 struct SceneRecords {
     std::vector<DevNode> nodes;          // the scene's records (texel pointers patched per device at upload)
     std::vector<DevShader> shaders;
     std::vector<DevTex> textures;
-    std::vector<size_t> tex_offset;      // per texture, in texels (general-form bitmaps only)
-    std::vector<long long> quad_offset, pal_offset;   // per texture; -1 = general form
+    std::vector<int> tex_slot;           // per texture record: the description texture it holds (its slot in the offset tables)
     int mode;                            // kernel specialisation (render_kernel.cu MODE_*)
 };
 
 struct c2rt_scene : SceneRecords {
     uint64_t id;
+    SceneSource src;
     DevScene host;                       // constant block; record arrays copied in from the vectors when they fit
     std::vector<DevGeom> geoms;
     bool big = false;                    // beyond the constant block: the records go to global memory (MODE_BIG)
     bool no_solo = false;                // C2RT_NO_SOLO at creation (test hook: no MODE_SOLO)
     void* d_records[C2RT_MAX_GPUS][4];   // big scenes, per context device: nodes, geoms, shaders, textures
+    // per description texture, then the six environment faces: where its bitmap lives
+    std::vector<size_t> tex_offset;      // in texels (general-form bitmaps only)
+    std::vector<long long> quad_offset, pal_offset;   // -1 = general form
     std::vector<float4> texels;          // bitmaps in the general form, float4 per texel
     float4* d_texels[C2RT_MAX_GPUS];     // per context device
     // bitmaps with <= 256 distinct colours (scene_dev.h DevTex::quads): index quads + 256-entry palettes
@@ -401,7 +416,71 @@ void build_bitmap(c2rt_scene* s, const DevTex& t, const float* src, int slot) {
     }
 }
 
-void derive_records(const c2rt_scene& s, SceneRecords& rec);
+void derive_records(const c2rt_scene& s, const SceneSource& src, SceneRecords& rec);
+
+// The shader record of one description entry (c2rt_scene_desc shader arrays): a negative texture index is "none", -1
+DevShader derive_shader(int type, const float* color, int tex, double exponent, float strength) {
+    DevShader sh;
+    memset(&sh, 0, sizeof sh);
+    sh.type = type;
+    sh.tex = tex < 0 ? -1 : tex;
+    memcpy(sh.color, color, sizeof sh.color);
+    sh.exponent = exponent;
+    sh.strength = strength;
+    return sh;
+}
+
+// The parameters of texture record t (whose type, and for a bitmap size and texels, are set) from one description entry:
+// colors [18] and params [6].  A bitmap reads params[0] (scaling) only.  Checker keeps 1 / size; Procedure2 keeps its
+// frequencies in 2^-32 revolutions per unit (render_kernel.cu sin_phase / sin_rev) and, per axis, the |u|, |v| up to which
+// every phase stays below 2^18 revolutions, as the high word of a double (compared against the coordinate's high word).
+void derive_texture(DevTex& t, const float* colors, const double* params) {
+    if (t.type == C2RT_TEX_BITMAP) {
+        t.d[0] = params[0];
+        return;
+    }
+    memcpy(t.c, colors, 18 * sizeof(float));
+    memcpy(t.d, params, 6 * sizeof(double));
+    if (t.type == C2RT_TEX_CHECKER) t.d[1] = 1.0 / t.d[0];
+    if (t.type == C2RT_TEX_PROCEDURE2) {
+        for (int a = 0; a < 2; a++) {
+            double fmax = 0.0;
+            for (int k = 0; k < 3; k++) {
+                double& f = t.d[3 * a + k];
+                f = f / 6.283185307179586476925 * 4294967296.0;
+                fmax = std::isfinite(f) ? std::max(fmax, std::fabs(f)) : INFINITY;
+            }
+            const double lim = fmax > 0 ? 262144.0 * 4294967296.0 / fmax : INFINITY;   // (fmax = inf: 0, always the two-step path)
+            uint64_t bits;
+            memcpy(&bits, &lim, 8);
+            (a ? t.h : t.w) = (int)(uint32_t)(bits >> 32);
+        }
+    }
+}
+
+// The light record of one description entry (c2rt_scene_desc light arrays)
+DevLight derive_light(const double* pos, const float* color, float power) {
+    DevLight L;
+    memset(&L, 0, sizeof L);
+    memcpy(L.pos, pos, 3 * sizeof(double));
+    // light.d:11-14: Color * float in FP32
+    for (int k = 0; k < 3; k++) L.color[k] = color[k] * power;
+    float intensity = (L.color[0] + L.color[1] + L.color[2]) / 3;  // color.d:141-144
+    L.lit = intensity != 0;
+    for (int k = 0; k < 3; k++) L.posf[k] = (float)L.pos[k];
+    L.near2 = (float)(0.0576 * (L.pos[0] * L.pos[0] + L.pos[1] * L.pos[1] + L.pos[2] * L.pos[2]));
+    return L;
+}
+
+// The scene block's lights and its list of lit ones
+void set_lights(DevScene& h, const std::vector<DevLight>& lights) {
+    h.n_lit = 0;
+    memset(h.lit, 0, sizeof h.lit);
+    for (size_t i = 0; i < lights.size(); i++) {
+        h.lights[i] = lights[i];
+        if (lights[i].lit) h.lit[h.n_lit++] = (int)i;
+    }
+}
 
 int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
     if (!d) return fail(C2RT_ERR_INVALID_ARG, "scene description is null");
@@ -429,12 +508,14 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
 
     DevScene& h = s->host;
     memset(&h, 0, sizeof h);
-    DevNode zn; DevGeom zg; DevShader zs; DevTex zt;
-    memset(&zn, 0, sizeof zn); memset(&zg, 0, sizeof zg); memset(&zs, 0, sizeof zs); memset(&zt, 0, sizeof zt);
-    s->nodes.assign(d->n_nodes, zn);
+    DevNode zn; DevGeom zg; DevTex zt;
+    memset(&zn, 0, sizeof zn); memset(&zg, 0, sizeof zg); memset(&zt, 0, sizeof zt);
+    SceneSource& src = s->src;
+    src.nodes.assign(d->n_nodes, zn);
     s->geoms.assign(d->n_geoms, zg);
-    s->shaders.assign(d->n_shaders, zs);
-    s->textures.assign(d->n_textures, zt);
+    src.shaders.resize(d->n_shaders);
+    src.textures.assign(d->n_textures, zt);
+    src.lights.resize(d->n_lights);
     h.n_nodes = d->n_nodes; h.n_geoms = d->n_geoms; h.n_shaders = d->n_shaders; h.n_textures = d->n_textures; h.n_lights = d->n_lights;
 
     for (uint32_t i = 0; i < d->n_geoms; i++) {
@@ -461,28 +542,9 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
     s->quad_offset.assign(d->n_textures + 6, -1);
     s->pal_offset.assign(d->n_textures + 6, -1);
     for (uint32_t i = 0; i < d->n_textures; i++) {
-        DevTex& t = s->textures[i];
+        DevTex& t = src.textures[i];
         t.type = d->tex_type[i];
         if (t.type < C2RT_TEX_CHECKER || t.type > C2RT_TEX_BITMAP) return fail(C2RT_ERR_INVALID_ARG, "texture %u: unknown type %d", i, t.type);
-        memcpy(t.c, d->tex_colors + 18 * i, 18 * sizeof(float));
-        memcpy(t.d, d->tex_params + 6 * i, 6 * sizeof(double));
-        if (t.type == C2RT_TEX_CHECKER) t.d[1] = 1.0 / t.d[0];
-        if (t.type == C2RT_TEX_PROCEDURE2) {
-            // frequencies in 2^-32 revolutions per unit (render_kernel.cu sin_phase / sin_rev), and the |u|, |v| up to which every
-            // phase stays below 2^18 revolutions, as the high word of a double (compared against the coordinate's high word)
-            for (int a = 0; a < 2; a++) {
-                double fmax = 0.0;
-                for (int k = 0; k < 3; k++) {
-                    double& f = t.d[3 * a + k];
-                    f = f / 6.283185307179586476925 * 4294967296.0;
-                    fmax = std::isfinite(f) ? std::max(fmax, std::fabs(f)) : INFINITY;
-                }
-                const double lim = fmax > 0 ? 262144.0 * 4294967296.0 / fmax : INFINITY;   // (fmax = inf: 0, always the two-step path)
-                uint64_t bits;
-                memcpy(&bits, &lim, 8);
-                (a ? t.h : t.w) = (int)(uint32_t)(bits >> 32);
-            }
-        }
         if (t.type == C2RT_TEX_BITMAP) {
             t.w = d->tex_width[i]; t.h = d->tex_height[i];
             if (t.w <= 0 || t.h <= 0) return fail(C2RT_ERR_INVALID_ARG, "texture %u: empty bitmap", i);
@@ -490,6 +552,7 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
             if (!d->texels || off + n > d->n_texels) return fail(C2RT_ERR_INVALID_ARG, "texture %u: texel range outside `texels`", i);
             build_bitmap(s, t, d->texels + 3 * off, (int)i);
         }
+        derive_texture(t, d->tex_colors + 18 * i, d->tex_params + 6 * i);
     }
     // environment (c2rt.h C2RT_ENV_CUBEMAP): six more bitmap records, slots n_textures .. n_textures + 5 of the offset tables
     h.env_type = d->env_type;
@@ -505,30 +568,15 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
             build_bitmap(s, t, d->texels + 3 * off, (int)d->n_textures + f);
         }
     for (uint32_t i = 0; i < d->n_shaders; i++) {
-        DevShader& sh = s->shaders[i];
-        sh.type = d->shader_type[i];
-        if (sh.type != C2RT_SHADER_LAMBERT && sh.type != C2RT_SHADER_PHONG) return fail(C2RT_ERR_INVALID_ARG, "shader %u: unknown type %d", i, sh.type);
-        sh.tex = d->shader_texture[i];
-        if (sh.tex >= (int)d->n_textures) return fail(C2RT_ERR_INVALID_ARG, "shader %u: texture index %d out of range", i, sh.tex);
-        if (sh.tex < 0) sh.tex = -1;
-        memcpy(sh.color, d->shader_color + 3 * i, 3 * sizeof(float));
-        sh.exponent = d->shader_exponent[i];
-        sh.strength = d->shader_strength[i];
+        const int type = d->shader_type[i], tex = d->shader_texture[i];
+        if (type != C2RT_SHADER_LAMBERT && type != C2RT_SHADER_PHONG) return fail(C2RT_ERR_INVALID_ARG, "shader %u: unknown type %d", i, type);
+        if (tex >= (int)d->n_textures) return fail(C2RT_ERR_INVALID_ARG, "shader %u: texture index %d out of range", i, tex);
+        src.shaders[i] = derive_shader(type, d->shader_color + 3 * i, tex, d->shader_exponent[i], d->shader_strength[i]);
     }
-    for (uint32_t i = 0; i < d->n_lights; i++) {
-        DevLight& L = h.lights[i];
-        memcpy(L.pos, d->light_pos + 3 * i, 3 * sizeof(double));
-        // light.d:11-14: Color * float in FP32
-        float pw = d->light_power[i];
-        for (int k = 0; k < 3; k++) L.color[k] = d->light_color[3 * i + k] * pw;
-        float intensity = (L.color[0] + L.color[1] + L.color[2]) / 3;  // color.d:141-144
-        L.lit = intensity != 0;
-        for (int k = 0; k < 3; k++) L.posf[k] = (float)L.pos[k];
-        L.near2 = (float)(0.0576 * (L.pos[0] * L.pos[0] + L.pos[1] * L.pos[1] + L.pos[2] * L.pos[2]));
-        if (L.lit) h.lit[h.n_lit++] = (int)i;
-    }
+    for (uint32_t i = 0; i < d->n_lights; i++) src.lights[i] = derive_light(d->light_pos + 3 * i, d->light_color + 3 * i, d->light_power[i]);
+    set_lights(h, src.lights);
     for (uint32_t i = 0; i < d->n_nodes; i++) {
-        DevNode& nd = s->nodes[i];
+        DevNode& nd = src.nodes[i];
         nd.geom = d->node_geom[i];
         nd.shader = d->node_shader[i];
         if (nd.geom < 0 || nd.geom >= (int)d->n_geoms) return fail(C2RT_ERR_INVALID_ARG, "node %u: geometry index %d out of range", i, nd.geom);
@@ -540,7 +588,7 @@ int validate_and_build(const c2rt_scene_desc* d, c2rt_scene* s) {
     }
     const char* no_solo = getenv("C2RT_NO_SOLO");   // test hook: keep one-plane scenes on the general plane-only kernel
     s->no_solo = no_solo && no_solo[0] == '1';
-    derive_records(*s, *s);
+    derive_records(*s, src, *s);
     return C2RT_OK;
 }
 
@@ -565,23 +613,19 @@ static int proc2_u_pattern(const DevTex& t) {
     return UPAT_DISTINCT;   // (unreachable: first1 == 0 and first2 == 1 contradict each other)
 }
 
-// Everything that follows from the raw node fields (geom, shader, M, Minv, MinvT, off) of r.nodes: per node the bound, its FP32
-// form for the cull, NODE_IDENTITY / NODE_UNBOUNDED, kind and wp; then the scene class r.mode with MODE_SOLO's swap.  It reads
-// the scene's geometry records, its light count and the decisions taken at creation (big, no_solo), and no description, so
-// c2rt_scene_create (r is the scene itself) and c2rt_scene_set_nodes (r is the edit's copy) derive alike.
-void derive_records(const c2rt_scene& s, SceneRecords& rec) {
+// The device records of src: per node the bound, its FP32 form for the cull, NODE_IDENTITY / NODE_UNBOUNDED, kind and wp; then
+// the scene class rec.mode with MODE_SOLO's swap.  It reads the scene's geometry records, its light count and the decisions
+// taken at creation (big, no_solo), and no description, so c2rt_scene_create (rec is the scene itself) and the edits (rec is
+// the edit's copy) derive alike.
+void derive_records(const c2rt_scene& s, const SceneSource& src, SceneRecords& rec) {
+    rec.nodes = src.nodes;   // raw fields only: every derived field below starts from zero
+    rec.shaders = src.shaders;
+    rec.textures = src.textures;
+    rec.tex_slot.resize(src.textures.size());
+    for (size_t t = 0; t < rec.tex_slot.size(); t++) rec.tex_slot[t] = (int)t;
     const int n_nodes = (int)rec.nodes.size();
     for (int i = 0; i < n_nodes; i++) {
-        // only the raw fields carry over: a node that changes class keeps nothing of its old derived fields
-        const DevNode raw = rec.nodes[i];
         DevNode& nd = rec.nodes[i];
-        memset(&nd, 0, sizeof nd);
-        nd.geom = raw.geom;
-        nd.shader = raw.shader;
-        memcpy(nd.M, raw.M, sizeof nd.M);
-        memcpy(nd.Minv, raw.Minv, sizeof nd.Minv);
-        memcpy(nd.MinvT, raw.MinvT, sizeof nd.MinvT);
-        memcpy(nd.off, raw.off, sizeof nd.off);
         if (is_identity(nd.M) && is_identity(nd.Minv) && is_identity(nd.MinvT)) nd.flags |= NODE_IDENTITY;
         Bound b = bound_of(s.geoms, nd.geom);
         if (b.finite) {
@@ -654,8 +698,7 @@ void derive_records(const c2rt_scene& s, SceneRecords& rec) {
         if (ng.type >= C2RT_GEOM_CSG_UNION && ng.depth != 1) rec.mode |= MODE_NESTED | MODE_GENERIC | MODE_BOUNDED;
     }
     // MODE_SOLO: exactly one node, a world-space plane, and exactly one light.  The node's shader and that shader's
-    // texture are swapped into record 0 so the kernel addresses every scene constant statically.  On records this swap
-    // has already been applied to (node 0's shader is 0, its texture 0) it changes nothing.
+    // texture are swapped into record 0 so the kernel addresses every scene constant statically.
     if (!s.big && rec.mode == 0 && n_nodes == 1 && s.host.n_lights == 1 && rec.nodes[0].kind == KIND_PLANE_W && !s.no_solo) {
         const int si = rec.nodes[0].shader;
         std::swap(rec.shaders[0], rec.shaders[si]);
@@ -663,9 +706,7 @@ void derive_records(const c2rt_scene& s, SceneRecords& rec) {
         const int ti = rec.shaders[0].tex;
         if (ti >= 0) {
             std::swap(rec.textures[0], rec.textures[ti]);
-            std::swap(rec.tex_offset[0], rec.tex_offset[ti]);
-            std::swap(rec.quad_offset[0], rec.quad_offset[ti]);
-            std::swap(rec.pal_offset[0], rec.pal_offset[ti]);
+            std::swap(rec.tex_slot[0], rec.tex_slot[ti]);
             for (DevShader& sh : rec.shaders) {
                 if (sh.tex == 0) sh.tex = ti;
                 else if (sh.tex == ti) sh.tex = 0;
@@ -727,10 +768,11 @@ int make_resident(c2rt_scene* s, int di, cudaStream_t st) {
     const int n_bmp_slots = s->host.n_textures + (s->host.env_type == C2RT_ENV_CUBEMAP ? 6 : 0);
     for (int t = 0; t < n_bmp_slots; t++) {
         DevTex& tx = t < s->host.n_textures ? s->textures[t] : s->host.env_faces[t - s->host.n_textures];
-        const bool bmp = tx.type == C2RT_TEX_BITMAP, pal = bmp && s->quad_offset[t] >= 0;
-        tx.texels = (bmp && !pal) ? s->d_texels[di] + s->tex_offset[t] : nullptr;
-        tx.quads = pal ? s->d_quads[di] + s->quad_offset[t] : nullptr;
-        tx.palette = pal ? s->d_palettes[di] + s->pal_offset[t] : nullptr;
+        const int slot = t < s->host.n_textures ? s->tex_slot[t] : t;
+        const bool bmp = tx.type == C2RT_TEX_BITMAP, pal = bmp && s->quad_offset[slot] >= 0;
+        tx.texels = (bmp && !pal) ? s->d_texels[di] + s->tex_offset[slot] : nullptr;
+        tx.quads = pal ? s->d_quads[di] + s->quad_offset[slot] : nullptr;
+        tx.palette = pal ? s->d_palettes[di] + s->pal_offset[slot] : nullptr;
     }
     if (s->big) {
         const void* src[4] = {s->nodes.data(), s->geoms.data(), s->shaders.data(), s->textures.data()};
@@ -1251,6 +1293,33 @@ int device_band_locked(c2rt_scene* s, const c2rt_camera* cam, const c2rt_setting
     return C2RT_OK;
 }
 
+// The edits' common part, after their argument checks: under the library lock, `edit` changes a copy of the scene's
+// description-order records, which is derived; nothing of the scene changes before the devices are idle.  Kernels in flight on
+// any stream of these devices read the bounds (and the scene block): wait for them, then rewrite the bounds in place and commit.
+// The scene block, or the global records of a big scene, is re-uploaded by make_resident at the next use on each device: the
+// scene gets a new id, which no device holds.
+template <class Edit>
+int edit_scene(c2rt_scene* s, Edit&& edit) {
+    std::lock_guard<std::mutex> g(g_mu);
+    if (s->n_dev != g_ctx.n) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
+    SceneSource src = s->src;
+    edit(src);
+    SceneRecords rec;
+    derive_records(*s, src, rec);
+    const std::vector<float4> bounds = node_bounds(rec);
+    for (int i = 0; i < s->n_dev; i++) {
+        CU(cudaSetDevice(g_ctx.d[i].dev));
+        CU(cudaDeviceSynchronize());
+        CU(cudaMemcpy(s->d_bounds[i], bounds.data(), bounds.size() * sizeof(float4), cudaMemcpyHostToDevice));
+    }
+    CU(cudaSetDevice(g_ctx.d[0].dev));
+    static_cast<SceneRecords&>(*s) = std::move(rec);
+    s->src = std::move(src);
+    set_lights(s->host, s->src.lights);
+    s->id = g_ctx.next_scene_id++;
+    return C2RT_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1342,39 +1411,82 @@ int c2rt_scene_set_nodes(c2rt_scene* s, size_t n, const uint32_t* nodes, const i
     if (n == 0) return C2RT_OK;
     if (!nodes) return fail(C2RT_ERR_INVALID_ARG, "nodes is null");
     for (size_t k = 0; k < n; k++) {
-        if (nodes[k] >= s->nodes.size())
-            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: node index %u out of range (%zu nodes)", k, nodes[k], s->nodes.size());
+        if (nodes[k] >= s->src.nodes.size())
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: node index %u out of range (%zu nodes)", k, nodes[k], s->src.nodes.size());
         if (geom && (geom[k] < 0 || (size_t)geom[k] >= s->geoms.size()))
             return fail(C2RT_ERR_INVALID_ARG, "entry %zu: geometry index %d out of range (%zu geometries)", k, geom[k], s->geoms.size());
     }
-    std::lock_guard<std::mutex> g(g_mu);
-    if (s->n_dev != g_ctx.n) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
-    // the edit and its derivation on a copy; nothing of the scene changes before the devices are idle
-    SceneRecords work = *s;
-    for (size_t k = 0; k < n; k++) {
-        DevNode& nd = work.nodes[nodes[k]];
-        if (geom) nd.geom = geom[k];
-        if (transform) {
-            memcpy(nd.M, transform + 9 * k, sizeof nd.M);
-            memcpy(nd.Minv, inverse + 9 * k, sizeof nd.Minv);
-            memcpy(nd.MinvT, inverse_t + 9 * k, sizeof nd.MinvT);
-            memcpy(nd.off, offset + 3 * k, sizeof nd.off);
+    return edit_scene(s, [&](SceneSource& src) {
+        for (size_t k = 0; k < n; k++) {
+            DevNode& nd = src.nodes[nodes[k]];
+            if (geom) nd.geom = geom[k];
+            if (transform) {
+                memcpy(nd.M, transform + 9 * k, sizeof nd.M);
+                memcpy(nd.Minv, inverse + 9 * k, sizeof nd.Minv);
+                memcpy(nd.MinvT, inverse_t + 9 * k, sizeof nd.MinvT);
+                memcpy(nd.off, offset + 3 * k, sizeof nd.off);
+            }
         }
+    });
+}
+
+int c2rt_scene_set_node_shaders(c2rt_scene* s, size_t n, const uint32_t* nodes, const int32_t* shader) {
+    if (!s) return fail(C2RT_ERR_INVALID_ARG, "scene is null");
+    if (n == 0) return C2RT_OK;
+    if (!nodes || !shader) return fail(C2RT_ERR_INVALID_ARG, "nodes and shader must be non-null");
+    for (size_t k = 0; k < n; k++) {
+        if (nodes[k] >= s->src.nodes.size())
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: node index %u out of range (%zu nodes)", k, nodes[k], s->src.nodes.size());
+        if (shader[k] < 0 || (size_t)shader[k] >= s->src.shaders.size())
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: shader index %d out of range (%zu shaders)", k, shader[k], s->src.shaders.size());
     }
-    derive_records(*s, work);
-    // kernels in flight on any stream of these devices read the bounds (and the scene block): wait for them, then rewrite the
-    // bounds in place.  The scene block, or the global records of a big scene, is re-uploaded by make_resident at the next use
-    // on each device: the scene gets a new id, which no device holds.
-    const std::vector<float4> bounds = node_bounds(work);
-    for (int i = 0; i < s->n_dev; i++) {
-        CU(cudaSetDevice(g_ctx.d[i].dev));
-        CU(cudaDeviceSynchronize());
-        CU(cudaMemcpy(s->d_bounds[i], bounds.data(), bounds.size() * sizeof(float4), cudaMemcpyHostToDevice));
+    return edit_scene(s, [&](SceneSource& src) {
+        for (size_t k = 0; k < n; k++) src.nodes[nodes[k]].shader = shader[k];
+    });
+}
+
+int c2rt_scene_set_shaders(c2rt_scene* s, size_t n, const uint32_t* shaders, const int32_t* type, const float* color,
+                           const int32_t* texture, const double* exponent, const float* strength) {
+    if (!s) return fail(C2RT_ERR_INVALID_ARG, "scene is null");
+    if (n == 0) return C2RT_OK;
+    if (!shaders || !type || !color || !texture || !exponent || !strength)
+        return fail(C2RT_ERR_INVALID_ARG, "shaders, type, color, texture, exponent and strength must be non-null");
+    for (size_t k = 0; k < n; k++) {
+        if (shaders[k] >= s->src.shaders.size())
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: shader index %u out of range (%zu shaders)", k, shaders[k], s->src.shaders.size());
+        if (type[k] != C2RT_SHADER_LAMBERT && type[k] != C2RT_SHADER_PHONG)
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: unknown shader type %d", k, type[k]);
+        if (texture[k] >= (int)s->src.textures.size())
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: texture index %d out of range (%zu textures)", k, texture[k], s->src.textures.size());
     }
-    CU(cudaSetDevice(g_ctx.d[0].dev));
-    static_cast<SceneRecords&>(*s) = std::move(work);
-    s->id = g_ctx.next_scene_id++;
-    return C2RT_OK;
+    return edit_scene(s, [&](SceneSource& src) {
+        for (size_t k = 0; k < n; k++)
+            src.shaders[shaders[k]] = derive_shader(type[k], color + 3 * k, texture[k], exponent[k], strength[k]);
+    });
+}
+
+int c2rt_scene_set_textures(c2rt_scene* s, size_t n, const uint32_t* textures, const float* colors, const double* params) {
+    if (!s) return fail(C2RT_ERR_INVALID_ARG, "scene is null");
+    if (n == 0) return C2RT_OK;
+    if (!textures || !colors || !params) return fail(C2RT_ERR_INVALID_ARG, "textures, colors and params must be non-null");
+    for (size_t k = 0; k < n; k++)
+        if (textures[k] >= s->src.textures.size())
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: texture index %u out of range (%zu textures)", k, textures[k], s->src.textures.size());
+    return edit_scene(s, [&](SceneSource& src) {
+        for (size_t k = 0; k < n; k++) derive_texture(src.textures[textures[k]], colors + 18 * k, params + 6 * k);
+    });
+}
+
+int c2rt_scene_set_lights(c2rt_scene* s, size_t n, const uint32_t* lights, const double* pos, const float* color, const float* power) {
+    if (!s) return fail(C2RT_ERR_INVALID_ARG, "scene is null");
+    if (n == 0) return C2RT_OK;
+    if (!lights || !pos || !color || !power) return fail(C2RT_ERR_INVALID_ARG, "lights, pos, color and power must be non-null");
+    for (size_t k = 0; k < n; k++)
+        if (lights[k] >= s->src.lights.size())
+            return fail(C2RT_ERR_INVALID_ARG, "entry %zu: light index %u out of range (%zu lights)", k, lights[k], s->src.lights.size());
+    return edit_scene(s, [&](SceneSource& src) {
+        for (size_t k = 0; k < n; k++) src.lights[lights[k]] = derive_light(pos + 3 * k, color + 3 * k, power[k]);
+    });
 }
 
 int c2rt_render_device(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, const c2rt_band* band, float* d_rgb,

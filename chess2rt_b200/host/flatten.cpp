@@ -1,6 +1,7 @@
 #include "flatten.hpp"
 
 #include <cstring>
+#include <string>
 
 namespace rt {
 namespace {
@@ -52,83 +53,41 @@ FlatScene flatten(const Scene& scene) {
     }
 
     // textures
-    for (size_t i = 0; i < scene.textures.size(); i++) {
-        const Texture* t = scene.textures[i].get();
-        float colors[18] = {0};
-        double params[6] = {0};
-        int type, w = 0, h = 0;
+    for (auto& t : scene.textures) {
+        const FlatTexture ft = flattenTexture(*t);
         uint64_t off = 0;
-        if (auto* ch = dynamic_cast<const Checker*>(t)) {
-            type = C2RT_TEX_CHECKER;
-            colors[0] = ch->color1.r; colors[1] = ch->color1.g; colors[2] = ch->color1.b;
-            colors[3] = ch->color2.r; colors[4] = ch->color2.g; colors[5] = ch->color2.b;
-            params[0] = ch->size;
-        } else if (auto* pr = dynamic_cast<const Procedure2*>(t)) {
-            type = C2RT_TEX_PROCEDURE2;
-            // texture.d:81 reads exactly three entries of each array (a D RangeError otherwise)
-            if (pr->colorU.size() < 3 || pr->colorV.size() < 3 || pr->freqU.size() < 3 || pr->freqV.size() < 3)
-                throw InvalidSceneException("Procedure2 needs three colorU / colorV / freqU / freqV entries");
-            for (int k = 0; k < 3; k++) {
-                colors[3 * k + 0] = pr->colorU[k].r; colors[3 * k + 1] = pr->colorU[k].g; colors[3 * k + 2] = pr->colorU[k].b;
-                colors[9 + 3 * k + 0] = pr->colorV[k].r; colors[9 + 3 * k + 1] = pr->colorV[k].g; colors[9 + 3 * k + 2] = pr->colorV[k].b;
-                params[k] = pr->freqU[k];
-                params[3 + k] = pr->freqV[k];
-            }
-        } else if (auto* bm = dynamic_cast<const BitmapTexture*>(t)) {
-            type = C2RT_TEX_BITMAP;
-            w = (int)bm->bmp.width();
-            h = (int)bm->bmp.height();
-            params[0] = (double)bm->scaling;  // `u *= scaling` widens the float (texture.d:118)
+        if (auto* bm = dynamic_cast<const BitmapTexture*>(t.get())) {
             off = f.texels.size() / 3;
             for (const Color& c : bm->bmp.data.pixels) {
                 f.texels.push_back(c.r);
                 f.texels.push_back(c.g);
                 f.texels.push_back(c.b);
             }
-        } else {
-            throw InvalidSceneException("unknown Texture subclass");
         }
-        f.tex_type.push_back(type);
-        f.tex_width.push_back(w);
-        f.tex_height.push_back(h);
+        f.tex_type.push_back(ft.type);
+        f.tex_width.push_back(ft.width);
+        f.tex_height.push_back(ft.height);
         f.tex_texel_offset.push_back(off);
-        f.tex_colors.insert(f.tex_colors.end(), colors, colors + 18);
-        f.tex_params.insert(f.tex_params.end(), params, params + 6);
+        f.tex_colors.insert(f.tex_colors.end(), ft.colors, ft.colors + 18);
+        f.tex_params.insert(f.tex_params.end(), ft.params, ft.params + 6);
     }
 
     // shaders
-    for (size_t i = 0; i < scene.shaders.size(); i++) {
-        const Shader* s = scene.shaders[i].get();
-        int type, tex = -1;
-        double exponent = 0;
-        float strength = 0;
-        if (auto* la = dynamic_cast<const Lambert*>(s)) {
-            type = C2RT_SHADER_LAMBERT;
-            if (la->texture) tex = indexOf(scene.textures, la->texture);
-        } else if (auto* ph = dynamic_cast<const Phong*>(s)) {
-            type = C2RT_SHADER_PHONG;
-            if (ph->texture) tex = indexOf(scene.textures, ph->texture);
-            exponent = ph->exponent;
-            strength = ph->strength;
-        } else {
-            throw InvalidSceneException("unknown Shader subclass");
-        }
-        f.shader_type.push_back(type);
-        f.shader_texture.push_back(tex);
-        f.shader_color.push_back(s->color.r);
-        f.shader_color.push_back(s->color.g);
-        f.shader_color.push_back(s->color.b);
-        f.shader_exponent.push_back(exponent);
-        f.shader_strength.push_back(strength);
+    for (auto& s : scene.shaders) {
+        const FlatShader fs = flattenShader(scene, *s);
+        f.shader_type.push_back(fs.type);
+        f.shader_texture.push_back(fs.texture);
+        f.shader_color.insert(f.shader_color.end(), fs.color, fs.color + 3);
+        f.shader_exponent.push_back(fs.exponent);
+        f.shader_strength.push_back(fs.strength);
     }
 
-    // lights (PointLight is the only Light subclass the reference has: light.d:52)
+    // lights
     for (auto& l : scene.lights) {
-        auto* pl = dynamic_cast<const PointLight*>(l.get());
-        if (!pl) throw InvalidSceneException("unknown Light subclass");
-        f.light_pos.push_back(pl->pos.x); f.light_pos.push_back(pl->pos.y); f.light_pos.push_back(pl->pos.z);
-        f.light_color.push_back(pl->lightColor.r); f.light_color.push_back(pl->lightColor.g); f.light_color.push_back(pl->lightColor.b);
-        f.light_power.push_back(pl->lightPower);
+        const FlatLight fl = flattenLight(*l);
+        f.light_pos.insert(f.light_pos.end(), fl.pos, fl.pos + 3);
+        f.light_color.insert(f.light_color.end(), fl.color, fl.color + 3);
+        f.light_power.push_back(fl.power);
     }
 
     // environment (cubemap extension: rt.hpp Environment): the six faces follow the bitmap textures' texels
@@ -172,6 +131,128 @@ FlatNode flattenNode(const Scene& scene, const Node& n) {
     f.offset[1] = n.transform.offset.y;
     f.offset[2] = n.transform.offset.z;
     return f;
+}
+
+FlatShader flattenShader(const Scene& scene, const Shader& s) {
+    FlatShader f;
+    f.texture = -1;
+    f.exponent = 0;
+    f.strength = 0;
+    if (auto* la = dynamic_cast<const Lambert*>(&s)) {
+        f.type = C2RT_SHADER_LAMBERT;
+        if (la->texture) f.texture = indexOf(scene.textures, la->texture);
+    } else if (auto* ph = dynamic_cast<const Phong*>(&s)) {
+        f.type = C2RT_SHADER_PHONG;
+        if (ph->texture) f.texture = indexOf(scene.textures, ph->texture);
+        f.exponent = ph->exponent;
+        f.strength = ph->strength;
+    } else {
+        throw InvalidSceneException("unknown Shader subclass");
+    }
+    f.color[0] = s.color.r; f.color[1] = s.color.g; f.color[2] = s.color.b;
+    return f;
+}
+
+FlatTexture flattenTexture(const Texture& t) {
+    FlatTexture f{};
+    if (auto* ch = dynamic_cast<const Checker*>(&t)) {
+        f.type = C2RT_TEX_CHECKER;
+        f.colors[0] = ch->color1.r; f.colors[1] = ch->color1.g; f.colors[2] = ch->color1.b;
+        f.colors[3] = ch->color2.r; f.colors[4] = ch->color2.g; f.colors[5] = ch->color2.b;
+        f.params[0] = ch->size;
+    } else if (auto* pr = dynamic_cast<const Procedure2*>(&t)) {
+        f.type = C2RT_TEX_PROCEDURE2;
+        // texture.d:81 reads exactly three entries of each array (a D RangeError otherwise)
+        if (pr->colorU.size() < 3 || pr->colorV.size() < 3 || pr->freqU.size() < 3 || pr->freqV.size() < 3)
+            throw InvalidSceneException("Procedure2 needs three colorU / colorV / freqU / freqV entries");
+        for (int k = 0; k < 3; k++) {
+            f.colors[3 * k + 0] = pr->colorU[k].r; f.colors[3 * k + 1] = pr->colorU[k].g; f.colors[3 * k + 2] = pr->colorU[k].b;
+            f.colors[9 + 3 * k + 0] = pr->colorV[k].r; f.colors[9 + 3 * k + 1] = pr->colorV[k].g; f.colors[9 + 3 * k + 2] = pr->colorV[k].b;
+            f.params[k] = pr->freqU[k];
+            f.params[3 + k] = pr->freqV[k];
+        }
+    } else if (auto* bm = dynamic_cast<const BitmapTexture*>(&t)) {
+        f.type = C2RT_TEX_BITMAP;
+        f.width = (int)bm->bmp.width();
+        f.height = (int)bm->bmp.height();
+        f.params[0] = (double)bm->scaling;  // `u *= scaling` widens the float (texture.d:118)
+    } else {
+        throw InvalidSceneException("unknown Texture subclass");
+    }
+    return f;
+}
+
+FlatLight flattenLight(const Light& l) {
+    // PointLight is the only Light subclass the reference has: light.d:52
+    auto* pl = dynamic_cast<const PointLight*>(&l);
+    if (!pl) throw InvalidSceneException("unknown Light subclass");
+    FlatLight f;
+    f.pos[0] = pl->pos.x; f.pos[1] = pl->pos.y; f.pos[2] = pl->pos.z;
+    f.color[0] = pl->lightColor.r; f.color[1] = pl->lightColor.g; f.color[2] = pl->lightColor.b;
+    f.power = pl->lightPower;
+    return f;
+}
+
+namespace {
+
+std::vector<uint32_t> editIds(const std::vector<int>& indices, size_t count, const char* what) {
+    std::vector<uint32_t> ids;
+    for (int i : indices) {
+        if (i < 0 || (size_t)i >= count) throw RTException(std::string(what) + " index " + std::to_string(i) + " out of range");
+        ids.push_back((uint32_t)i);
+    }
+    return ids;
+}
+
+}  // namespace
+
+int setNodeShaders(c2rt_scene* device, const Scene& scene, const std::vector<int>& nodes) {
+    const std::vector<uint32_t> ids = editIds(nodes, scene.nodes.size(), "node");
+    std::vector<int32_t> shader;
+    for (uint32_t i : ids) shader.push_back(flattenNode(scene, *scene.nodes[i]).shader);
+    return c2rt_scene_set_node_shaders(device, ids.size(), ids.data(), shader.data());
+}
+
+int setShaders(c2rt_scene* device, const Scene& scene, const std::vector<int>& shaders) {
+    const std::vector<uint32_t> ids = editIds(shaders, scene.shaders.size(), "shader");
+    std::vector<int32_t> type, texture;
+    std::vector<float> color, strength;
+    std::vector<double> exponent;
+    for (uint32_t i : ids) {
+        const FlatShader f = flattenShader(scene, *scene.shaders[i]);
+        type.push_back(f.type);
+        texture.push_back(f.texture);
+        color.insert(color.end(), f.color, f.color + 3);
+        exponent.push_back(f.exponent);
+        strength.push_back(f.strength);
+    }
+    return c2rt_scene_set_shaders(device, ids.size(), ids.data(), type.data(), color.data(), texture.data(), exponent.data(),
+                                  strength.data());
+}
+
+int setTextures(c2rt_scene* device, const Scene& scene, const std::vector<int>& textures) {
+    const std::vector<uint32_t> ids = editIds(textures, scene.textures.size(), "texture");
+    std::vector<float> colors;
+    std::vector<double> params;
+    for (uint32_t i : ids) {
+        const FlatTexture f = flattenTexture(*scene.textures[i]);
+        colors.insert(colors.end(), f.colors, f.colors + 18);
+        params.insert(params.end(), f.params, f.params + 6);
+    }
+    return c2rt_scene_set_textures(device, ids.size(), ids.data(), colors.data(), params.data());
+}
+
+int setLights(c2rt_scene* device, const Scene& scene, const std::vector<int>& lights) {
+    const std::vector<uint32_t> ids = editIds(lights, scene.lights.size(), "light");
+    std::vector<double> pos;
+    std::vector<float> color, power;
+    for (uint32_t i : ids) {
+        const FlatLight f = flattenLight(*scene.lights[i]);
+        pos.insert(pos.end(), f.pos, f.pos + 3);
+        color.insert(color.end(), f.color, f.color + 3);
+        power.push_back(f.power);
+    }
+    return c2rt_scene_set_lights(device, ids.size(), ids.data(), pos.data(), color.data(), power.data());
 }
 
 c2rt_scene_desc FlatScene::desc() const {

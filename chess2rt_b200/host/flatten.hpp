@@ -42,8 +42,41 @@ struct FlatNode {
     double transform[9], inverse[9], inverse_t[9], offset[3];
 };
 
+// One shader's entries of the shader arrays (c2rt_scene_desc, c2rt_scene_set_shaders)
+struct FlatShader {
+    int32_t type, texture;
+    float color[3];
+    double exponent;
+    float strength;
+};
+
+// One texture's entries of the texture arrays (c2rt_scene_desc, c2rt_scene_set_textures); a bitmap's texels are not among them
+struct FlatTexture {
+    int32_t type, width, height;
+    float colors[18];
+    double params[6];
+};
+
+// One light's entries of the light arrays (c2rt_scene_desc, c2rt_scene_set_lights)
+struct FlatLight {
+    double pos[3];
+    float color[3];
+    float power;
+};
+
 FlatScene flatten(const Scene& scene);                        // throws InvalidSceneException on dangling references
 FlatNode flattenNode(const Scene& scene, const Node& node);   // the same for one node
+FlatShader flattenShader(const Scene& scene, const Shader& shader);
+FlatTexture flattenTexture(const Texture& texture);
+FlatLight flattenLight(const Light& light);
+
+// c2rt_scene_set_node_shaders / _set_shaders / _set_textures / _set_lights of the listed entities of `scene` (indices into its
+// vectors), re-flattened through the routines above, on the uploaded scene `device`: the c2rt status.  Throws RTException on
+// an index out of range, before any call.
+int setNodeShaders(c2rt_scene* device, const Scene& scene, const std::vector<int>& nodes);
+int setShaders(c2rt_scene* device, const Scene& scene, const std::vector<int>& shaders);
+int setTextures(c2rt_scene* device, const Scene& scene, const std::vector<int>& textures);
+int setLights(c2rt_scene* device, const Scene& scene, const std::vector<int>& lights);
 c2rt_camera flattenCamera(const Camera& cam);                 // call after Camera.beginFrame
 c2rt_settings flattenSettings(const GlobalSettings& s, uint64_t rngSeed = 0, bool countRays = false);
 

@@ -140,6 +140,222 @@ int c2rt_host_scene_place_node(c2rt_host_scene* h, int node, const char* geometr
     }
 }
 
+}  // extern "C"
+
+namespace {
+
+int refuse(const std::string& message) {
+    g_host_err = message;
+    return C2RT_ERR_INVALID_ARG;
+}
+
+// An edit of the host scene, `edit` (which checks every argument before it changes anything), under the error handling of the
+// entry points: a library error is its c2rt status, any other exception C2RT_ERR_INVALID_ARG
+template <class F>
+int guarded(F edit) {
+    try {
+        return edit();
+    } catch (const BackendException& e) {
+        g_host_err = e.what();
+        return e.status;
+    } catch (const std::exception& e) {
+        g_host_err = e.what();
+        return C2RT_ERR_INVALID_ARG;
+    }
+}
+
+// The render_device scene follows an edit of entity `index` through `set` (flatten.hpp setShaders, ...); on a library error it
+// is dropped, and the next use re-creates it from the edited scene
+template <class Set>
+int followDevice(c2rt_host_scene* h, int index, Set set) {
+    if (!h->device) return 0;
+    int rc = set(h->device, *h->scene, {index});
+    if (rc != C2RT_OK) {
+        g_host_err = std::string("libc2rt: ") + c2rt_last_error();
+        c2rt_scene_destroy(h->device);
+        h->device = nullptr;
+    }
+    return rc;
+}
+
+template <class T>
+int indexIn(const std::vector<std::unique_ptr<T>>& v, const std::map<std::string, T*>& names, const char* name) {
+    auto it = name ? names.find(name) : names.end();
+    if (it == names.end()) return -1;
+    for (size_t i = 0; i < v.size(); i++)
+        if (v[i].get() == it->second) return (int)i;
+    return -1;
+}
+
+template <class T>
+const char* nameOf(const std::vector<std::unique_ptr<T>>& v, const std::map<std::string, T*>& names, int index) {
+    if (index < 0 || (size_t)index >= v.size()) return nullptr;
+    for (auto& named : names)
+        if (named.second == v[index].get()) return named.first.c_str();
+    return nullptr;
+}
+
+bool inRange(int i, size_t n, const char* what, const char* call) {
+    if (i >= 0 && (size_t)i < n) return true;
+    refuse(std::string(call) + ": " + what + " index " + std::to_string(i) + " out of range (" + std::to_string(n) + " " + what + "s)");
+    return false;
+}
+
+const Texture*& shaderTexture(Shader& s) {
+    if (auto* la = dynamic_cast<Lambert*>(&s)) return la->texture;
+    return dynamic_cast<Phong&>(s).texture;
+}
+
+}  // namespace
+
+extern "C" {
+
+// index of the entity of `section` ("nodes", "shaders", "textures" or "lights") the scene file names `name` (its place in
+// c2rt_scene_desc's arrays), -1 if there is none
+int c2rt_host_scene_index(const c2rt_host_scene* h, const char* section, const char* name) {
+    const Scene& s = *h->scene;
+    const std::string sec = section ? section : "";
+    if (sec == "nodes") return indexIn(s.nodes, s.namedEntities.nodes, name);
+    if (sec == "shaders") return indexIn(s.shaders, s.namedEntities.shaders, name);
+    if (sec == "textures") return indexIn(s.textures, s.namedEntities.textures, name);
+    if (sec == "lights") return indexIn(s.lights, s.namedEntities.lights, name);
+    return -1;
+}
+
+// the name the scene file gives entity `index` of `section` ("nodes", "shaders", "textures" or "lights"), NULL if it has none
+const char* c2rt_host_scene_name(const c2rt_host_scene* h, const char* section, int index) {
+    const Scene& s = *h->scene;
+    const std::string sec = section ? section : "";
+    if (sec == "nodes") return nameOf(s.nodes, s.namedEntities.nodes, index);
+    if (sec == "shaders") return nameOf(s.shaders, s.namedEntities.shaders, index);
+    if (sec == "textures") return nameOf(s.textures, s.namedEntities.textures, index);
+    if (sec == "lights") return nameOf(s.lights, s.namedEntities.lights, index);
+    return nullptr;
+}
+
+// As if node `node`'s `shader` key in the scene file named `shader`.  The flat description and both uploaded scenes (the
+// render_device one and the Renderer's) follow with c2rt_scene_set_node_shaders.  A bad index or name changes nothing.
+int c2rt_host_scene_set_node_shader(c2rt_host_scene* h, int node, const char* shader) {
+    return guarded([&]() -> int {
+        Scene& sc = *h->scene;
+        if (!inRange(node, sc.nodes.size(), "node", "set_node_shader")) return C2RT_ERR_INVALID_ARG;
+        auto it = shader ? sc.namedEntities.shaders.find(shader) : sc.namedEntities.shaders.end();
+        if (it == sc.namedEntities.shaders.end()) return refuse(std::string("set_node_shader: no shader named \"") + (shader ? shader : "") + "\"");
+        Node& nd = *sc.nodes[node];
+        nd.shader = it->second;
+        if (h->flat_valid) h->flat.node_shader[node] = flattenNode(sc, nd).shader;   // in place: handed-out pointers stay valid
+        sc.nodeShadersEdited({node});
+        return followDevice(h, node, setNodeShaders);
+    });
+}
+
+// As if shader `shader`'s entry in the scene file had been edited: `kind` ("Lambert" or "Phong"; NULL keeps the object)
+// replaces it with a fresh object of that kind, with that kind's defaults, under the same name and index; then the given keys
+// apply as the loader applies them (Phong's exponent and strength clamped).  texture: a texture name, "" for none, NULL keeps
+// it; exponent and strength are Phong keys.  The flat description and both uploaded scenes follow with c2rt_scene_set_shaders.
+// A bad index, kind, texture name or key changes nothing.
+int c2rt_host_scene_set_shader(c2rt_host_scene* h, int shader, const char* kind, const float* color, const char* texture,
+                               const double* exponent, const float* strength) {
+    return guarded([&]() -> int {
+        Scene& sc = *h->scene;
+        if (!inRange(shader, sc.shaders.size(), "shader", "set_shader")) return C2RT_ERR_INVALID_ARG;
+        const std::string k = kind ? kind : "";
+        if (kind && k != "Lambert" && k != "Phong") return refuse("set_shader: unknown shader kind \"" + k + "\"");
+        const Texture* tex = nullptr;
+        if (texture && texture[0]) {
+            auto it = sc.namedEntities.textures.find(texture);
+            if (it == sc.namedEntities.textures.end()) return refuse(std::string("set_shader: no texture named \"") + texture + "\"");
+            tex = it->second;
+        }
+        const bool phong = kind ? k == "Phong" : dynamic_cast<const Phong*>(sc.shaders[shader].get()) != nullptr;
+        if (!phong && (exponent || strength)) return refuse("set_shader: exponent and strength are Phong keys; the shader is a Lambert");
+        if (kind) {   // a fresh object in the same slot: the nodes and the name that referred to the old one refer to it
+            std::unique_ptr<Shader> fresh;
+            if (phong) fresh = std::make_unique<Phong>();
+            else fresh = std::make_unique<Lambert>();
+            const Shader* old = sc.shaders[shader].get();
+            for (auto& nd : sc.nodes)
+                if (nd->shader == old) nd->shader = fresh.get();
+            for (auto& named : sc.namedEntities.shaders)
+                if (named.second == old) named.second = fresh.get();
+            sc.shaders[shader] = std::move(fresh);
+        }
+        Shader& s = *sc.shaders[shader];
+        if (color) s.color = Color(color[0], color[1], color[2]);
+        if (texture) shaderTexture(s) = tex;
+        if (exponent) static_cast<Phong&>(s).exponent = Phong::clampExponent(*exponent);
+        if (strength) static_cast<Phong&>(s).strength = Phong::clampStrength(*strength);
+        if (h->flat_valid) {
+            const FlatShader f = flattenShader(sc, s);
+            FlatScene& fl = h->flat;
+            fl.shader_type[shader] = f.type;
+            fl.shader_texture[shader] = f.texture;
+            std::copy(f.color, f.color + 3, fl.shader_color.begin() + 3 * shader);
+            fl.shader_exponent[shader] = f.exponent;
+            fl.shader_strength[shader] = f.strength;
+        }
+        sc.shadersEdited({shader});
+        return followDevice(h, shader, setShaders);
+    });
+}
+
+// As if texture `texture`'s entry in the scene file had its given keys replaced (NULL: kept).  Checker: color1, color2 [3],
+// size; Procedure2: colorU, colorV [9] (three colours), freqU, freqV [3]; BitmapTexture: scaling.  A texture keeps its kind,
+// file and gamma.  The flat description and both uploaded scenes follow with c2rt_scene_set_textures.  A bad index or a key
+// of another kind changes nothing.
+int c2rt_host_scene_set_texture(c2rt_host_scene* h, int texture, const float* color1, const float* color2, const double* size,
+                                const float* colorU, const float* colorV, const double* freqU, const double* freqV,
+                                const float* scaling) {
+    return guarded([&]() -> int {
+        Scene& sc = *h->scene;
+        if (!inRange(texture, sc.textures.size(), "texture", "set_texture")) return C2RT_ERR_INVALID_ARG;
+        Texture& t = *sc.textures[texture];
+        auto* ch = dynamic_cast<Checker*>(&t);
+        auto* pr = dynamic_cast<Procedure2*>(&t);
+        auto* bm = dynamic_cast<BitmapTexture*>(&t);
+        if (!ch && (color1 || color2 || size)) return refuse("set_texture: color1, color2 and size are Checker keys");
+        if (!pr && (colorU || colorV || freqU || freqV)) return refuse("set_texture: colorU, colorV, freqU and freqV are Procedure2 keys");
+        if (!bm && scaling) return refuse("set_texture: scaling is a BitmapTexture key");
+        auto colors3 = [](const float* c) { return std::vector<Color>{Color(c[0], c[1], c[2]), Color(c[3], c[4], c[5]), Color(c[6], c[7], c[8])}; };
+        if (color1) ch->color1 = Color(color1[0], color1[1], color1[2]);
+        if (color2) ch->color2 = Color(color2[0], color2[1], color2[2]);
+        if (size) ch->size = *size;
+        if (colorU) pr->colorU = colors3(colorU);
+        if (colorV) pr->colorV = colors3(colorV);
+        if (freqU) pr->freqU.assign(freqU, freqU + 3);
+        if (freqV) pr->freqV.assign(freqV, freqV + 3);
+        if (scaling) bm->scaling = *scaling;
+        if (h->flat_valid) {
+            const FlatTexture f = flattenTexture(t);
+            std::copy(f.colors, f.colors + 18, h->flat.tex_colors.begin() + 18 * texture);
+            std::copy(f.params, f.params + 6, h->flat.tex_params.begin() + 6 * texture);
+        }
+        sc.texturesEdited({texture});
+        return followDevice(h, texture, setTextures);
+    });
+}
+
+// As if light `light`'s entry in the scene file had its given keys (pos [3], color [3], power) replaced (NULL: kept).  The flat
+// description and both uploaded scenes follow with c2rt_scene_set_lights.  A bad index changes nothing.
+int c2rt_host_scene_set_light(c2rt_host_scene* h, int light, const double* pos, const float* color, const float* power) {
+    return guarded([&]() -> int {
+        Scene& sc = *h->scene;
+        if (!inRange(light, sc.lights.size(), "light", "set_light")) return C2RT_ERR_INVALID_ARG;
+        auto& l = dynamic_cast<PointLight&>(*sc.lights[light]);
+        if (pos) l.pos = Vector(pos[0], pos[1], pos[2]);
+        if (color) l.lightColor = Color(color[0], color[1], color[2]);
+        if (power) l.lightPower = *power;
+        if (h->flat_valid) {
+            const FlatLight f = flattenLight(l);
+            std::copy(f.pos, f.pos + 3, h->flat.light_pos.begin() + 3 * light);
+            std::copy(f.color, f.color + 3, h->flat.light_color.begin() + 3 * light);
+            h->flat.light_power[light] = f.power;
+        }
+        sc.lightsEdited({light});
+        return followDevice(h, light, setLights);
+    });
+}
+
 // per-frame blocks: runs scene.beginFrame() first, like renderSceneAsync (renderer.d:31)
 void c2rt_host_frame_blocks(c2rt_host_scene* h, uint64_t seed, int count_rays, c2rt_camera* cam, c2rt_settings* set) {
     h->scene->beginFrame();

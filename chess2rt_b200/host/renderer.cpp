@@ -59,6 +59,26 @@ void Scene::nodesEdited(const std::vector<int>& indices) {
     }
 }
 
+namespace {
+
+// An edit of the uploaded scene (when there is one) through `set` (flatten.hpp setShaders, ...)
+template <class Set>
+void editDeviceScene(Scene& scene, const std::vector<int>& indices, Set set) {
+    if (!scene.deviceScene || indices.empty()) return;   // (no uploaded scene: the next frame flattens the whole scene)
+    int rc = set(static_cast<DeviceSceneHolder*>(scene.deviceScene.get())->handle, scene, indices);
+    if (rc != C2RT_OK) {
+        scene.invalidateDeviceScene();   // the next frame re-creates it from the edited scene
+        raise(rc);
+    }
+}
+
+}  // namespace
+
+void Scene::nodeShadersEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setNodeShaders); }
+void Scene::shadersEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setShaders); }
+void Scene::texturesEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setTextures); }
+void Scene::lightsEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setLights); }
+
 void Renderer::renderRT() {
     struct Done {  // renderer.d:87-91 end()
         std::atomic<bool>* flag;

@@ -219,6 +219,9 @@ struct Phong : Shader {
     double exponent = 16.0;
     float strength = 1.0f;
     Phong() { color = Color(1, 1, 1); }
+    // the ranges shader.d:263-280 clamps a loaded exponent and strength to
+    static double clampExponent(double e) { return e < 1e-6 ? 1e-6 : (e > 1e6 ? 1e6 : e); }
+    static float clampStrength(float s) { return s < 0.f ? 0.f : (s > 1e6f ? 1e6f : s); }
 };
 
 struct Light {
@@ -272,14 +275,23 @@ public:
 
     // New with the CUDA backend: the uploaded (flattened) scene, created on first render and
     // reused by every later frame; see renderer.cpp.  Call invalidateDeviceScene() after
-    // editing geometry / shaders / textures / lights, or adding / removing nodes (camera and
-    // settings are per-frame).  After changing only the geom or transform of existing nodes, call
-    // nodesEdited(indices) instead: it re-flattens those nodes and edits the uploaded scene in
-    // place (c2rt_scene_set_nodes) rather than re-creating it.  Throws BackendException on a
-    // library error, after dropping the uploaded scene.
+    // editing geometry or the environment, adding / removing entities, changing a texture's kind
+    // or a bitmap's pixels (camera and settings are per-frame).  After changing only existing
+    // entities' properties, call the matching hook instead: it re-flattens the listed entities
+    // (indices into the vectors above) and edits the uploaded scene in place rather than
+    // re-creating it.  nodesEdited: a node's geom or transform (c2rt_scene_set_nodes);
+    // nodeShadersEdited: a node's shader (c2rt_scene_set_node_shaders); shadersEdited: a shader's
+    // properties, or a shader replaced by another object in the same slot (c2rt_scene_set_shaders);
+    // texturesEdited: a texture's colours, size, frequencies or scaling (c2rt_scene_set_textures);
+    // lightsEdited: a light's pos, colour or power (c2rt_scene_set_lights).  They throw
+    // BackendException on a library error, after dropping the uploaded scene.
     mutable std::shared_ptr<void> deviceScene;
     void invalidateDeviceScene() { deviceScene.reset(); }
     void nodesEdited(const std::vector<int>& indices);
+    void nodeShadersEdited(const std::vector<int>& indices);
+    void shadersEdited(const std::vector<int>& indices);
+    void texturesEdited(const std::vector<int>& indices);
+    void lightsEdited(const std::vector<int>& indices);
 };
 
 // rt/scene_loader.d:20-41

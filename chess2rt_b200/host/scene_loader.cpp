@@ -217,9 +217,9 @@ std::unique_ptr<Shader> makeShader(const DscNode& n, SceneLoadContext& c) {
         auto s = std::make_unique<Phong>();
         c.set(s->color, n, "color");
         c.set(s->exponent, n, "exponent");  // shader.d:263-280
-        s->exponent = s->exponent < 1e-6 ? 1e-6 : (s->exponent > 1e6 ? 1e6 : s->exponent);
+        s->exponent = Phong::clampExponent(s->exponent);
         c.set(s->strength, n, "strength");
-        s->strength = s->strength < 0.f ? 0.f : (s->strength > 1e6f ? 1e6f : s->strength);
+        s->strength = Phong::clampStrength(s->strength);
         s->texture = optionalTexture(n, c, "texture");
         return s;
     }

@@ -225,8 +225,8 @@ void c2rt_scene_destroy(c2rt_scene* scene);
  * without re-creating the scene.  Entry i edits node nodes[i]; the arrays have the layout of c2rt_scene_desc's node arrays
  * ([n], [n*9], [n*9], [n*9], [n*3]).  geom == NULL keeps every edited node's geometry; the four transform arrays are given
  * together, or all NULL to keep every edited node's transform; at least one of the two must be given.  Entries apply in array
- * order, so a later entry for the same node wins.  Shaders, textures, lights, the environment, the node count and the node
- * order stay as created.
+ * order, so a later entry for the same node wins.  Node shaders, shaders, textures and lights have edits of their own (below);
+ * the environment, the node count and the node order stay as created.
  * Afterwards every call on the scene (frames, _device frames, hit frames, the pixel pick, ray queries, visibility, shaded rays)
  * gives the same result, bit for bit, as on a scene c2rt_scene_create built from the edited description, on every device.
  * Errors: a null scene, nodes == NULL with n > 0, a node index >= n_nodes, a geometry index outside 0..n_geoms-1 or a partial
@@ -237,6 +237,28 @@ void c2rt_scene_destroy(c2rt_scene* scene);
  * device, must be issued outside any CUDA stream capture, and a graph captured before the edit must not be replayed after it. */
 int c2rt_scene_set_nodes(c2rt_scene* scene, size_t n, const uint32_t* nodes, const int32_t* geom,
                          const double* transform, const double* inverse, const double* inverse_t, const double* offset);
+
+/* Shading and light edits in place: point nodes at other shaders (highlight a piece and back), replace shaders (colour, kind,
+ * Phong exponent / strength, texture), textures (Checker colours and size, Procedure2 colours and frequencies, a bitmap's
+ * scaling) and lights (position, colour, power) without re-creating the scene.  Entry i replaces the whole entry the description
+ * gave for index nodes[i] / shaders[i] / textures[i] / lights[i]; every index is a description index (a position in the
+ * c2rt_scene_desc arrays the scene was created from), and the arrays have the layout of the matching c2rt_scene_desc arrays for
+ * n entries.  A shader's texture index < 0 means none.  A texture keeps its kind, and a bitmap its texels and size: a bitmap
+ * entry reads params[0] (scaling) only, a Checker or Procedure2 entry all of colors [18] and params [6].  Values
+ * c2rt_scene_create accepts are accepted here (non-finite colours, zero power).  Entries apply in array order, so a later
+ * entry for the same index wins.  The environment and the counts and kinds stay as created.
+ * Afterwards every call on the scene gives the same result, bit for bit, as on a scene c2rt_scene_create built from the
+ * edited description, on every device; a GI frame's refusal of Phong-shaded nodes follows the edited shaders.
+ * Errors: a null scene, a null array with n > 0, an index out of range, a node's shader outside 0..n_shaders-1, an unknown
+ * shader type or a shader texture >= n_textures is C2RT_ERR_INVALID_ARG.  Every check runs before anything changes: on any of
+ * these errors the scene is unchanged.  n == 0 is a no-op.  A C2RT_ERR_CUDA leaves the scene fit only for c2rt_scene_destroy.
+ * Blocking, locking and stream capture: as c2rt_scene_set_nodes. */
+int c2rt_scene_set_node_shaders(c2rt_scene* scene, size_t n, const uint32_t* nodes, const int32_t* shader);
+int c2rt_scene_set_shaders(c2rt_scene* scene, size_t n, const uint32_t* shaders, const int32_t* type, const float* color,
+                           const int32_t* texture, const double* exponent, const float* strength);
+int c2rt_scene_set_textures(c2rt_scene* scene, size_t n, const uint32_t* textures, const float* colors, const double* params);
+int c2rt_scene_set_lights(c2rt_scene* scene, size_t n, const uint32_t* lights, const double* pos, const float* color,
+                          const float* power);
 
 /* Replaces Renderer.renderRT (renderer.d:83-189): blocking, one frame into caller-owned HOST
  * memory.  rgb: frame_width*frame_height*3 floats laid out as Image!Color.pixels
@@ -261,7 +283,7 @@ int c2rt_cancel(void);
  * A device holds ONE scene block at a time: rendering a different scene than the previous call on this device first waits
  * for all work on the device and re-uploads the block, so (i) frames of two scenes never overlap on one device and
  * (ii) the first frame of a scene on a device must be issued outside any CUDA stream capture (later ones may be captured).
- * The same holds for the first frame after a c2rt_scene_set_nodes: the edit re-uploads the block, and a frame captured into a
+ * The same holds for the first frame after a c2rt_scene_set_* edit: the edit re-uploads the block, and a frame captured into a
  * graph before the edit is not valid after it. */
 int c2rt_render_device(c2rt_scene* scene, const c2rt_camera* camera, const c2rt_settings* settings,
                        const c2rt_band* band, float* d_rgb, uint32_t* d_argb, void* stream, c2rt_stats* stats);
