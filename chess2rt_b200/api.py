@@ -163,7 +163,6 @@ host_lib.c2rt_host_scene_override.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_
 host_lib.c2rt_host_scene_override.restype = None
 host_lib.c2rt_host_scene_desc.argtypes = [C.c_void_p]
 host_lib.c2rt_host_scene_desc.restype = C.POINTER(SceneDesc)
-host_lib.c2rt_host_scene_node_index.argtypes = [C.c_void_p, C.c_char_p]
 host_lib.c2rt_host_scene_place_node.argtypes = [C.c_void_p, C.c_int, C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p]
 host_lib.c2rt_host_scene_index.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p]
 host_lib.c2rt_host_scene_name.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
@@ -283,10 +282,7 @@ class HostScene:
 
     def node_index(self, name):
         """The index of the node the scene file names `name` (its place in the description's node arrays)."""
-        i = host_lib.c2rt_host_scene_node_index(self._h, str(name).encode())
-        if i < 0:
-            raise KeyError(f"no node named {name!r}")
-        return i
+        return self.index("nodes", str(name))
 
     def place_node(self, node, geometry=None, scale=None, rotate=None, translate=None):
         """As if the node's entry in the scene file had been edited: `geometry` (a geometry name; None keeps it) and the keys

@@ -1,5 +1,6 @@
 #include "flatten.hpp"
 
+#include <algorithm>
 #include <cstring>
 #include <string>
 
@@ -18,10 +19,71 @@ void putMatrix(double dst[9], const Matrix& m) {
         for (int c = 0; c < 3; c++) dst[3 * r + c] = m.c[r][c];
 }
 
+// entry i of an array whose entries are N values each
+template <class T, size_t N>
+void putEntry(std::vector<T>& v, size_t i, const T (&entry)[N]) {
+    std::copy(entry, entry + N, v.begin() + N * i);
+}
+
 }  // namespace
+
+void FlatScene::resize(size_t nodes, size_t shaders, size_t textures, size_t lights) {
+    node_geom.resize(nodes);
+    node_shader.resize(nodes);
+    node_transform.resize(9 * nodes);
+    node_inverse.resize(9 * nodes);
+    node_inverse_t.resize(9 * nodes);
+    node_offset.resize(3 * nodes);
+    shader_type.resize(shaders);
+    shader_texture.resize(shaders);
+    shader_color.resize(3 * shaders);
+    shader_exponent.resize(shaders);
+    shader_strength.resize(shaders);
+    tex_type.resize(textures);
+    tex_width.resize(textures);
+    tex_height.resize(textures);
+    tex_texel_offset.resize(textures);
+    tex_colors.resize(18 * textures);
+    tex_params.resize(6 * textures);
+    light_pos.resize(3 * lights);
+    light_color.resize(3 * lights);
+    light_power.resize(lights);
+}
+
+void FlatScene::put(size_t i, const FlatNode& n) {
+    node_geom[i] = n.geom;
+    node_shader[i] = n.shader;
+    putEntry(node_transform, i, n.transform);
+    putEntry(node_inverse, i, n.inverse);
+    putEntry(node_inverse_t, i, n.inverse_t);
+    putEntry(node_offset, i, n.offset);
+}
+
+void FlatScene::put(size_t i, const FlatShader& s) {
+    shader_type[i] = s.type;
+    shader_texture[i] = s.texture;
+    putEntry(shader_color, i, s.color);
+    shader_exponent[i] = s.exponent;
+    shader_strength[i] = s.strength;
+}
+
+void FlatScene::put(size_t i, const FlatTexture& t) {
+    tex_type[i] = t.type;
+    tex_width[i] = t.width;
+    tex_height[i] = t.height;
+    putEntry(tex_colors, i, t.colors);
+    putEntry(tex_params, i, t.params);
+}
+
+void FlatScene::put(size_t i, const FlatLight& l) {
+    putEntry(light_pos, i, l.pos);
+    putEntry(light_color, i, l.color);
+    light_power[i] = l.power;
+}
 
 FlatScene flatten(const Scene& scene) {
     FlatScene f;
+    f.resize(scene.nodes.size(), scene.shaders.size(), scene.textures.size(), scene.lights.size());
 
     // geometries, in declaration order (CSG children are always earlier: geometry.d:343-347)
     for (size_t i = 0; i < scene.geometries.size(); i++) {
@@ -52,43 +114,22 @@ FlatScene flatten(const Scene& scene) {
         f.geom_params.insert(f.geom_params.end(), p, p + 4);
     }
 
-    // textures
-    for (auto& t : scene.textures) {
-        const FlatTexture ft = flattenTexture(*t);
-        uint64_t off = 0;
-        if (auto* bm = dynamic_cast<const BitmapTexture*>(t.get())) {
-            off = f.texels.size() / 3;
+    // textures; a bitmap's texels are appended to `texels`
+    for (size_t i = 0; i < scene.textures.size(); i++) {
+        const Texture* t = scene.textures[i].get();
+        f.put(i, flattenTexture(*t));
+        if (auto* bm = dynamic_cast<const BitmapTexture*>(t)) {
+            f.tex_texel_offset[i] = f.texels.size() / 3;
             for (const Color& c : bm->bmp.data.pixels) {
                 f.texels.push_back(c.r);
                 f.texels.push_back(c.g);
                 f.texels.push_back(c.b);
             }
         }
-        f.tex_type.push_back(ft.type);
-        f.tex_width.push_back(ft.width);
-        f.tex_height.push_back(ft.height);
-        f.tex_texel_offset.push_back(off);
-        f.tex_colors.insert(f.tex_colors.end(), ft.colors, ft.colors + 18);
-        f.tex_params.insert(f.tex_params.end(), ft.params, ft.params + 6);
     }
 
-    // shaders
-    for (auto& s : scene.shaders) {
-        const FlatShader fs = flattenShader(scene, *s);
-        f.shader_type.push_back(fs.type);
-        f.shader_texture.push_back(fs.texture);
-        f.shader_color.insert(f.shader_color.end(), fs.color, fs.color + 3);
-        f.shader_exponent.push_back(fs.exponent);
-        f.shader_strength.push_back(fs.strength);
-    }
-
-    // lights
-    for (auto& l : scene.lights) {
-        const FlatLight fl = flattenLight(*l);
-        f.light_pos.insert(f.light_pos.end(), fl.pos, fl.pos + 3);
-        f.light_color.insert(f.light_color.end(), fl.color, fl.color + 3);
-        f.light_power.push_back(fl.power);
-    }
+    for (size_t i = 0; i < scene.shaders.size(); i++) f.put(i, flattenShader(scene, *scene.shaders[i]));
+    for (size_t i = 0; i < scene.lights.size(); i++) f.put(i, flattenLight(*scene.lights[i]));
 
     // environment (cubemap extension: rt.hpp Environment): the six faces follow the bitmap textures' texels
     if (scene.environment.cubemap) {
@@ -106,16 +147,7 @@ FlatScene flatten(const Scene& scene) {
         }
     }
 
-    // nodes
-    for (auto& n : scene.nodes) {
-        const FlatNode fn = flattenNode(scene, *n);
-        f.node_geom.push_back(fn.geom);
-        f.node_shader.push_back(fn.shader);
-        f.node_transform.insert(f.node_transform.end(), fn.transform, fn.transform + 9);
-        f.node_inverse.insert(f.node_inverse.end(), fn.inverse, fn.inverse + 9);
-        f.node_inverse_t.insert(f.node_inverse_t.end(), fn.inverse_t, fn.inverse_t + 9);
-        f.node_offset.insert(f.node_offset.end(), fn.offset, fn.offset + 3);
-    }
+    for (size_t i = 0; i < scene.nodes.size(); i++) f.put(i, flattenNode(scene, *scene.nodes[i]));
     return f;
 }
 
@@ -206,53 +238,46 @@ std::vector<uint32_t> editIds(const std::vector<int>& indices, size_t count, con
 
 }  // namespace
 
+int setNodes(c2rt_scene* device, const Scene& scene, const std::vector<int>& nodes) {
+    const std::vector<uint32_t> ids = editIds(nodes, scene.nodes.size(), "node");
+    FlatScene f;
+    f.resize(ids.size(), 0, 0, 0);
+    for (size_t k = 0; k < ids.size(); k++) f.put(k, flattenNode(scene, *scene.nodes[ids[k]]));
+    return c2rt_scene_set_nodes(device, ids.size(), ids.data(), f.node_geom.data(), f.node_transform.data(), f.node_inverse.data(),
+                                f.node_inverse_t.data(), f.node_offset.data());
+}
+
 int setNodeShaders(c2rt_scene* device, const Scene& scene, const std::vector<int>& nodes) {
     const std::vector<uint32_t> ids = editIds(nodes, scene.nodes.size(), "node");
-    std::vector<int32_t> shader;
-    for (uint32_t i : ids) shader.push_back(flattenNode(scene, *scene.nodes[i]).shader);
-    return c2rt_scene_set_node_shaders(device, ids.size(), ids.data(), shader.data());
+    FlatScene f;
+    f.resize(ids.size(), 0, 0, 0);
+    for (size_t k = 0; k < ids.size(); k++) f.put(k, flattenNode(scene, *scene.nodes[ids[k]]));
+    return c2rt_scene_set_node_shaders(device, ids.size(), ids.data(), f.node_shader.data());
 }
 
 int setShaders(c2rt_scene* device, const Scene& scene, const std::vector<int>& shaders) {
     const std::vector<uint32_t> ids = editIds(shaders, scene.shaders.size(), "shader");
-    std::vector<int32_t> type, texture;
-    std::vector<float> color, strength;
-    std::vector<double> exponent;
-    for (uint32_t i : ids) {
-        const FlatShader f = flattenShader(scene, *scene.shaders[i]);
-        type.push_back(f.type);
-        texture.push_back(f.texture);
-        color.insert(color.end(), f.color, f.color + 3);
-        exponent.push_back(f.exponent);
-        strength.push_back(f.strength);
-    }
-    return c2rt_scene_set_shaders(device, ids.size(), ids.data(), type.data(), color.data(), texture.data(), exponent.data(),
-                                  strength.data());
+    FlatScene f;
+    f.resize(0, ids.size(), 0, 0);
+    for (size_t k = 0; k < ids.size(); k++) f.put(k, flattenShader(scene, *scene.shaders[ids[k]]));
+    return c2rt_scene_set_shaders(device, ids.size(), ids.data(), f.shader_type.data(), f.shader_color.data(), f.shader_texture.data(),
+                                  f.shader_exponent.data(), f.shader_strength.data());
 }
 
 int setTextures(c2rt_scene* device, const Scene& scene, const std::vector<int>& textures) {
     const std::vector<uint32_t> ids = editIds(textures, scene.textures.size(), "texture");
-    std::vector<float> colors;
-    std::vector<double> params;
-    for (uint32_t i : ids) {
-        const FlatTexture f = flattenTexture(*scene.textures[i]);
-        colors.insert(colors.end(), f.colors, f.colors + 18);
-        params.insert(params.end(), f.params, f.params + 6);
-    }
-    return c2rt_scene_set_textures(device, ids.size(), ids.data(), colors.data(), params.data());
+    FlatScene f;
+    f.resize(0, 0, ids.size(), 0);
+    for (size_t k = 0; k < ids.size(); k++) f.put(k, flattenTexture(*scene.textures[ids[k]]));
+    return c2rt_scene_set_textures(device, ids.size(), ids.data(), f.tex_colors.data(), f.tex_params.data());
 }
 
 int setLights(c2rt_scene* device, const Scene& scene, const std::vector<int>& lights) {
     const std::vector<uint32_t> ids = editIds(lights, scene.lights.size(), "light");
-    std::vector<double> pos;
-    std::vector<float> color, power;
-    for (uint32_t i : ids) {
-        const FlatLight f = flattenLight(*scene.lights[i]);
-        pos.insert(pos.end(), f.pos, f.pos + 3);
-        color.insert(color.end(), f.color, f.color + 3);
-        power.push_back(f.power);
-    }
-    return c2rt_scene_set_lights(device, ids.size(), ids.data(), pos.data(), color.data(), power.data());
+    FlatScene f;
+    f.resize(0, 0, 0, ids.size());
+    for (size_t k = 0; k < ids.size(); k++) f.put(k, flattenLight(*scene.lights[ids[k]]));
+    return c2rt_scene_set_lights(device, ids.size(), ids.data(), f.light_pos.data(), f.light_color.data(), f.light_power.data());
 }
 
 c2rt_scene_desc FlatScene::desc() const {

@@ -13,28 +13,6 @@
 
 namespace rt {
 
-struct FlatScene {
-    std::vector<int32_t> node_geom, node_shader;
-    std::vector<double> node_transform, node_inverse, node_inverse_t, node_offset;
-    std::vector<int32_t> geom_type, geom_left, geom_right;
-    std::vector<double> geom_params;
-    std::vector<int32_t> shader_type, shader_texture;
-    std::vector<float> shader_color, shader_strength;
-    std::vector<double> shader_exponent;
-    std::vector<int32_t> tex_type, tex_width, tex_height;
-    std::vector<float> tex_colors;
-    std::vector<double> tex_params;
-    std::vector<uint64_t> tex_texel_offset;
-    std::vector<float> texels;
-    std::vector<double> light_pos;
-    std::vector<float> light_color, light_power;
-    int32_t env_type = C2RT_ENV_BLACK;
-    int32_t env_face_width[6] = {0}, env_face_height[6] = {0};
-    uint64_t env_face_texel_offset[6] = {0};
-
-    c2rt_scene_desc desc() const;  // borrows the vectors above
-};
-
 // One node's entries of the node arrays (c2rt_scene_desc, c2rt_scene_set_nodes): geometry and shader index, the three
 // matrices row-major, the offset
 struct FlatNode {
@@ -64,15 +42,45 @@ struct FlatLight {
     float power;
 };
 
+struct FlatScene {
+    std::vector<int32_t> node_geom, node_shader;
+    std::vector<double> node_transform, node_inverse, node_inverse_t, node_offset;
+    std::vector<int32_t> geom_type, geom_left, geom_right;
+    std::vector<double> geom_params;
+    std::vector<int32_t> shader_type, shader_texture;
+    std::vector<float> shader_color, shader_strength;
+    std::vector<double> shader_exponent;
+    std::vector<int32_t> tex_type, tex_width, tex_height;
+    std::vector<float> tex_colors;
+    std::vector<double> tex_params;
+    std::vector<uint64_t> tex_texel_offset;
+    std::vector<float> texels;
+    std::vector<double> light_pos;
+    std::vector<float> light_color, light_power;
+    int32_t env_type = C2RT_ENV_BLACK;
+    int32_t env_face_width[6] = {0}, env_face_height[6] = {0};
+    uint64_t env_face_texel_offset[6] = {0};
+
+    // Sizes the node, shader, texture and light arrays for that many entries of each (new entries are zero)
+    void resize(size_t nodes, size_t shaders, size_t textures, size_t lights);
+    // Entry i of one kind's arrays; the texture writer leaves tex_texel_offset alone
+    void put(size_t i, const FlatNode& node);
+    void put(size_t i, const FlatShader& shader);
+    void put(size_t i, const FlatTexture& texture);
+    void put(size_t i, const FlatLight& light);
+    c2rt_scene_desc desc() const;  // borrows the vectors above
+};
+
 FlatScene flatten(const Scene& scene);                        // throws InvalidSceneException on dangling references
 FlatNode flattenNode(const Scene& scene, const Node& node);   // the same for one node
 FlatShader flattenShader(const Scene& scene, const Shader& shader);
 FlatTexture flattenTexture(const Texture& texture);
 FlatLight flattenLight(const Light& light);
 
-// c2rt_scene_set_node_shaders / _set_shaders / _set_textures / _set_lights of the listed entities of `scene` (indices into its
-// vectors), re-flattened through the routines above, on the uploaded scene `device`: the c2rt status.  Throws RTException on
-// an index out of range, before any call.
+// c2rt_scene_set_nodes / _set_node_shaders / _set_shaders / _set_textures / _set_lights of the listed entities of `scene`
+// (indices into its vectors), re-flattened through the routines above, on the uploaded scene `device`: the c2rt status.
+// setNodes sets each node's geometry and transform.  Throws RTException on an index out of range, before any call.
+int setNodes(c2rt_scene* device, const Scene& scene, const std::vector<int>& nodes);
 int setNodeShaders(c2rt_scene* device, const Scene& scene, const std::vector<int>& nodes);
 int setShaders(c2rt_scene* device, const Scene& scene, const std::vector<int>& shaders);
 int setTextures(c2rt_scene* device, const Scene& scene, const std::vector<int>& textures);

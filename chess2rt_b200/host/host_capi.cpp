@@ -1,7 +1,6 @@
 // C entry points over the C++ host mirror, for the Python harness (tests/, bench.py) — the same
 // calls the headless executable makes: load a scene file with the reference-compatible loader,
 // flatten it, render through libc2rt.so.  No torch types, no CPU rendering.
-#include <algorithm>
 #include <cstring>
 #include <string>
 
@@ -15,7 +14,6 @@ struct c2rt_host_scene {
     FlatScene flat;          // kept alive: c2rt_host_scene_desc() hands out pointers into it
     c2rt_scene_desc desc;
     bool flat_valid = false;
-    c2rt_scene* device = nullptr;  // for the render_device path
 };
 
 static thread_local std::string g_host_err;
@@ -35,11 +33,7 @@ c2rt_host_scene* c2rt_host_scene_load(const char* path) {
     }
 }
 
-void c2rt_host_scene_free(c2rt_host_scene* h) {
-    if (!h) return;
-    if (h->device) c2rt_scene_destroy(h->device);
-    delete h;
-}
+void c2rt_host_scene_free(c2rt_host_scene* h) { delete h; }
 
 // as if the scene file had been edited: settings.frameWidth/Height + camera.setFrameSize (camera.d:254)
 void c2rt_host_scene_set_frame_size(c2rt_host_scene* h, uint32_t w, uint32_t hgt) {
@@ -73,70 +67,14 @@ const c2rt_scene_desc* c2rt_host_scene_desc(c2rt_host_scene* h) {
         return nullptr;
     }
 }
-// index of the node the scene file names `name` (its place in c2rt_scene_desc's node arrays), -1 if there is none
-int c2rt_host_scene_node_index(const c2rt_host_scene* h, const char* name) {
-    const Scene& s = *h->scene;
-    auto it = name ? s.namedEntities.nodes.find(name) : s.namedEntities.nodes.end();
-    if (it == s.namedEntities.nodes.end()) return -1;
-    for (size_t i = 0; i < s.nodes.size(); i++)
-        if (s.nodes[i].get() == it->second) return (int)i;
-    return -1;
-}
-
-// As if the scene file's entry of node `node` had been edited: its geometry becomes the one named `geometry` (NULL: kept), its
-// Transform is reset and the given keys are applied the way the loader applies them (makeNode: scale, then rotate through
-// scale as the reference does, then translate; NULL: key absent).  The flat description and both uploaded scenes (the
-// render_device one and the Renderer's) follow with c2rt_scene_set_nodes.  A bad node index or geometry name changes nothing.
-int c2rt_host_scene_place_node(c2rt_host_scene* h, int node, const char* geometry, const double* scale, const double* rotate,
-                               const double* translate) {
+// The uploaded scene (Scene::deviceScene) every c2rt_host_* call renders through, created on first use under the current
+// c2rt_init; the edits below change it in place.  NULL on an error.
+c2rt_scene* c2rt_host_device_scene(c2rt_host_scene* h) {
     try {
-        Scene& sc = *h->scene;
-        if (node < 0 || (size_t)node >= sc.nodes.size()) {
-            g_host_err = "place_node: node index " + std::to_string(node) + " out of range (" + std::to_string(sc.nodes.size()) + " nodes)";
-            return C2RT_ERR_INVALID_ARG;
-        }
-        const Geometry* g = nullptr;
-        if (geometry) {
-            auto it = sc.namedEntities.geometries.find(geometry);
-            if (it == sc.namedEntities.geometries.end()) {
-                g_host_err = std::string("place_node: no geometry named \"") + geometry + "\"";
-                return C2RT_ERR_INVALID_ARG;
-            }
-            g = it->second;
-        }
-        Node& nd = *sc.nodes[node];
-        if (g) nd.geom = g;
-        nd.transform.reset();
-        if (scale) nd.transform.scale(scale[0], scale[1], scale[2]);
-        if (rotate) nd.transform.scale(rotate[0], rotate[1], rotate[2]);   // sic: scene_loader.cpp makeNode, node.d:89-90
-        if (translate) nd.transform.translate(Vector(translate[0], translate[1], translate[2]));
-        const FlatNode f = flattenNode(sc, nd);
-        if (h->flat_valid) {   // in place: the pointers c2rt_host_scene_desc handed out stay valid
-            FlatScene& fl = h->flat;
-            fl.node_geom[node] = f.geom;
-            std::copy(f.transform, f.transform + 9, fl.node_transform.begin() + 9 * node);
-            std::copy(f.inverse, f.inverse + 9, fl.node_inverse.begin() + 9 * node);
-            std::copy(f.inverse_t, f.inverse_t + 9, fl.node_inverse_t.begin() + 9 * node);
-            std::copy(f.offset, f.offset + 3, fl.node_offset.begin() + 3 * node);
-        }
-        sc.nodesEdited({node});
-        if (h->device) {
-            const uint32_t id = (uint32_t)node;
-            int rc = c2rt_scene_set_nodes(h->device, 1, &id, &f.geom, f.transform, f.inverse, f.inverse_t, f.offset);
-            if (rc != C2RT_OK) {
-                g_host_err = std::string("libc2rt: ") + c2rt_last_error();
-                c2rt_scene_destroy(h->device);   // the next use re-creates it from the edited scene
-                h->device = nullptr;
-                return rc;
-            }
-        }
-        return 0;
-    } catch (const BackendException& e) {
-        g_host_err = e.what();
-        return e.status;
+        return uploadedScene(*h->scene);
     } catch (const std::exception& e) {
         g_host_err = e.what();
-        return C2RT_ERR_INVALID_ARG;
+        return nullptr;
     }
 }
 
@@ -150,7 +88,9 @@ int refuse(const std::string& message) {
 }
 
 // An edit of the host scene, `edit` (which checks every argument before it changes anything), under the error handling of the
-// entry points: a library error is its c2rt status, any other exception C2RT_ERR_INVALID_ARG
+// entry points: a library error is its c2rt status, any other exception C2RT_ERR_INVALID_ARG.  An edit ends with its
+// Scene::*Edited hook, which edits the uploaded scene in place or, on a library error, drops it (the next use re-creates it
+// from the edited scene) and throws.
 template <class F>
 int guarded(F edit) {
     try {
@@ -164,17 +104,14 @@ int guarded(F edit) {
     }
 }
 
-// The render_device scene follows an edit of entity `index` through `set` (flatten.hpp setShaders, ...); on a library error it
-// is dropped, and the next use re-creates it from the edited scene
-template <class Set>
-int followDevice(c2rt_host_scene* h, int index, Set set) {
-    if (!h->device) return 0;
-    int rc = set(h->device, *h->scene, {index});
-    if (rc != C2RT_OK) {
-        g_host_err = std::string("libc2rt: ") + c2rt_last_error();
-        c2rt_scene_destroy(h->device);
-        h->device = nullptr;
-    }
+// `call` (a libc2rt call) on the uploaded scene: C2RT_ERR_CUDA when there is none, else the call's status, with the library's
+// message for any status but C2RT_OK (C2RT_CANCELLED included)
+template <class F>
+int onDevice(c2rt_host_scene* h, F call) {
+    c2rt_scene* dev = c2rt_host_device_scene(h);
+    if (!dev) return C2RT_ERR_CUDA;
+    int rc = call(dev);
+    if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
     return rc;
 }
 
@@ -233,8 +170,35 @@ const char* c2rt_host_scene_name(const c2rt_host_scene* h, const char* section, 
     return nullptr;
 }
 
-// As if node `node`'s `shader` key in the scene file named `shader`.  The flat description and both uploaded scenes (the
-// render_device one and the Renderer's) follow with c2rt_scene_set_node_shaders.  A bad index or name changes nothing.
+// As if the scene file's entry of node `node` had been edited: its geometry becomes the one named `geometry` (NULL: kept), its
+// Transform is reset and the given keys are applied the way the loader applies them (makeNode: scale, then rotate through
+// scale as the reference does, then translate; NULL: key absent).  The flat description and the uploaded scene follow
+// (Scene::nodesEdited).  A bad node index or geometry name changes nothing.
+int c2rt_host_scene_place_node(c2rt_host_scene* h, int node, const char* geometry, const double* scale, const double* rotate,
+                               const double* translate) {
+    return guarded([&]() -> int {
+        Scene& sc = *h->scene;
+        if (!inRange(node, sc.nodes.size(), "node", "place_node")) return C2RT_ERR_INVALID_ARG;
+        const Geometry* g = nullptr;
+        if (geometry) {
+            auto it = sc.namedEntities.geometries.find(geometry);
+            if (it == sc.namedEntities.geometries.end()) return refuse(std::string("place_node: no geometry named \"") + geometry + "\"");
+            g = it->second;
+        }
+        Node& nd = *sc.nodes[node];
+        if (g) nd.geom = g;
+        nd.transform.reset();
+        if (scale) nd.transform.scale(scale[0], scale[1], scale[2]);
+        if (rotate) nd.transform.scale(rotate[0], rotate[1], rotate[2]);   // sic: scene_loader.cpp makeNode, node.d:89-90
+        if (translate) nd.transform.translate(Vector(translate[0], translate[1], translate[2]));
+        if (h->flat_valid) h->flat.put(node, flattenNode(sc, nd));   // in place: handed-out pointers stay valid
+        sc.nodesEdited({node});
+        return 0;
+    });
+}
+
+// As if node `node`'s `shader` key in the scene file named `shader`.  The flat description and the uploaded scene follow
+// (Scene::nodeShadersEdited).  A bad index or name changes nothing.
 int c2rt_host_scene_set_node_shader(c2rt_host_scene* h, int node, const char* shader) {
     return guarded([&]() -> int {
         Scene& sc = *h->scene;
@@ -243,17 +207,17 @@ int c2rt_host_scene_set_node_shader(c2rt_host_scene* h, int node, const char* sh
         if (it == sc.namedEntities.shaders.end()) return refuse(std::string("set_node_shader: no shader named \"") + (shader ? shader : "") + "\"");
         Node& nd = *sc.nodes[node];
         nd.shader = it->second;
-        if (h->flat_valid) h->flat.node_shader[node] = flattenNode(sc, nd).shader;   // in place: handed-out pointers stay valid
+        if (h->flat_valid) h->flat.put(node, flattenNode(sc, nd));
         sc.nodeShadersEdited({node});
-        return followDevice(h, node, setNodeShaders);
+        return 0;
     });
 }
 
 // As if shader `shader`'s entry in the scene file had been edited: `kind` ("Lambert" or "Phong"; NULL keeps the object)
 // replaces it with a fresh object of that kind, with that kind's defaults, under the same name and index; then the given keys
 // apply as the loader applies them (Phong's exponent and strength clamped).  texture: a texture name, "" for none, NULL keeps
-// it; exponent and strength are Phong keys.  The flat description and both uploaded scenes follow with c2rt_scene_set_shaders.
-// A bad index, kind, texture name or key changes nothing.
+// it; exponent and strength are Phong keys.  The flat description and the uploaded scene follow (Scene::shadersEdited).  A bad
+// index, kind, texture name or key changes nothing.
 int c2rt_host_scene_set_shader(c2rt_host_scene* h, int shader, const char* kind, const float* color, const char* texture,
                                const double* exponent, const float* strength) {
     return guarded([&]() -> int {
@@ -285,24 +249,16 @@ int c2rt_host_scene_set_shader(c2rt_host_scene* h, int shader, const char* kind,
         if (texture) shaderTexture(s) = tex;
         if (exponent) static_cast<Phong&>(s).exponent = Phong::clampExponent(*exponent);
         if (strength) static_cast<Phong&>(s).strength = Phong::clampStrength(*strength);
-        if (h->flat_valid) {
-            const FlatShader f = flattenShader(sc, s);
-            FlatScene& fl = h->flat;
-            fl.shader_type[shader] = f.type;
-            fl.shader_texture[shader] = f.texture;
-            std::copy(f.color, f.color + 3, fl.shader_color.begin() + 3 * shader);
-            fl.shader_exponent[shader] = f.exponent;
-            fl.shader_strength[shader] = f.strength;
-        }
+        if (h->flat_valid) h->flat.put(shader, flattenShader(sc, s));
         sc.shadersEdited({shader});
-        return followDevice(h, shader, setShaders);
+        return 0;
     });
 }
 
 // As if texture `texture`'s entry in the scene file had its given keys replaced (NULL: kept).  Checker: color1, color2 [3],
 // size; Procedure2: colorU, colorV [9] (three colours), freqU, freqV [3]; BitmapTexture: scaling.  A texture keeps its kind,
-// file and gamma.  The flat description and both uploaded scenes follow with c2rt_scene_set_textures.  A bad index or a key
-// of another kind changes nothing.
+// file and gamma.  The flat description and the uploaded scene follow (Scene::texturesEdited).  A bad index
+// or a key of another kind changes nothing.
 int c2rt_host_scene_set_texture(c2rt_host_scene* h, int texture, const float* color1, const float* color2, const double* size,
                                 const float* colorU, const float* colorV, const double* freqU, const double* freqV,
                                 const float* scaling) {
@@ -325,18 +281,14 @@ int c2rt_host_scene_set_texture(c2rt_host_scene* h, int texture, const float* co
         if (freqU) pr->freqU.assign(freqU, freqU + 3);
         if (freqV) pr->freqV.assign(freqV, freqV + 3);
         if (scaling) bm->scaling = *scaling;
-        if (h->flat_valid) {
-            const FlatTexture f = flattenTexture(t);
-            std::copy(f.colors, f.colors + 18, h->flat.tex_colors.begin() + 18 * texture);
-            std::copy(f.params, f.params + 6, h->flat.tex_params.begin() + 6 * texture);
-        }
+        if (h->flat_valid) h->flat.put(texture, flattenTexture(t));
         sc.texturesEdited({texture});
-        return followDevice(h, texture, setTextures);
+        return 0;
     });
 }
 
 // As if light `light`'s entry in the scene file had its given keys (pos [3], color [3], power) replaced (NULL: kept).  The flat
-// description and both uploaded scenes follow with c2rt_scene_set_lights.  A bad index changes nothing.
+// description and the uploaded scene follow (Scene::lightsEdited).  A bad index changes nothing.
 int c2rt_host_scene_set_light(c2rt_host_scene* h, int light, const double* pos, const float* color, const float* power) {
     return guarded([&]() -> int {
         Scene& sc = *h->scene;
@@ -345,14 +297,9 @@ int c2rt_host_scene_set_light(c2rt_host_scene* h, int light, const double* pos, 
         if (pos) l.pos = Vector(pos[0], pos[1], pos[2]);
         if (color) l.lightColor = Color(color[0], color[1], color[2]);
         if (power) l.lightPower = *power;
-        if (h->flat_valid) {
-            const FlatLight f = flattenLight(l);
-            std::copy(f.pos, f.pos + 3, h->flat.light_pos.begin() + 3 * light);
-            std::copy(f.color, f.color + 3, h->flat.light_color.begin() + 3 * light);
-            h->flat.light_power[light] = f.power;
-        }
+        if (h->flat_valid) h->flat.put(light, flattenLight(l));
         sc.lightsEdited({light});
-        return followDevice(h, light, setLights);
+        return 0;
     });
 }
 
@@ -362,121 +309,51 @@ void c2rt_host_frame_blocks(c2rt_host_scene* h, uint64_t seed, int count_rays, c
     *cam = flattenCamera(h->scene->camera);
     *set = flattenSettings(h->scene->settings, seed, count_rays != 0);
 }
-// uploaded scene for c2rt_render_device (created on first use under the current c2rt_init)
-c2rt_scene* c2rt_host_device_scene(c2rt_host_scene* h) {
-    if (h->device) return h->device;
-    const c2rt_scene_desc* d = c2rt_host_scene_desc(h);
-    if (!d) return nullptr;
-    int rc = c2rt_scene_create(d, &h->device);
-    if (rc != C2RT_OK) {
-        g_host_err = std::string("libc2rt: ") + c2rt_last_error();
-        h->device = nullptr;
-    }
-    return h->device;
-}
-
 // Renderer(scene, output).renderRT() with HOST buffers (rgb: W*H*3 floats, argb nullable)
 int c2rt_host_render(c2rt_host_scene* h, float* rgb, uint32_t* argb, uint64_t seed, int count_rays, c2rt_stats* stats) {
-    try {
-        Scene& sc = *h->scene;
-        const uint32_t W = sc.settings.frameWidth, H = sc.settings.frameHeight;
-        sc.beginFrame();
-        // render straight into the caller's buffer: borrow it as the Image's storage
-        c2rt_camera cam = flattenCamera(sc.camera);
-        c2rt_settings set = flattenSettings(sc.settings, seed, count_rays != 0);
-        c2rt_scene* dev = c2rt_host_device_scene(h);
-        if (!dev) return C2RT_ERR_CUDA;
-        (void)W; (void)H;
-        int rc = c2rt_render(dev, &cam, &set, rgb, argb, stats);
-        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
-        return rc;
-    } catch (const std::exception& e) {
-        g_host_err = e.what();
-        return C2RT_ERR_INVALID_ARG;
-    }
+    Scene& sc = *h->scene;
+    sc.beginFrame();
+    const c2rt_camera cam = flattenCamera(sc.camera);
+    const c2rt_settings set = flattenSettings(sc.settings, seed, count_rays != 0);
+    return onDevice(h, [&](c2rt_scene* dev) { return c2rt_render(dev, &cam, &set, rgb, argb, stats); });
 }
 
 // renderPixel's hit record for every pixel into caller-owned HOST planes (c2rt_render_hits; `seed`: DOF / stereo frames)
 int c2rt_host_render_hits(c2rt_host_scene* h, const c2rt_hit_planes* planes, uint64_t seed, c2rt_stats* stats) {
-    try {
-        Scene& sc = *h->scene;
-        sc.beginFrame();
-        c2rt_camera cam = flattenCamera(sc.camera);
-        c2rt_settings set = flattenSettings(sc.settings, seed, false);
-        c2rt_scene* dev = c2rt_host_device_scene(h);
-        if (!dev) return C2RT_ERR_CUDA;
-        int rc = c2rt_render_hits(dev, &cam, &set, planes, stats);
-        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
-        return rc;
-    } catch (const std::exception& e) {
-        g_host_err = e.what();
-        return C2RT_ERR_INVALID_ARG;
-    }
+    Scene& sc = *h->scene;
+    sc.beginFrame();
+    const c2rt_camera cam = flattenCamera(sc.camera);
+    const c2rt_settings set = flattenSettings(sc.settings, seed, false);
+    return onDevice(h, [&](c2rt_scene* dev) { return c2rt_render_hits(dev, &cam, &set, planes, stats); });
 }
 
 // the closest hit of n caller-supplied rays into caller-owned HOST arrays (c2rt_trace_rays)
 int c2rt_host_trace_rays(c2rt_host_scene* h, size_t n, const double* origins, const double* dirs, const c2rt_ray_hits* out,
                          c2rt_stats* stats) {
-    try {
-        c2rt_scene* dev = c2rt_host_device_scene(h);
-        if (!dev) return C2RT_ERR_CUDA;
-        int rc = c2rt_trace_rays(dev, n, origins, dirs, out, stats);
-        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
-        return rc;
-    } catch (const std::exception& e) {
-        g_host_err = e.what();
-        return C2RT_ERR_INVALID_ARG;
-    }
+    return onDevice(h, [&](c2rt_scene* dev) { return c2rt_trace_rays(dev, n, origins, dirs, out, stats); });
 }
 
 // testVisibility(from[i], to[i]) for n pairs into a caller-owned HOST array (c2rt_test_visibility)
 int c2rt_host_test_visibility(c2rt_host_scene* h, size_t n, const double* from, const double* to, uint8_t* visible, c2rt_stats* stats) {
-    try {
-        c2rt_scene* dev = c2rt_host_device_scene(h);
-        if (!dev) return C2RT_ERR_CUDA;
-        int rc = c2rt_test_visibility(dev, n, from, to, visible, stats);
-        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
-        return rc;
-    } catch (const std::exception& e) {
-        g_host_err = e.what();
-        return C2RT_ERR_INVALID_ARG;
-    }
+    return onDevice(h, [&](c2rt_scene* dev) { return c2rt_test_visibility(dev, n, from, to, visible, stats); });
 }
 
 // trace(ray) at depth 0 for n caller-supplied rays into caller-owned HOST arrays (c2rt_shade_rays; rgb / argb nullable), with
 // the scene file's ambientLightColor
 int c2rt_host_shade_rays(c2rt_host_scene* h, size_t n, const double* origins, const double* dirs, float* rgb, uint32_t* argb,
                          c2rt_stats* stats) {
-    try {
-        const Color& amb = h->scene->settings.ambientLightColor;
-        const float ambient[3] = {amb.r, amb.g, amb.b};
-        c2rt_scene* dev = c2rt_host_device_scene(h);
-        if (!dev) return C2RT_ERR_CUDA;
-        int rc = c2rt_shade_rays(dev, ambient, n, origins, dirs, rgb, argb, stats);
-        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
-        return rc;
-    } catch (const std::exception& e) {
-        g_host_err = e.what();
-        return C2RT_ERR_INVALID_ARG;
-    }
+    const Color& amb = h->scene->settings.ambientLightColor;
+    const float ambient[3] = {amb.r, amb.g, amb.b};
+    return onDevice(h, [&](c2rt_scene* dev) { return c2rt_shade_rays(dev, ambient, n, origins, dirs, rgb, argb, stats); });
 }
 
 // renderPixel(scene, output, x, y) (renderer.d:46-57)
 int c2rt_host_render_pixel(c2rt_host_scene* h, int x, int y, float rgb[3], c2rt_hit* hit) {
-    try {
-        Scene& sc = *h->scene;
-        sc.beginFrame();
-        c2rt_camera cam = flattenCamera(sc.camera);
-        c2rt_settings set = flattenSettings(sc.settings, 0, false);
-        c2rt_scene* dev = c2rt_host_device_scene(h);
-        if (!dev) return C2RT_ERR_CUDA;
-        int rc = c2rt_render_pixel(dev, &cam, &set, x, y, rgb, hit);
-        if (rc != C2RT_OK) g_host_err = std::string("libc2rt: ") + c2rt_last_error();
-        return rc;
-    } catch (const std::exception& e) {
-        g_host_err = e.what();
-        return C2RT_ERR_INVALID_ARG;
-    }
+    Scene& sc = *h->scene;
+    sc.beginFrame();
+    const c2rt_camera cam = flattenCamera(sc.camera);
+    const c2rt_settings set = flattenSettings(sc.settings, 0, false);
+    return onDevice(h, [&](c2rt_scene* dev) { return c2rt_render_pixel(dev, &cam, &set, x, y, rgb, hit); });
 }
 
 // camera.d:211-229 rotate / :181-204 move — what the GUI's key handlers call between frames (raytracer_demo.d:268-340)

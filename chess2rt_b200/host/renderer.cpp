@@ -1,6 +1,5 @@
 #include "renderer.hpp"
 
-#include <algorithm>
 #include <cstring>
 
 namespace rt {
@@ -23,40 +22,16 @@ void setRenderDevices(int nGpus, const int* deviceIds) {
 Renderer::Renderer(const Scene& scene, Image<Color>& output, std::atomic<bool>* isRendering, const std::atomic<bool>* isStopRequested)
     : scene_(scene), output_(output), isRendering_(isRendering), isStopRequested_(isStopRequested) {}
 
-c2rt_scene* Renderer::device() {
-    if (!scene_.deviceScene) {
-        FlatScene flat = flatten(scene_);
+c2rt_scene* uploadedScene(const Scene& scene) {
+    if (!scene.deviceScene) {
+        FlatScene flat = flatten(scene);
         c2rt_scene_desc d = flat.desc();
         auto holder = std::make_shared<DeviceSceneHolder>();
         int rc = c2rt_scene_create(&d, &holder->handle);
         if (rc != C2RT_OK) raise(rc);
-        scene_.deviceScene = holder;
+        scene.deviceScene = holder;
     }
-    return static_cast<DeviceSceneHolder*>(scene_.deviceScene.get())->handle;
-}
-
-void Scene::nodesEdited(const std::vector<int>& indices) {
-    if (!deviceScene || indices.empty()) return;   // (no uploaded scene: the next frame flattens the whole scene)
-    const size_t n = indices.size();
-    std::vector<uint32_t> ids(n);
-    std::vector<int32_t> geom(n);
-    std::vector<double> m(9 * n), inv(9 * n), inv_t(9 * n), off(3 * n);
-    for (size_t k = 0; k < n; k++) {
-        if (indices[k] < 0 || (size_t)indices[k] >= nodes.size()) throw RTException("nodesEdited: node index out of range");
-        const FlatNode f = flattenNode(*this, *nodes[indices[k]]);
-        ids[k] = (uint32_t)indices[k];
-        geom[k] = f.geom;
-        std::copy(f.transform, f.transform + 9, m.begin() + 9 * k);
-        std::copy(f.inverse, f.inverse + 9, inv.begin() + 9 * k);
-        std::copy(f.inverse_t, f.inverse_t + 9, inv_t.begin() + 9 * k);
-        std::copy(f.offset, f.offset + 3, off.begin() + 3 * k);
-    }
-    c2rt_scene* handle = static_cast<DeviceSceneHolder*>(deviceScene.get())->handle;
-    int rc = c2rt_scene_set_nodes(handle, n, ids.data(), geom.data(), m.data(), inv.data(), inv_t.data(), off.data());
-    if (rc != C2RT_OK) {
-        invalidateDeviceScene();   // the next frame re-creates it from the edited scene
-        raise(rc);
-    }
+    return static_cast<DeviceSceneHolder*>(scene.deviceScene.get())->handle;
 }
 
 namespace {
@@ -74,6 +49,7 @@ void editDeviceScene(Scene& scene, const std::vector<int>& indices, Set set) {
 
 }  // namespace
 
+void Scene::nodesEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setNodes); }
 void Scene::nodeShadersEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setNodeShaders); }
 void Scene::shadersEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setShaders); }
 void Scene::texturesEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setTextures); }
@@ -100,7 +76,7 @@ void Renderer::renderRT() {
     static_assert(sizeof(Color) == 3 * sizeof(float), "Color must be three packed floats (color.d:27-35)");
     if (options.argbOnly && !argb) throw RTException("argbOnly needs RenderOptions::argb");
     float* rgb = options.argbOnly ? nullptr : reinterpret_cast<float*>(output_.pixels.data());
-    int rc = c2rt_render(device(), &cam, &set, rgb, argb, &lastStats);
+    int rc = c2rt_render(uploadedScene(scene_), &cam, &set, rgb, argb, &lastStats);
     cancelled = rc == C2RT_CANCELLED;   // a stop request reached the frame in flight: return like the reference's `return end()`
     if (rc != C2RT_OK && !cancelled) raise(rc);
 }
@@ -117,7 +93,7 @@ void Renderer::renderHits(HitPlanes& planes) {
     p.dist = planes.dist.empty() ? nullptr : planes.dist.data();
     p.normal = planes.normal.empty() ? nullptr : planes.normal.data();
     p.uv = planes.uv.empty() ? nullptr : planes.uv.data();
-    int rc = c2rt_render_hits(device(), &cam, &set, &p, &lastStats);
+    int rc = c2rt_render_hits(uploadedScene(scene_), &cam, &set, &p, &lastStats);
     if (rc != C2RT_OK) raise(rc);
 }
 
@@ -143,7 +119,7 @@ void Renderer::traceRays(const std::vector<Vector>& orig, const std::vector<Vect
     p.p = hits.p.empty() ? nullptr : hits.p.data();
     p.normal = hits.normal.empty() ? nullptr : hits.normal.data();
     p.uv = hits.uv.empty() ? nullptr : hits.uv.data();
-    int rc = c2rt_trace_rays(device(), n, o.data(), d.data(), &p, &lastStats);
+    int rc = c2rt_trace_rays(uploadedScene(scene_), n, o.data(), d.data(), &p, &lastStats);
     if (rc != C2RT_OK) raise(rc);
 }
 
@@ -151,7 +127,7 @@ void Renderer::testVisibility(const std::vector<Vector>& from, const std::vector
     if (to.size() != from.size()) throw RTException("testVisibility: as many `to` points as `from` points are needed");
     const std::vector<double> f = flattenVectors(from), t = flattenVectors(to);
     visible.resize(from.size());
-    int rc = c2rt_test_visibility(device(), from.size(), f.data(), t.data(), visible.data(), &lastStats);
+    int rc = c2rt_test_visibility(uploadedScene(scene_), from.size(), f.data(), t.data(), visible.data(), &lastStats);
     if (rc != C2RT_OK) raise(rc);
 }
 
@@ -165,7 +141,7 @@ void Renderer::shadeRays(const std::vector<Vector>& orig, const std::vector<Vect
     const float ambient[3] = {amb.r, amb.g, amb.b};
     out.resize(n);
     if (argb) argb->resize(n);
-    int rc = c2rt_shade_rays(device(), ambient, n, o.data(), d.data(), reinterpret_cast<float*>(out.data()),
+    int rc = c2rt_shade_rays(uploadedScene(scene_), ambient, n, o.data(), d.data(), reinterpret_cast<float*>(out.data()),
                              argb ? argb->data() : nullptr, &lastStats);
     if (rc != C2RT_OK) raise(rc);
 }
@@ -180,7 +156,7 @@ Color Renderer::renderPixelNoAA(int x, int y) {
     c2rt_settings set = flattenSettings(scene_.settings, options.rngSeed, false);
     float rgb[3];
     c2rt_hit hit;
-    int rc = c2rt_render_pixel(device(), &cam, &set, x, y, rgb, &hit);
+    int rc = c2rt_render_pixel(uploadedScene(scene_), &cam, &set, x, y, rgb, &hit);
     if (rc != C2RT_OK) raise(rc);
     Color c(rgb[0], rgb[1], rgb[2]);
     output_(x, y) = c;  // renderer.d:226

@@ -78,7 +78,6 @@ private:
     Image<Color>& output_;
     std::atomic<bool>* isRendering_;
     const std::atomic<bool>* isStopRequested_;
-    c2rt_scene* device();
 };
 
 // Spawns the render thread like the reference does; `worker` (optional) receives the thread so a
@@ -96,5 +95,10 @@ void requestStop(std::atomic<bool>* isStopRequested);
 
 // c2rt_init wrapper: selects the GPUs the next frames are banded over (default: device 0 only).
 void setRenderDevices(int nGpus, const int* deviceIds = nullptr);
+
+// The scene's uploaded copy (Scene::deviceScene), which every frame and query renders through: created from flatten(scene) on
+// first use, under the GPUs setRenderDevices selected, and kept until the scene drops it.  Throws BackendException on a library
+// error (InvalidSceneException on a dangling reference).
+c2rt_scene* uploadedScene(const Scene& scene);
 
 }  // namespace rt

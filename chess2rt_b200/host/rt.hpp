@@ -273,8 +273,9 @@ public:
 
     void beginFrame() { camera.beginFrame(); }
 
-    // New with the CUDA backend: the uploaded (flattened) scene, created on first render and
-    // reused by every later frame; see renderer.cpp.  Call invalidateDeviceScene() after
+    // New with the CUDA backend: the uploaded (flattened) scene, created on first use by
+    // uploadedScene (renderer.hpp) and reused by every later frame and query, the Renderer's and
+    // the C entry points' (host_capi.cpp) alike.  Call invalidateDeviceScene() after
     // editing geometry or the environment, adding / removing entities, changing a texture's kind
     // or a bitmap's pixels (camera and settings are per-frame).  After changing only existing
     // entities' properties, call the matching hook instead: it re-flattens the listed entities
