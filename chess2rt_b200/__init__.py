@@ -11,6 +11,7 @@ _API_NAMES = (
     "C2rtError", "HostScene", "HitPlanes", "Stats", "band_rows_owned", "device_count", "init", "lib", "host_lib", "render_device",
     "render_hits_device", "RayHits", "trace_rays_device", "test_visibility_device", "shade_rays_device", "scene_set_nodes", "scene_set_node_shaders", "scene_set_shaders",
     "scene_set_textures", "scene_set_lights", "read_ray_counters", "deinterleave", "measure_fma_peak", "srgb_table", "rng_u31", "shutdown",
+    "FrameCache", "render_update",
 )
 
 

@@ -52,6 +52,14 @@ class Stats(C.Structure):
                 ("shadow_rays", C.c_uint64), ("n_gpus", C.c_uint32), ("launches", C.c_uint32)]
 
 
+class UpdateInfo(C.Structure):
+    """c2rt_update_info: the tiles of a c2rt_render_update"""
+    _fields_ = [("tiles_total", C.c_uint32), ("tiles_rendered", C.c_uint32), ("full", C.c_uint32), ("reserved", C.c_uint32)]
+
+    def as_dict(self):
+        return {"tiles_total": self.tiles_total, "tiles_rendered": self.tiles_rendered, "full": bool(self.full)}
+
+
 class Hit(C.Structure):
     _fields_ = [("node", C.c_int32), ("reserved", C.c_int32), ("dist", C.c_double), ("p", C.c_double * 3),
                 ("normal", C.c_double * 3), ("u", C.c_double), ("v", C.c_double)]
@@ -96,6 +104,7 @@ C_ABI_SYMBOLS = [
     "c2rt_shade_rays", "c2rt_shade_rays_device", "c2rt_band_rows_owned", "c2rt_rng_u31", "c2rt_srgb_table",
     "c2rt_frame_alloc", "c2rt_frame_free", "c2rt_frame_export", "c2rt_frame_import", "c2rt_frame_unimport", "c2rt_frame_memset", "c2rt_frame_download", "c2rt_pin_host_buffer", "c2rt_unpin_host_buffer", "c2rt_gate",
     "c2rt_measure_fma_peak", "c2rt_selftest_device_pool", "c2rt_selftest_scene_class",
+    "c2rt_frame_cache_create", "c2rt_frame_cache_destroy", "c2rt_render_update",
 ]
 
 lib.c2rt_last_error.restype = C.c_char_p
@@ -112,6 +121,11 @@ lib.c2rt_scene_set_shaders.argtypes = [C.c_void_p, C.c_size_t] + [C.c_void_p] * 
 lib.c2rt_scene_set_textures.argtypes = [C.c_void_p, C.c_size_t] + [C.c_void_p] * 3
 lib.c2rt_scene_set_lights.argtypes = [C.c_void_p, C.c_size_t] + [C.c_void_p] * 4
 lib.c2rt_render.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.c_void_p, C.c_void_p, C.POINTER(Stats)]
+lib.c2rt_frame_cache_create.argtypes = [C.POINTER(C.c_void_p)]
+lib.c2rt_frame_cache_destroy.argtypes = [C.c_void_p]
+lib.c2rt_frame_cache_destroy.restype = None
+lib.c2rt_render_update.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.POINTER(Stats), C.POINTER(UpdateInfo)]
 lib.c2rt_render_device.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Settings), C.POINTER(Band), C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.POINTER(Stats)]
 lib.c2rt_read_ray_counters.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
@@ -176,6 +190,8 @@ host_lib.c2rt_host_frame_blocks.restype = None
 host_lib.c2rt_host_device_scene.argtypes = [C.c_void_p]
 host_lib.c2rt_host_device_scene.restype = C.c_void_p
 host_lib.c2rt_host_render.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.POINTER(Stats)]
+host_lib.c2rt_host_render_update.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.POINTER(Stats),
+                                            C.POINTER(UpdateInfo)]
 host_lib.c2rt_host_render_pixel.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(Hit)]
 host_lib.c2rt_host_render_hits.argtypes = [C.c_void_p, C.POINTER(HitPlanes), C.c_uint64, C.POINTER(Stats)]
 host_lib.c2rt_host_trace_rays.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.POINTER(RayHits), C.POINTER(Stats)]
@@ -378,6 +394,28 @@ class HostScene:
             _check_host(rc)
         return rgb, a, st
 
+    def render_update(self, argb=False, argb_only=False, seed=0, count_rays=False):
+        """render()'s frame, bit for bit, through the scene's frame cache (c2rt_render_update): after edits only the tiles they
+        can have changed are rendered.  The frame goes into arrays this object keeps for the frame size and planes (the cache
+        needs the buffers of the previous frame), so the returned arrays are overwritten by the next render_update: copy them
+        to keep them.  -> (rgb[H,W,3] float32 | None with argb_only, argb[H,W] uint32 | None, Stats, info dict: tiles_total,
+        tiles_rendered, full)"""
+        w, h = self.frame_size
+        key = (w, h, bool(argb or argb_only), bool(argb_only))
+        if getattr(self, "_update_key", None) != key:   # new buffers: the next frame is a full one
+            self._update_key = key
+            self._update_rgb = None if argb_only else np.zeros((h, w, 3), np.float32)
+            self._update_argb = np.zeros((h, w), np.uint32) if key[2] else None
+        rgb, a = self._update_rgb, self._update_argb
+        st, info = Stats(), UpdateInfo()
+        rc = host_lib.c2rt_host_render_update(self._h, rgb.ctypes.data if rgb is not None else None,
+                                              a.ctypes.data if a is not None else None, seed, int(count_rays), C.byref(st),
+                                              C.byref(info))
+        self.cancelled = rc == 1   # C2RT_CANCELLED (the cache starts over at the next call)
+        if rc != 1:
+            _check_host(rc)
+        return rgb, a, st, info.as_dict()
+
     def camera_rotate(self, d_yaw, d_roll=0.0, d_pitch=0.0):
         host_lib.c2rt_host_camera_rotate(self._h, d_yaw, d_roll, d_pitch)
 
@@ -554,6 +592,37 @@ def scene_set_lights(scene_handle, lights, pos, color, power):
     n = len(ids)
     arrs = [_entries(pos, n, 3, np.float64, "pos"), _entries(color, n, 3, np.float32, "color"), _entries(power, n, 1, np.float32, "power")]
     _check(lib.c2rt_scene_set_lights(scene_handle, n, ids.ctypes.data, *[a.ctypes.data for a in arrs]))
+
+
+class FrameCache:
+    """A c2rt_frame_cache for render_update (destroyed by close() or when collected)."""
+
+    def __init__(self):
+        h = C.c_void_p()
+        _check(lib.c2rt_frame_cache_create(C.byref(h)))
+        self.handle = h.value
+
+    def close(self):
+        if self.handle:
+            lib.c2rt_frame_cache_destroy(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def render_update(scene_handle, cam, settings, cache, rgb, argb=None):
+    """c2rt_render_update into HOST numpy arrays (rgb [H,W,3] float32 and argb [H,W] uint32, either None), which must hold what
+    the previous render_update with `cache` (a FrameCache, or a raw handle) wrote into them -> (Stats, info dict).  A cancelled
+    frame raises C2rtError with code 1."""
+    st, info = Stats(), UpdateInfo()
+    handle = cache.handle if isinstance(cache, FrameCache) else cache
+    _check(lib.c2rt_render_update(scene_handle, C.byref(cam), C.byref(settings), handle, rgb.ctypes.data if rgb is not None else None,
+                                  argb.ctypes.data if argb is not None else None, C.byref(st), C.byref(info)))
+    return st, info.as_dict()
 
 
 def render_device(scene_handle, cam, settings, d_rgb_ptr, d_argb_ptr=None, band=None, stream=None):

@@ -36,6 +36,11 @@ cudaError_t launch_deinterleave(const void* src, void* dst, uint32_t row_words, 
 cudaError_t launch_fma_peak(bool fp64, int blocks, int threads, int iters, void* d_out, cudaStream_t st);
 cudaError_t launch_gate(void* gate, uint32_t round, uint32_t n_ranks, void* err, cudaStream_t st);
 cudaError_t launch_signal(void* flag, uint32_t frame_no, cudaStream_t st);
+cudaError_t launch_frame_record(const FrameParams& fp, int mode, const uint32_t* tiles, PatchRecord* patches, uint32_t n, cudaStream_t st);
+cudaError_t launch_dirty_tiles(const FrameParams& fp, const PatchRecord* patches, const float4* edits, uint32_t n_edits, uint32_t n_tiles,
+                               uint32_t* list, cudaStream_t st);
+cudaError_t launch_gather_tiles(const float* rgb, const uint32_t* argb, uint32_t W, uint32_t rows, const uint32_t* tiles, uint32_t n,
+                                float* out_rgb, uint32_t* out_argb, cudaStream_t st);
 }  // namespace c2rt
 
 using namespace c2rt;
@@ -84,6 +89,7 @@ struct Context {
     int n = 0;
     DeviceCtx d[C2RT_MAX_GPUS];
     uint64_t next_scene_id = 1;
+    uint64_t generation = 0;   // bumped by every c2rt_init: a c2rt_frame_cache filled under another configuration starts over
     uint8_t lut[4097];
 };
 
@@ -207,6 +213,7 @@ int init_locked(int n_gpus, const int* ids) {
     for (int i = 0; i < g_ctx.n; i++) destroy_device(g_ctx.d[i]);
     g_ctx.n = 0;
     g_ctx.inited = false;
+    g_ctx.generation++;
     for (int i = 0; i < 4097; i++) g_ctx.lut[i] = srgb8((float)i / 4096.f);
     for (int i = 0; i < n_gpus; i++) {
         int dev = ids ? ids[i] : i;
@@ -284,7 +291,8 @@ struct SceneRecords {
 };
 
 struct c2rt_scene : SceneRecords {
-    uint64_t id;
+    uint64_t id;                         // new after every edit: which scene block a device holds
+    uint64_t serial;                     // the id c2rt_scene_create gave it, kept through edits (c2rt_frame_cache's key)
     SceneSource src;
     DevScene host;                       // constant block; record arrays copied in from the vectors when they fit
     std::vector<DevGeom> geoms;
@@ -984,12 +992,68 @@ int check_hit_args(const c2rt_scene* s, const c2rt_camera* cam, const c2rt_setti
     return C2RT_OK;
 }
 
+// One device's part of a c2rt_frame_cache (c2rt_render_update): the frame's compact planes and patch records in render_bands'
+// layout, the dirty-tile list, and the staging of a partial frame's tiles on their way to the host planes.
+struct CacheSlot {
+    int dev = -1;                    // the device the buffers live on
+    float* d_rgb = nullptr;
+    uint32_t* d_argb = nullptr;
+    PatchRecord* d_patches = nullptr;    // one per warp patch of the slot's tiles (scene_dev.h PatchRecord)
+    uint32_t* d_list = nullptr;      // [0] dirty tiles, [1..] their local indices (dirty_tiles_kernel)
+    float4* d_edits = nullptr;       // the changed nodes' bounds, before and after
+    uint32_t* d_stage = nullptr;     // gathered tiles: rgb words, then argb words
+    uint32_t* h_list = nullptr;      // pinned read-back of d_list's head
+    uint32_t* h_stage = nullptr;     // pinned read-back of d_stage
+    size_t rgb_cap = 0, argb_cap = 0, patch_cap = 0, list_cap = 0, edit_cap = 0, stage_cap = 0, h_list_cap = 0, h_stage_cap = 0;
+    uint32_t tiles_rendered = 0;     // by the current call
+};
+
+void free_slot(CacheSlot& u) {
+    if (u.dev >= 0 && cudaSetDevice(u.dev) == cudaSuccess) {
+        cudaFree(u.d_rgb); cudaFree(u.d_argb); cudaFree(u.d_patches); cudaFree(u.d_list); cudaFree(u.d_edits); cudaFree(u.d_stage);
+        cudaFreeHost(u.h_list); cudaFreeHost(u.h_stage);
+    }
+    cudaGetLastError();
+    u = CacheSlot();
+}
+
+// Grows a pinned host buffer to at least `elems` elements (by half again, so a growing partial frame does not pin anew every
+// call); its contents are not kept.
+template <class T>
+int grow_pinned(T*& buf, size_t& cap, size_t elems) {
+    if (cap >= elems) return C2RT_OK;
+    cudaFreeHost(buf);
+    buf = nullptr; cap = 0;
+    elems = std::max<size_t>(elems + elems / 2, 1024);
+    CU(cudaMallocHost((void**)&buf, elems * sizeof(T)));
+    cap = elems;
+    return C2RT_OK;
+}
+
+// The bands of device slot i of an n-device frame of H rows in bands of brows (frame_band_rows): fn(b, y0, rows, local_row) for
+// its b-th band, frame rows [y0, y0 + rows), held from row local_row on in the slot's compact buffers.  Stops at the first
+// non-zero status and returns it; *bands gets the number of bands visited.
+template <class F>
+int for_each_band(int i, int n, uint32_t H, uint32_t brows, uint32_t* bands, F&& fn) {
+    uint32_t local_row = 0, b = 0;
+    for (uint32_t y0 = (uint32_t)i * brows; y0 < H; y0 += (uint32_t)n * brows, b++) {
+        const uint32_t rows = std::min<uint32_t>(brows, H - y0);
+        const int rc = fn(b, y0, rows, local_row);
+        if (rc) return rc;
+        local_row += rows;
+    }
+    *bands = b;
+    return C2RT_OK;
+}
+
 // Device slot i's share of an n-device frame: its bands (frame_band_rows) render into the slot's compact buffers, which hold
 // only its own rows in order (the whole frame when n == 1), and each band is copied to its rows of the caller's host planes
 // on copy_stream once its launch has finished.  A colour frame (c2rt_render: rgb, argb) or, with `hits`, a hit frame
 // (c2rt_render_hits: its host planes).  Returns when the copies are complete.
+// `slot` (c2rt_render_update's full frames; colour frames only): the compact buffers are the slot's, and with `record` the
+// MODE_RECORD kernel also fills the slot's patch records.
 int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb,
-                 const c2rt_hit_planes* hits, uint32_t* launches_out, float* kernel_ms_out) {
+                 const c2rt_hit_planes* hits, CacheSlot* slot, bool record, uint32_t* launches_out, float* kernel_ms_out) {
     const uint32_t W = set->frame_width, H = set->frame_height;
     const uint32_t brows = frame_band_rows(n, H, W);
     DeviceCtx& c = g_ctx.d[i];
@@ -1019,18 +1083,22 @@ int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt
         d_hits.uv = hits->uv ? (float*)planes[3].dev : nullptr;
     } else {
         fp.cancel = c.d_cancel;
-        rc = rgb ? grow_buffer(c.d_rgb, c.rgb_cap, need * 3) : C2RT_OK;
-        if (rc == C2RT_OK && argb) rc = grow_buffer(c.d_argb, c.argb_cap, need);
+        float*& d_rgb = slot ? slot->d_rgb : c.d_rgb;
+        uint32_t*& d_argb = slot ? slot->d_argb : c.d_argb;
+        rc = rgb ? grow_buffer(d_rgb, slot ? slot->rgb_cap : c.rgb_cap, need * 3) : C2RT_OK;
+        if (rc == C2RT_OK && argb) rc = grow_buffer(d_argb, slot ? slot->argb_cap : c.argb_cap, need);
+        if (rc == C2RT_OK && record)
+            rc = grow_buffer(slot->d_patches, slot->patch_cap,
+                             (size_t)(W + TILE_W - 1) / TILE_W * local_tile_rows(H, fp.rank, fp.n_ranks, brows) * (BLOCK_THREADS / 32));
         if (rc) return rc;
-        fp.rgb = rgb ? c.d_rgb : nullptr;
-        fp.argb = argb ? c.d_argb : nullptr;
-        planes[0] = {rgb, (uint32_t*)c.d_rgb, 3};
-        planes[1] = {argb, c.d_argb, 1};
+        fp.rgb = rgb ? d_rgb : nullptr;
+        fp.argb = argb ? d_argb : nullptr;
+        planes[0] = {rgb, (uint32_t*)d_rgb, 3};
+        planes[1] = {argb, d_argb, 1};
     }
     CU(cudaEventRecord(c.e0, c.stream));
-    uint32_t local_row = 0, b = 0;
-    for (uint32_t y0 = (uint32_t)i * brows; y0 < H; y0 += (uint32_t)n * brows, b++) {
-        const uint32_t rows = std::min<uint32_t>(brows, H - y0);
+    uint32_t bands = 0;
+    rc = for_each_band(i, n, H, brows, &bands, [&](uint32_t b, uint32_t y0, uint32_t rows, uint32_t local_row) -> int {
         if (b >= c.band_done.size()) {
             cudaEvent_t e;
             CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -1039,6 +1107,7 @@ int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt
         fp.tile_row0 = b * fp.tiles_per_band;
         const uint32_t tile_rows = (rows + TILE_H - 1) / TILE_H;
         if (hits) CU(launch_hits(fp, s->mode, tile_rows, d_hits, c.stream));
+        else if (record) CU(launch_frame_record(fp, s->mode, nullptr, slot->d_patches, tile_rows, c.stream));
         else CU(launch_frame(fp, s->mode, tile_rows, c.stream));
         CU(cudaEventRecord(c.band_done[b], c.stream));
         CU(cudaStreamWaitEvent(c.copy_stream, c.band_done[b], 0));
@@ -1046,13 +1115,15 @@ int render_bands(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt
             if (p.host)
                 CU(cudaMemcpyAsync((uint32_t*)p.host + (size_t)y0 * W * p.words, p.dev + (size_t)local_row * W * p.words,
                                    (size_t)rows * W * p.words * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.copy_stream));
-        local_row += rows;
-    }
+        return C2RT_OK;
+    });
+    if (rc) return rc;
     CU(cudaEventRecord(c.e1, c.stream));
     CU(cudaStreamSynchronize(c.copy_stream));
     CU(cudaEventSynchronize(c.e1));
     CU(cudaEventElapsedTime(kernel_ms_out, c.e0, c.e1));
-    *launches_out = b;   // one launch per band
+    *launches_out = bands;   // one launch per band
+    if (slot) slot->tiles_rendered = (W + TILE_W - 1) / TILE_W * local_tile_rows(H, fp.rank, fp.n_ranks, brows);
     return C2RT_OK;
 }
 
@@ -1097,8 +1168,86 @@ int run_devices_locked(c2rt_scene* s, Work&& work, uint32_t& launches, double& k
 int render_devices_locked(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb,
                           const c2rt_hit_planes* hits, uint32_t& launches, double& kernel_ms) {
     return run_devices_locked(
-        s, [&](int i, uint32_t* l, float* ms) { return render_bands(i, g_ctx.n, s, cam, set, rgb, argb, hits, l, ms); }, launches,
+        s, [&](int i, uint32_t* l, float* ms) { return render_bands(i, g_ctx.n, s, cam, set, rgb, argb, hits, nullptr, false, l, ms); }, launches,
         kernel_ms);
+}
+
+// ---- partial frames (c2rt_render_update)
+// Device slot i's part of a partial frame: the dirty test of its tiles against `edits` (the changed nodes' bounds, before and
+// after), one read-back of the count and the head of the list, the MODE_RECORD kernel over the listed tiles (which refreshes their
+// patch records), their gather into tile-major staging, one copy of that to pinned memory, and the scatter of each tile's rows
+// into the host planes.  When more tiles are dirty than the read-back holds (a quarter of the slot's tiles and 256 more), the
+// slot renders all its tiles instead, as a full frame does.
+int update_tiles(int i, int n, c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, float* rgb, uint32_t* argb,
+                 CacheSlot& u, const std::vector<float4>& edits, uint32_t* launches_out, float* kernel_ms_out) {
+    const uint32_t W = set->frame_width, H = set->frame_height;
+    const uint32_t brows = frame_band_rows(n, H, W);
+    DeviceCtx& c = g_ctx.d[i];
+    CU(cudaSetDevice(c.dev));
+    FrameParams fp;
+    fill_params(fp, cam, set, s, i);
+    set_bands(fp, c, (uint32_t)i, (uint32_t)n, brows, true);
+    const uint32_t tiles_x = (W + TILE_W - 1) / TILE_W, n_tiles = tiles_x * local_tile_rows(H, fp.rank, fp.n_ranks, brows);
+    const uint32_t head = std::min(n_tiles, n_tiles / 4 + 256);
+    int rc = grow_buffer(u.d_list, u.list_cap, 1 + (size_t)n_tiles);
+    if (rc == C2RT_OK) rc = grow_buffer(u.d_edits, u.edit_cap, edits.size());
+    if (rc == C2RT_OK) rc = grow_pinned(u.h_list, u.h_list_cap, 1 + (size_t)head);
+    if (rc) return rc;
+    fp.cancel = c.d_cancel;
+    fp.rgb = rgb ? u.d_rgb : nullptr;
+    fp.argb = argb ? u.d_argb : nullptr;
+    CU(cudaMemcpyAsync(u.d_edits, edits.data(), edits.size() * sizeof(float4), cudaMemcpyHostToDevice, c.stream));
+    CU(cudaEventRecord(c.e0, c.stream));
+    CU(launch_dirty_tiles(fp, u.d_patches, u.d_edits, (uint32_t)edits.size(), n_tiles, u.d_list, c.stream));
+    CU(cudaMemcpyAsync(u.h_list, u.d_list, (1 + (size_t)head) * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
+    CU(cudaStreamSynchronize(c.stream));
+    const uint32_t count = u.h_list[0];
+    if (count > head) {
+        rc = render_bands(i, n, s, cam, set, rgb, argb, nullptr, &u, true, launches_out, kernel_ms_out);
+        ++*launches_out;   // (the dirty test)
+        return rc;
+    }
+    u.tiles_rendered = count;
+    *launches_out = 1;
+    if (count == 0) {
+        CU(cudaEventRecord(c.e1, c.stream));
+        CU(cudaEventSynchronize(c.e1));
+        CU(cudaEventElapsedTime(kernel_ms_out, c.e0, c.e1));
+        return C2RT_OK;
+    }
+    const size_t px = (size_t)count * BLOCK_THREADS, words = px * ((rgb ? 3 : 0) + (argb ? 1 : 0));
+    rc = grow_buffer(u.d_stage, u.stage_cap, words);
+    if (rc == C2RT_OK) rc = grow_pinned(u.h_stage, u.h_stage_cap, words);
+    if (rc) return rc;
+    const uint32_t* tiles = u.d_list + 1;
+    CU(launch_frame_record(fp, s->mode, tiles, u.d_patches, count, c.stream));
+    uint32_t* st_rgb = rgb ? u.d_stage : nullptr;
+    uint32_t* st_argb = argb ? u.d_stage + (rgb ? 3 * px : 0) : nullptr;
+    CU(launch_gather_tiles(fp.rgb, fp.argb, W, c2rt_band_rows_owned(H, fp.rank, fp.n_ranks, brows), tiles, count, (float*)st_rgb,
+                           st_argb, c.stream));
+    CU(cudaEventRecord(c.e1, c.stream));
+    CU(cudaMemcpyAsync(u.h_stage, u.d_stage, words * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
+    CU(cudaStreamSynchronize(c.stream));
+    CU(cudaEventElapsedTime(kernel_ms_out, c.e0, c.e1));
+    *launches_out = 3;
+    // the frame row of each compact row of this slot (render_bands' bands), then each tile's rows into the host planes
+    std::vector<uint32_t> frame_row(c2rt_band_rows_owned(H, fp.rank, fp.n_ranks, brows));
+    uint32_t bands;
+    for_each_band(i, n, H, brows, &bands, [&](uint32_t, uint32_t y0, uint32_t rows, uint32_t local_row) -> int {
+        for (uint32_t r = 0; r < rows; r++) frame_row[local_row + r] = y0 + r;
+        return C2RT_OK;
+    });
+    const uint32_t* h_rgb = u.h_stage;
+    const uint32_t* h_argb = u.h_stage + (rgb ? 3 * px : 0);
+    for (uint32_t k = 0; k < count; k++) {
+        const uint32_t t = u.h_list[1 + k], l = t / tiles_x, x0 = (t - l * tiles_x) * TILE_W, w = std::min<uint32_t>(TILE_W, W - x0);
+        for (uint32_t r = 0; r < (uint32_t)TILE_H && l * TILE_H + r < frame_row.size(); r++) {
+            const size_t dst = (size_t)frame_row[l * TILE_H + r] * W + x0, src = (size_t)k * BLOCK_THREADS + r * TILE_W;
+            if (rgb) memcpy(rgb + 3 * dst, h_rgb + 3 * src, 3 * w * sizeof(float));
+            if (argb) memcpy(argb + dst, h_argb + src, w * sizeof(uint32_t));
+        }
+    }
+    return C2RT_OK;
 }
 
 // ---- ray queries (c2rt_trace_rays, c2rt_test_visibility, c2rt_shade_rays)
@@ -1320,6 +1469,75 @@ int edit_scene(c2rt_scene* s, Edit&& edit) {
     return C2RT_OK;
 }
 
+// c2rt_render's stats: kernel time, devices, launches, with count_rays the counters of every device (read and zeroed), total time
+int frame_stats_locked(const c2rt_settings* set, uint32_t launches, double kernel_ms, std::chrono::steady_clock::time_point t0,
+                       c2rt_stats* stats) {
+    if (!stats) return C2RT_OK;
+    memset(stats, 0, sizeof *stats);
+    stats->kernel_ms = kernel_ms;
+    stats->n_gpus = (uint32_t)g_ctx.n;
+    stats->launches = launches;
+    if (set->count_rays) {
+        for (int i = 0; i < g_ctx.n; i++) {
+            DeviceCtx& c = g_ctx.d[i];
+            CU(cudaSetDevice(c.dev));
+            uint64_t p, sh;
+            const int rc = take_ray_counters(c, c.stream, &p, &sh);
+            if (rc) return rc;
+            stats->primary_rays += p;
+            stats->shadow_rays += sh;
+        }
+        CU(cudaSetDevice(g_ctx.d[0].dev));
+    }
+    stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return C2RT_OK;
+}
+
+}  // namespace
+
+// What c2rt_render_update delivered last: the scene (its creation serial) and the copy of its records the frame was rendered from
+// (description order, derive_records' outputs: node raw fields and bounds, shaders, textures, lights), the camera, settings,
+// output pointers and c2rt_init generation, and per context device the buffers (CacheSlot).  valid: a recorded frame that a
+// partial one may follow.
+struct c2rt_frame_cache {
+    bool valid = false;
+    uint64_t serial = 0, id = 0, generation = 0;
+    int mode = 0;
+    c2rt_camera cam;
+    c2rt_settings set;
+    float* rgb = nullptr;
+    uint32_t* argb = nullptr;
+    std::vector<DevNode> nodes;
+    std::vector<float4> bounds;
+    std::vector<DevShader> shaders;
+    std::vector<DevTex> textures;
+    std::vector<DevLight> lights;
+    CacheSlot slot[C2RT_MAX_GPUS];
+};
+
+namespace {
+
+template <class T>
+bool same_records(const std::vector<T>& a, const std::vector<T>& b) {
+    return a.size() == b.size() && (a.empty() || memcmp(a.data(), b.data(), a.size() * sizeof(T)) == 0);
+}
+
+// The changed nodes of scene s against the cache's copy: their bounds before and after into `edits`.  False when a record other
+// than a node's changed, or a changed node is unbounded before or after (the whole frame is rendered then).
+bool find_edits(const c2rt_frame_cache& k, const c2rt_scene& s, const std::vector<float4>& bounds, std::vector<float4>& edits) {
+    edits.clear();
+    if (!same_records(k.shaders, s.src.shaders) || !same_records(k.textures, s.src.textures) || !same_records(k.lights, s.src.lights) ||
+        k.nodes.size() != s.src.nodes.size())
+        return false;
+    for (size_t i = 0; i < k.nodes.size(); i++) {
+        if (memcmp(&k.nodes[i], &s.src.nodes[i], sizeof(DevNode)) == 0 && memcmp(&k.bounds[i], &bounds[i], sizeof(float4)) == 0) continue;
+        if (!(k.bounds[i].w >= 0.f && bounds[i].w >= 0.f)) return false;
+        edits.push_back(k.bounds[i]);
+        edits.push_back(bounds[i]);
+    }
+    return true;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1373,7 +1591,7 @@ int c2rt_scene_create(const c2rt_scene_desc* desc, c2rt_scene** out) {
     int rc = validate_and_build(desc, s);
     if (rc == C2RT_OK) rc = ensure_init_locked();
     if (rc == C2RT_OK) {
-        s->id = g_ctx.next_scene_id++;
+        s->id = s->serial = g_ctx.next_scene_id++;
         rc = upload_to_devices(s);
     }
     if (rc != C2RT_OK) {
@@ -1551,25 +1769,8 @@ int c2rt_render(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set,
     double kernel_ms;
     rc = render_devices_locked(s, cam, set, rgb, argb, nullptr, launches, kernel_ms);
     if (rc) return rc;
-    if (stats) {
-        memset(stats, 0, sizeof *stats);
-        stats->kernel_ms = kernel_ms;
-        stats->n_gpus = (uint32_t)g_ctx.n;
-        stats->launches = launches;
-        if (set->count_rays) {
-            for (int i = 0; i < g_ctx.n; i++) {
-                DeviceCtx& c = g_ctx.d[i];
-                CU(cudaSetDevice(c.dev));
-                uint64_t p, sh;
-                rc = take_ray_counters(c, c.stream, &p, &sh);
-                if (rc) return rc;
-                stats->primary_rays += p;
-                stats->shadow_rays += sh;
-            }
-            CU(cudaSetDevice(g_ctx.d[0].dev));
-        }
-        stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    }
+    rc = frame_stats_locked(set, launches, kernel_ms, t0, stats);
+    if (rc) return rc;
     if (take_cancel_request()) {
         g_err = "frame cancelled by c2rt_cancel: the output holds the tiles rendered before the request";
         return C2RT_CANCELLED;
@@ -1591,6 +1792,95 @@ int c2rt_cancel(void) {
     }
     if (prev >= 0) cudaSetDevice(prev);
     cudaGetLastError();
+    return C2RT_OK;
+}
+
+int c2rt_frame_cache_create(c2rt_frame_cache** out) {
+    if (!out) return fail(C2RT_ERR_INVALID_ARG, "out is null");
+    *out = new c2rt_frame_cache();
+    return C2RT_OK;
+}
+
+void c2rt_frame_cache_destroy(c2rt_frame_cache* k) {
+    if (!k) return;
+    std::lock_guard<std::mutex> g(g_mu);
+    for (CacheSlot& u : k->slot) free_slot(u);
+    if (g_ctx.inited) cudaSetDevice(g_ctx.d[0].dev);
+    delete k;
+}
+
+int c2rt_render_update(c2rt_scene* s, const c2rt_camera* cam, const c2rt_settings* set, c2rt_frame_cache* k, float* rgb,
+                       uint32_t* argb, c2rt_stats* stats, c2rt_update_info* info) {
+    const auto t0 = std::chrono::steady_clock::now();
+    int rc = check_frame_args(s, cam, set);
+    if (rc) return rc;
+    if (!rgb && !argb) return fail(C2RT_ERR_INVALID_ARG, "rgb and argb are both null");
+    if (!k) return fail(C2RT_ERR_INVALID_ARG, "cache is null");
+    const uint32_t W = set->frame_width, H = set->frame_height;
+    if (info) {
+        memset(info, 0, sizeof *info);
+        info->tiles_total = (W + TILE_W - 1) / TILE_W * ((H + TILE_H - 1) / TILE_H);
+    }
+    if (set->prepass_only && !set->prepass_enabled) {  // as c2rt_render: nothing is drawn, the image (and so the cache) stays
+        if (stats) memset(stats, 0, sizeof *stats);
+        return C2RT_OK;
+    }
+    std::lock_guard<std::mutex> g(g_mu);
+    rc = ensure_init_locked();
+    if (rc) return rc;
+    if (s->n_dev != g_ctx.n) return fail(C2RT_ERR_INVALID_ARG, "scene was created under a different c2rt_init configuration");
+    take_cancel_request();   // a cancel that arrived while no frame was in progress cancels nothing
+    if (k->generation != g_ctx.generation) {   // buffers of another configuration's devices
+        for (CacheSlot& u : k->slot) free_slot(u);
+        k->valid = false;
+        k->generation = g_ctx.generation;
+        CU(cudaSetDevice(g_ctx.d[0].dev));
+    }
+    for (int i = 0; i < g_ctx.n; i++) k->slot[i].dev = g_ctx.d[i].dev;
+    // frames that can be recorded: the camera-masked scene classes (launch_frame's sampling frames are not), no GI or preview
+    const bool sampling = cam->dof || cam->stereo_separation != 0;
+    const bool record = camera_masked(s->mode | (sampling ? MODE_SAMPLING : 0)) && !(set->gi_enabled && !cam->dof) && !set->prepass_only;
+    const std::vector<float4> bounds = node_bounds(*s);
+    std::vector<float4> edits;
+    const bool partial = record && k->valid && k->serial == s->serial && k->mode == s->mode && k->rgb == rgb && k->argb == argb &&
+                         memcmp(&k->cam, cam, sizeof *cam) == 0 && memcmp(&k->set, set, sizeof *set) == 0 &&
+                         (k->id == s->id || find_edits(*k, *s, bounds, edits));
+    k->valid = false;   // until this call completes
+    uint32_t launches = 0;
+    double kernel_ms = 0;
+    for (CacheSlot& u : k->slot) u.tiles_rendered = 0;
+    if (!partial)
+        rc = run_devices_locked(
+            s, [&](int i, uint32_t* l, float* ms) { return render_bands(i, g_ctx.n, s, cam, set, rgb, argb, nullptr, &k->slot[i], record, l, ms); },
+            launches, kernel_ms);
+    else if (!edits.empty())
+        rc = run_devices_locked(
+            s, [&](int i, uint32_t* l, float* ms) { return update_tiles(i, g_ctx.n, s, cam, set, rgb, argb, k->slot[i], edits, l, ms); },
+            launches, kernel_ms);
+    if (rc) return rc;
+    rc = frame_stats_locked(set, launches, kernel_ms, t0, stats);
+    if (rc) return rc;
+    if (info) {
+        info->full = !partial;
+        for (int i = 0; i < g_ctx.n; i++) info->tiles_rendered += k->slot[i].tiles_rendered;
+    }
+    if (take_cancel_request()) {
+        g_err = "frame cancelled by c2rt_cancel: the output holds the tiles rendered before the request";
+        return C2RT_CANCELLED;
+    }
+    k->valid = record;
+    k->serial = s->serial;
+    k->id = s->id;
+    k->mode = s->mode;
+    k->cam = *cam;
+    k->set = *set;
+    k->rgb = rgb;
+    k->argb = argb;
+    k->nodes = s->src.nodes;
+    k->bounds = bounds;
+    k->shaders = s->src.shaders;
+    k->textures = s->src.textures;
+    k->lights = s->src.lights;
     return C2RT_OK;
 }
 

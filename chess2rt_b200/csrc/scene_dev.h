@@ -138,6 +138,12 @@ struct FrameParams {
     uint32_t solo_zrows;
 };
 
+// What a MODE_RECORD frame (render_kernel.cu render_frame_kernel) keeps of one warp patch for c2rt_render_update's dirty test
+// (dirty_tiles_kernel), at (local tile row * tiles_x + tile column) * 4 + warp of its rank's tiles: a
+// sphere (x, y, z, radius) holding the FP32 origins of every shadow ray the patch's camera hits shoot, over all AA taps, as
+// shadow_mask bounds them (the centre and half-diagonal of their bounding box); radius < 0: no camera ray of the patch hit.
+typedef float4 PatchRecord;
+
 // Kernel specialisations by scene class (chosen at scene-create time, c2rt_api.cu):
 //   MODE_BOUNDED  some node has a finite bounding sphere -> FP32 ray shadow + conservative cull
 //   MODE_GENERIC  some node needs the object-space path (non-identity transform, CSG, bounded plane)
@@ -158,6 +164,9 @@ constexpr int MODE_BIG = 512;
 //                 per distinct frequency (render_kernel.cu texture_uv); 0 (all distinct) for every other scene class.  Term i
 //                 reads the sine of term upat_first(pattern, i).
 constexpr int MODE_UPAT_SHIFT = 10, MODE_UPAT_MASK = 7 << MODE_UPAT_SHIFT;
+//   MODE_RECORD   a launch flag, never a scene class: the frame body of a camera-masked class that also writes each warp patch's
+//                 PatchRecord and can render a list of tiles (render_kernel.cu g_record, c2rt_render_update)
+constexpr int MODE_RECORD = 8192;
 enum : int { UPAT_DISTINCT = 0, UPAT_01 = 1, UPAT_02 = 2, UPAT_12 = 3, UPAT_ALL = 4 };
 #ifdef __CUDACC__
 __host__ __device__

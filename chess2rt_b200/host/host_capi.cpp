@@ -318,6 +318,17 @@ int c2rt_host_render(c2rt_host_scene* h, float* rgb, uint32_t* argb, uint64_t se
     return onDevice(h, [&](c2rt_scene* dev) { return c2rt_render(dev, &cam, &set, rgb, argb, stats); });
 }
 
+// c2rt_host_render's frame through the scene's frame cache (c2rt_render_update): rgb / argb must be what the last
+// c2rt_host_render_update of this scene wrote into them
+int c2rt_host_render_update(c2rt_host_scene* h, float* rgb, uint32_t* argb, uint64_t seed, int count_rays, c2rt_stats* stats,
+                            c2rt_update_info* info) {
+    Scene& sc = *h->scene;
+    sc.beginFrame();
+    const c2rt_camera cam = flattenCamera(sc.camera);
+    const c2rt_settings set = flattenSettings(sc.settings, seed, count_rays != 0);
+    return onDevice(h, [&](c2rt_scene* dev) { return c2rt_render_update(dev, &cam, &set, frameCache(sc), rgb, argb, stats, info); });
+}
+
 // renderPixel's hit record for every pixel into caller-owned HOST planes (c2rt_render_hits; `seed`: DOF / stereo frames)
 int c2rt_host_render_hits(c2rt_host_scene* h, const c2rt_hit_planes* planes, uint64_t seed, c2rt_stats* stats) {
     Scene& sc = *h->scene;

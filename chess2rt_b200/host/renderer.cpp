@@ -12,6 +12,11 @@ struct DeviceSceneHolder {
     ~DeviceSceneHolder() { c2rt_scene_destroy(handle); }
 };
 
+struct FrameCacheHolder {
+    c2rt_frame_cache* handle = nullptr;
+    ~FrameCacheHolder() { c2rt_frame_cache_destroy(handle); }
+};
+
 }  // namespace
 
 void setRenderDevices(int nGpus, const int* deviceIds) {
@@ -32,6 +37,16 @@ c2rt_scene* uploadedScene(const Scene& scene) {
         scene.deviceScene = holder;
     }
     return static_cast<DeviceSceneHolder*>(scene.deviceScene.get())->handle;
+}
+
+c2rt_frame_cache* frameCache(const Scene& scene) {
+    if (!scene.frameCache) {
+        auto holder = std::make_shared<FrameCacheHolder>();
+        int rc = c2rt_frame_cache_create(&holder->handle);
+        if (rc != C2RT_OK) raise(rc);
+        scene.frameCache = holder;
+    }
+    return static_cast<FrameCacheHolder*>(scene.frameCache.get())->handle;
 }
 
 namespace {
@@ -55,7 +70,10 @@ void Scene::shadersEdited(const std::vector<int>& indices) { editDeviceScene(*th
 void Scene::texturesEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setTextures); }
 void Scene::lightsEdited(const std::vector<int>& indices) { editDeviceScene(*this, indices, setLights); }
 
-void Renderer::renderRT() {
+void Renderer::renderRT() { frame(false); }
+void Renderer::renderUpdate() { frame(true); }
+
+void Renderer::frame(bool update) {
     struct Done {  // renderer.d:87-91 end()
         std::atomic<bool>* flag;
         ~Done() { if (flag) flag->store(false); }
@@ -76,7 +94,8 @@ void Renderer::renderRT() {
     static_assert(sizeof(Color) == 3 * sizeof(float), "Color must be three packed floats (color.d:27-35)");
     if (options.argbOnly && !argb) throw RTException("argbOnly needs RenderOptions::argb");
     float* rgb = options.argbOnly ? nullptr : reinterpret_cast<float*>(output_.pixels.data());
-    int rc = c2rt_render(uploadedScene(scene_), &cam, &set, rgb, argb, &lastStats);
+    int rc = update ? c2rt_render_update(uploadedScene(scene_), &cam, &set, frameCache(scene_), rgb, argb, &lastStats, &lastUpdate)
+                    : c2rt_render(uploadedScene(scene_), &cam, &set, rgb, argb, &lastStats);
     cancelled = rc == C2RT_CANCELLED;   // a stop request reached the frame in flight: return like the reference's `return end()`
     if (rc != C2RT_OK && !cancelled) raise(rc);
 }

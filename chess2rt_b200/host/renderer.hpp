@@ -57,6 +57,10 @@ struct Renderer {
              const std::atomic<bool>* isStopRequested = nullptr);
 
     void renderRT();                               // renderer.d:83-189
+    // renderRT's frame, bit for bit, re-rendering only the tiles the scene's edits since the last renderUpdate can have changed
+    // (c2rt_render_update with the scene's frameCache).  The output image and options.argb must be the buffers the last
+    // renderUpdate of this scene wrote, unchanged since; lastUpdate tells how many tiles were rendered.
+    void renderUpdate();
     void renderHits(HitPlanes& planes);            // no counterpart: renderPixelNoAA's hit record for every pixel, no colour
     Color renderPixelNoAA(int x, int y);           // renderer.d:223-228 (also records lastTracingResult)
     // renderer.d:325-376's closest-hit loop on (orig[i], normalize(dir[i])) for every i (c2rt_trace_rays)
@@ -70,10 +74,12 @@ struct Renderer {
 
     TraceResult lastTracingResult;
     c2rt_stats lastStats{};
+    c2rt_update_info lastUpdate{};                 // the last renderUpdate's tiles
     RenderOptions options;
     bool cancelled = false;                        // the last renderRT ended early on a stop request (the frame is partial)
 
 private:
+    void frame(bool update);
     const Scene& scene_;
     Image<Color>& output_;
     std::atomic<bool>* isRendering_;
@@ -100,5 +106,7 @@ void setRenderDevices(int nGpus, const int* deviceIds = nullptr);
 // first use, under the GPUs setRenderDevices selected, and kept until the scene drops it.  Throws BackendException on a library
 // error (InvalidSceneException on a dangling reference).
 c2rt_scene* uploadedScene(const Scene& scene);
+// The scene's frame cache (Scene::frameCache) for c2rt_render_update, created on first use and kept with the scene.
+c2rt_frame_cache* frameCache(const Scene& scene);
 
 }  // namespace rt

@@ -288,6 +288,9 @@ public:
     // BackendException on a library error, after dropping the uploaded scene.
     mutable std::shared_ptr<void> deviceScene;
     void invalidateDeviceScene() { deviceScene.reset(); }
+    // The c2rt_frame_cache of Renderer::renderUpdate / c2rt_host_render_update (renderer.hpp frameCache): the last partial-or-full
+    // frame delivered from this scene.  It compares the uploaded scene's records itself, so edits need not tell it anything.
+    mutable std::shared_ptr<void> frameCache;
     void nodesEdited(const std::vector<int>& indices);
     void nodeShadersEdited(const std::vector<int>& indices);
     void shadersEdited(const std::vector<int>& indices);

@@ -275,6 +275,46 @@ int c2rt_render(c2rt_scene* scene, const c2rt_camera* camera, const c2rt_setting
  * to replace anyway: raytracer_demo.d:102-124).  A cancel that arrives while no frame is in progress cancels nothing. */
 int c2rt_cancel(void);
 
+/* Partial frames after edits: c2rt_render's frame, bit for bit, re-rendering only the CTA tiles (16x8 pixels) an edit since the
+ * previous frame can have changed.  A c2rt_frame_cache remembers the frame the last c2rt_render_update with it delivered: the
+ * scene records it was rendered from, its camera, settings and output pointers, and per 8x4 pixel patch a bound of the points
+ * its camera rays hit.  It owns device buffers on the devices of the c2rt_init it was filled under.  create touches no device;
+ * destroy frees the buffers (NULL is a no-op).  One cache serves one stream of frames into one pair of host buffers. */
+typedef struct c2rt_frame_cache c2rt_frame_cache;
+int c2rt_frame_cache_create(c2rt_frame_cache** out);
+void c2rt_frame_cache_destroy(c2rt_frame_cache* cache);
+
+typedef struct c2rt_update_info {
+    uint32_t tiles_total;     /* CTA tiles (16x8) of the frame */
+    uint32_t tiles_rendered;  /* tiles traced by this call (== tiles_total for a full frame) */
+    uint32_t full;            /* 1: the call rendered the whole frame (first frame, or a condition below did not hold) */
+    uint32_t reserved;
+} c2rt_update_info;
+
+/* Caller contract: on entry rgb / argb (HOST buffers, layout and nullability as c2rt_render) hold what the previous
+ * c2rt_render_update with this cache wrote into them; on return they hold exactly what c2rt_render writes for the scene's
+ * current state, camera and settings.  The call renders only the tiles that can differ from that previous frame when all of
+ * these hold, and the whole frame (refilling the cache) otherwise:
+ *   - the cache holds a frame of this scene (the same c2rt_scene_create; the scene's edits since are found by comparing its
+ *     records with the cache's copy, so any sequence of c2rt_scene_set_* calls, an edit and its undo included, is handled);
+ *   - camera and settings are byte-equal to that frame's, the same output pointers are given (and so the same planes), and the
+ *     c2rt_init configuration is the same;
+ *   - the scene class is the same and camera-masked: not plane-only (every node an unbounded world plane, a one-plane scene
+ *     included), no DOF or stereo camera, not a GI or prepass frame;
+ *   - the previous c2rt_render_update with this cache was not cancelled;
+ *   - only node records changed (transform, geometry, shader index), and every changed node has a finite bounding sphere
+ *     before and after; a shader, texture or light edit renders the whole frame.
+ * A tile is re-rendered when a changed node, in its old or its new place, can be reached by one of its camera rays or by a
+ * shadow ray from one of its camera hits (DESIGN.md §4.9); its rows are then copied to the host planes.  Every other tile of
+ * the host planes is left as it is.
+ * Errors, locking and cancellation as c2rt_render; a null cache is C2RT_ERR_INVALID_ARG.  A cancelled call returns
+ * C2RT_CANCELLED and empties the cache, so the next call renders the whole frame.  prepass_only without prepass_enabled draws
+ * nothing and leaves the cache as it is, as c2rt_render leaves the image.
+ * stats as c2rt_render (kernel_ms covers the dirty test and the gather of a partial frame); with count_rays, primary_rays /
+ * shadow_rays count the rays this call traced, only in the tiles it rendered.  info (nullable) reports the tiles. */
+int c2rt_render_update(c2rt_scene* scene, const c2rt_camera* camera, const c2rt_settings* settings, c2rt_frame_cache* cache,
+                       float* rgb, uint32_t* argb, c2rt_stats* stats, c2rt_update_info* info);
+
 /* Same frame, outputs in DEVICE memory of the CURRENT device, launched on `stream`
  * (a cudaStream_t, NULL = default stream) and NOT synchronised.  One process per GPU uses this
  * with its own band; a single-GPU caller passes band == NULL.  d_argb may be NULL.
